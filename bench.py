@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- gkm kernel entries/s (300 bp, L=11 k=7 d=3) on N B200s, next to the reference's CPU path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One process per GPU (torchrun sets RANK/LOCAL_RANK/WORLD_SIZE); torch.distributed is used for the barrier and the
 max-over-ranks only -- the path has no collective.  A "step" is one full pass of the hot path: the strict lower
@@ -18,6 +18,9 @@ its chunks of row tiles are sharded round-robin over the ranks.
             against the unmodified reference (oracle/_ref) -- a mismatch makes the run exit non-zero
   secondary configs[1] (10k, resident + e2e + one full unsampled run of the reference's own gkm_main_pywrapper),
             gkmQC's real default (wgkm L=10 k=6 d=3 on 600-bp sequences), non-uniform input, configs[4] batch scoring
+
+--dump-outputs DIR writes what the last timed e2e call returned to its caller (the resident pass behind `value` keeps its
+matrix on the device and returns nothing): a seeded sample of the rows rank 0 filled, their row ids and (npos, nneg).
 """
 import argparse
 import ctypes
@@ -268,6 +271,24 @@ def parity_rows(n, blk_cols, nblk, want=96, seed=7):
     return np.array(sorted(rows), np.int32)
 
 
+def dump_rows(owned, n, budget_bytes=48 << 20, seed=20240):
+    """row ids of the output sample, drawn from the rows this rank filled: the same for every build at a given n and
+    number of ranks, as many full float64 rows (n columns) as fit the budget"""
+    rng = np.random.default_rng(seed)
+    return np.sort(rng.choice(owned, size=min(len(owned), max(1, budget_bytes // (8 * n))), replace=False))
+
+
+def dump_outputs(out_dir, kmat, npos, nneg):
+    """what the caller of gkm_main_pywrapper received: rows of its matrix (strict lower triangle, unit diagonal, nothing
+    above) at dump_rows, and the (npos, nneg) pair the call wrote into kmat_size.  A sharded call fills only the rows of
+    this rank's chunks (their unit diagonal tells which); the sample is drawn from those"""
+    os.makedirs(out_dir, exist_ok=True)
+    rows = dump_rows(np.flatnonzero(np.diagonal(kmat) == 1.0), kmat.shape[0])
+    np.save(os.path.join(out_dir, "kmat_rows.npy"), np.ascontiguousarray(kmat[rows], np.float64))
+    np.save(os.path.join(out_dir, "kmat_row_ids.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "kmat_size.npy"), np.array([npos, nneg], np.float64))
+
+
 def check_parity(h, kmat, hist_of_rows, n, layout, threads, owned_only=True, want=96):
     """rows of the matrix the product returned (and their integer histograms) against the reference's own numbers"""
     nblk, blk_cols = layout[0], layout[1] or n
@@ -311,7 +332,12 @@ def main():
     ap.add_argument("--no-secondary", action="store_true")
     ap.add_argument("--no-parity", action="store_true", help="profiling runs only")
     ap.add_argument("--no-e2e", action="store_true", help="profiling runs only: skip the end-to-end leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed gkm_main_pywrapper call returned to DIR/<name>.npy (float64): a fixed, "
+                         "seeded sample of rows of the kernel matrix, their row ids and (npos, nneg) -- to compare two builds")
     args = ap.parse_args()
+    if args.dump_outputs and args.no_e2e:
+        ap.error("--dump-outputs writes what the end-to-end call returned: it cannot be combined with --no-e2e")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -421,6 +447,8 @@ def main():
         lib.gkmb200_get_stats(None, ctypes.byref(pst))
         h2d, d2h = int(pst.h2d_bytes), int(pst.d2h_bytes)
         e2e_stats = pst.as_dict()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, kmat, npos, nneg)
     if args.no_e2e:
         walls = [float("nan")]
     e2e_value = total_entries / float(np.mean(walls))

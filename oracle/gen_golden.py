@@ -106,8 +106,66 @@ def write_fixtures():
             # reallocs a by-value buffer and double-frees it (libgkm.c:1207-1225, :1312)
 
 
+# gkmb200_problem_index_layout() of the full-size problem below on a B200, per kernel type: (column blocks, columns per
+# block).  10 000 columns fit one block for both types (full blocks of 22 528 and 16 352 columns); a layout with more
+# blocks puts the stored rows and columns on both sides of every block boundary, like the rows the full-size GPU test
+# checks live.
+FULL10K_INDEX_LAYOUT = {2: (1, 22528), 4: (1, 16352)}
+
+
+def full_size_rows(nrows=32, ncols=256, seed=20261020):
+    """tests/golden/full10k_rows_kt{2,4}.npz: BASELINE configs[1] at full size (bench.synth(10000), 300 bp, L=11 k=7 d=3) --
+    kernel values and mismatch histograms of the rows tests/test_gpu_parity.py's full-size test checks (bench.parity_rows on
+    the index layout: both sides of every column block and chunk boundary), at ncols seeded columns below each row plus the
+    block boundary columns.  Where oracle/_ref is built the numbers are the unmodified reference's (RefHook.rows_values) and
+    the C restatement must give the same; elsewhere they are the C restatement's, which is bit-identical to the reference
+    on every golden set above.
+        python oracle/gen_golden.py --full-size"""
+    import tempfile
+    sys.path.insert(0, os.path.dirname(HERE))
+    import bench
+    n = 10000
+    arr = bench.synth(n)
+    tmp = tempfile.mkdtemp(prefix="gkmgold_")
+    pos, neg = os.path.join(tmp, "p.fa"), os.path.join(tmp, "n.fa")
+    bench.write_fasta(pos, arr[: n // 2], 0)
+    bench.write_fasta(neg, arr[n // 2:], n // 2)
+    for kt in (2, 4):
+        nblk, blk_cols = FULL10K_INDEX_LAYOUT[kt]
+        rows = bench.parity_rows(n, blk_cols, nblk, want=nrows)[:40]
+        edges = np.array([k * blk_cols + e for k in range(1, nblk) for e in (-1, 0, 1)], np.int64)
+        rng = np.random.default_rng(seed + kt)
+        pairs = [(int(r), int(c)) for r in rows
+                 for c in np.union1d(rng.choice(r, size=min(r, ncols), replace=False), edges[edges < r])]
+        row, col = (np.array(x, np.int32) for x in zip(*pairs))
+        o = pyoracle.Oracle(kt, 11, 7, 3)
+        assert o.read_problem(pos, neg) == n
+        K = np.array([o.kernel(a, b) for a, b in pairs])
+        Hm = np.array([o.hist(a, b) for a, b in pairs], np.int32)
+        o.close()
+        source = "C restatement"
+        if pyoracle.have_ref():
+            h = pyoracle.RefHook(pos, neg, kt, 11, 7, 3)
+            try:
+                Kr, Hr, _ = h.rows_values(rows, os.cpu_count() or 1)
+            finally:
+                h.close()
+            at = {int(r): i for i, r in enumerate(rows)}
+            Kref = np.array([Kr[at[a], b] for a, b in pairs])
+            Href = np.array([Hr[at[a], :, b] for a, b in pairs], np.int32)
+            assert np.array_equal(Kref, K) and np.array_equal(Href, Hm), "C restatement differs from the reference"
+            K, Hm, source = Kref, Href, "reference (C restatement identical)"
+        np.savez_compressed(os.path.join(GOLD, "full10k_rows_kt%d.npz" % kt), row=row, col=col, kmat=K, hist=Hm)
+        print("full10k_rows_kt%d: %d entries of %d rows, from the %s" % (kt, len(pairs), len(rows), source))
+    for f in (pos, neg):
+        os.remove(f)
+    os.rmdir(tmp)
+
+
 def main():
     pyoracle.build_oracle()
+    if sys.argv[1:] == ["--full-size"]:
+        return full_size_rows()
     if not pyoracle.build_ref():
         raise SystemExit("reference sources not present; cannot generate golden vectors")
     write_fixtures()

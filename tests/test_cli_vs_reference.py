@@ -14,10 +14,10 @@ import numpy as np
 import pytest
 
 import pyoracle
-from conftest import random_seqs, write_fasta
+from conftest import load_golden, random_seqs, write_fasta
 
 REF_CLI = os.path.join(pyoracle.REF_DIR, "gkmkern")
-pytestmark = pytest.mark.skipif(not os.path.exists(REF_CLI), reason="oracle/_ref/gkmkern (the compiled reference CLI) is not here")
+needs_ref_cli = pytest.mark.skipif(not os.path.exists(REF_CLI), reason="oracle/_ref/gkmkern (the compiled reference CLI) is not here")
 
 
 @pytest.fixture(scope="module")
@@ -36,6 +36,7 @@ def files(tmp_path, n, seed):
     return str(pos), str(neg)
 
 
+@needs_ref_cli
 @pytest.mark.parametrize("n", [24, 8])
 def test_same_output_file_as_the_reference_cli(tmp_path, cli, n):
     pos, neg = files(tmp_path, n, seed=n)
@@ -47,6 +48,7 @@ def test_same_output_file_as_the_reference_cli(tmp_path, cli, n):
     assert a.count(b"\n") == n
 
 
+@needs_ref_cli
 def test_rows_the_reference_cli_drops(tmp_path, cli):
     pos, neg = files(tmp_path, 26, seed=3)
     ref_out, our_out = str(tmp_path / "ref.tsv"), str(tmp_path / "ours.tsv")
@@ -59,26 +61,27 @@ def test_rows_the_reference_cli_drops(tmp_path, cli):
 
 def test_options_reach_the_engine(tmp_path, cli):
     """-t -l -k -d -M -H and -p 17 (loss-free doubles) / -b (binary): the values are those the reference's gkm_main_pywrapper
-    returns for the same parameters"""
-    if not pyoracle.have_ref():
-        pytest.skip("oracle/_ref (the compiled reference) is not here")
-    pos, neg = files(tmp_path, 10, seed=9)
-    ret, K, npos, nneg = pyoracle.call_pywrapper(pyoracle.ref_pywrapper(), pos, neg, kernel_type=4, L=8, k=5, d=3, M=40, H=30.0, nmax=16)
-    assert ret == 0 and (npos, nneg) == (5, 5)
+    returned for the same parameters and files (tests/golden, written from the unmodified reference by oracle/gen_golden.py);
+    the two stored sets move -t -M -H and -l -k -d off the CLI's defaults"""
     txt, binf = str(tmp_path / "o.tsv"), str(tmp_path / "o.bin")
-    common = ["-v", "0", "-t", "4", "-l", "8", "-k", "5", "-d", "3", "-M", "40", "-H", "30"]
-    assert subprocess.run([cli] + common + ["-p", "17", pos, neg, txt], stdout=subprocess.DEVNULL).returncode == 0
-    assert subprocess.run([cli] + common + ["-b", pos, neg, binf], stdout=subprocess.DEVNULL).returncode == 0
-    rows = [np.array([float(x) for x in line.split("\t")[:-1]]) for line in open(txt).read().splitlines()]
-    raw = open(binf, "rb").read()
-    assert np.frombuffer(raw[:4], np.int32)[0] == 10
-    flat = np.frombuffer(raw[4:], np.float64)
-    at = 0
-    for a in range(10):
-        assert np.array_equal(rows[a][:a], K[a, :a]) and rows[a][a] == 1.0
-        assert np.array_equal(flat[at:at + a], K[a, :a])
-        at += a
-    assert at == len(flat)
+    for name in ("mix_t4_L10k6d3_M255", "mix_t2_L8k4d4"):
+        g, cfg, pos, neg = load_golden(name)
+        K, n = g["kmat"], len(g["lens"])
+        common = ["-v", "0", "-t", str(cfg["kernel_type"]), "-l", str(cfg["L"]), "-k", str(cfg["k"]), "-d", str(cfg["d"]),
+                  "-M", str(cfg["M"]), "-H", repr(cfg["H"])]
+        assert subprocess.run([cli] + common + ["-p", "17", pos, neg, txt], stdout=subprocess.DEVNULL).returncode == 0
+        assert subprocess.run([cli] + common + ["-b", pos, neg, binf], stdout=subprocess.DEVNULL).returncode == 0
+        rows = [np.array([float(x) for x in line.split("\t")[:-1]]) for line in open(txt).read().splitlines()]
+        assert len(rows) == n
+        raw = open(binf, "rb").read()
+        assert np.frombuffer(raw[:4], np.int32)[0] == n
+        flat = np.frombuffer(raw[4:], np.float64)
+        at = 0
+        for a in range(n):
+            assert np.array_equal(rows[a][:a], K[a, :a]) and rows[a][a] == 1.0, (name, a)
+            assert np.array_equal(flat[at:at + a], K[a, :a]), (name, a)
+            at += a
+        assert at == len(flat)
     # what the gate refuses is refused here too, with the reference's message
     r = subprocess.run([cli, "-l", "13", pos, neg, txt], capture_output=True, text=True)
     assert r.returncode == 0 or "L" in r.stderr          # L = 13..16 is the CLI's documented extension

@@ -10,7 +10,7 @@ import numpy as np
 import pytest
 
 import pyoracle
-from conftest import golden_names, load_golden, random_seqs, write_fasta
+from conftest import GOLD, golden_names, load_golden, random_seqs, write_fasta
 from gkmqc_b200 import capi
 
 pytestmark = pytest.mark.gpu
@@ -454,6 +454,32 @@ def test_full_size_index_against_bitsliced_and_reference(kernel_type, tmp_path):
             assert np.array_equal(hist[int(r)], Hr[i, :, :r].T), "histograms of row %d differ from the reference" % r
     finally:
         h.close()
+
+
+@pytest.mark.parametrize("kernel_type", [2, 4])
+def test_full_size_index_against_stored_rows(kernel_type, tmp_path):
+    """the problem of test_full_size_index_against_bitsliced_and_reference, without a reference build: the index kernel's
+    matrix and integer histograms at the stored sample of tests/golden/full10k_rows_kt*.npz (oracle/gen_golden.py
+    --full-size: rows on both sides of the index column blocks and of the chunk boundaries, seeded columns below them)"""
+    import bench
+    stored = np.load(os.path.join(GOLD, "full10k_rows_kt%d.npz" % kernel_type))
+    n = 10000
+    arr = bench.synth(n)
+    pos, neg = str(tmp_path / "p.fa"), str(tmp_path / "n.fa")
+    bench.write_fasta(pos, arr[: n // 2], 0)
+    bench.write_fasta(neg, arr[n // 2:], n // 2)
+    capi.set_option("kernel", "index")
+    try:
+        with capi.Problem(kernel_type, 11, 7, 3) as P:
+            P.read(pos, neg)
+            K = P.kernel_lower()
+            assert P.stats()["kernel_variant"] == 4
+            hist = {int(r): P.hist_block(int(r), 1, 0, int(r))[0] for r in np.unique(stored["row"])}
+    finally:
+        capi.set_option("kernel", "auto")
+    rows, cols = stored["row"], stored["col"]
+    assert np.array_equal(K[rows, cols], stored["kmat"]), "kernel values differ from the stored ones"
+    assert np.array_equal(np.stack([hist[int(r)][c] for r, c in zip(rows, cols)]), stored["hist"]), "histograms differ from the stored ones"
 
 
 def test_one_core_affinity_still_correct(tmp_path):
