@@ -380,7 +380,10 @@ def svm_cv(y, splits, kmat=None, problem=None, C=1.0, eps=1e-3, max_iter=-1, lib
     alpha = np.zeros(len(tr))
     fits = (gkmb200_svm_fit * len(splits))()
     if kmat is not None:
-        kmat = np.ascontiguousarray(kmat, np.float64)
+        # rows of contiguous doubles are passed in place, with ld = the row stride (a view of a larger buffer: ld > n)
+        if not (isinstance(kmat, np.ndarray) and kmat.dtype == np.float64 and kmat.ndim == 2 and kmat.strides[1] == 8
+                and kmat.strides[0] % 8 == 0 and kmat.strides[0] >= 8 * kmat.shape[1]):
+            kmat = np.ascontiguousarray(kmat, np.float64)
         n, kptr, ld, h = kmat.shape[0], kmat.ctypes.data, kmat.strides[0] // 8, None
     else:
         n, kptr, ld, h = problem.n, None, 0, problem.h

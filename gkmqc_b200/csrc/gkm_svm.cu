@@ -316,6 +316,12 @@ int gkm_svm_run(const double *d_K, long long ld, int n, int ntasks, const gkm_sv
     }
     for (long long k = 0; k < ntrain; k++) if (train_idx[k] < 0 || train_idx[k] >= n || (train_y[k] != 1 && train_y[k] != -1)) { gkm_set_error("svm: bad training index or label"); return 1; }
     for (long long k = 0; k < ntest; k++) if (test_idx[k] < 0 || test_idx[k] >= n) { gkm_set_error("svm: bad test index"); return 1; }
+    /* one class only: the solver would stop at once and rho = (ub + lb) / 2 would be infinite */
+    for (int t = 0; t < ntasks; t++) {
+        int npos = 0;
+        for (int k = 0; k < tasks[t].ntrain; k++) npos += train_y[tasks[t].train_off + k] > 0;
+        if (npos == 0 || npos == tasks[t].ntrain) { gkm_set_error("svm task %d: the training labels must contain both +1 and -1", t); return 1; }
+    }
     if (max_iter < 0) max_iter = 10000000 > 100 * lmax ? 10000000 : 100 * lmax; /* libsvm's own ceiling */
 
     gkm_svm_task *d_tasks = NULL; int *d_tr = NULL, *d_te = NULL; signed char *d_y = NULL;

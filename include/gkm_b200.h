@@ -93,7 +93,8 @@ int gkmb200_decision_values(gkmb200_problem *p, int row0, int nrows, int col0, i
 /* One fit = one (train, test) split, like one call of _svm_train_proc in scripts/gkmsvm.py:104-122.
  * train_idx / test_idx hold sequence ids; the training ids of a fit must be grouped by class, label 0 (the
  * negatives) first -- the order libsvm gives them (svm_group_classes) -- and train_y must be +1 for that first
- * class and -1 for the other (libsvm's sub-problem labels).  gkmqc_b200/driver.py prepares both from 0/1 labels. */
+ * class and -1 for the other (libsvm's sub-problem labels); a fit whose training labels lack either is rejected.
+ * gkmqc_b200/driver.py prepares both from 0/1 labels. */
 typedef struct gkmb200_svm_task {
     long long train_off, test_off; /* first entry of this fit in train_idx / train_y and in test_idx / scores */
     int ntrain, ntest;
