@@ -38,14 +38,15 @@
  * Pipe balance (sm_100, measured, DESIGN.md): LOP3/SHF/IADD3 issue at 64
  * lanes/clk/SM on the ALU pipe, IMAD at 64 on the FMA pipe, POPC at 16 on the XU
  * pipe.  The counter is LOP3-only, so the ALU pipe is the bound; the XU pipe comes
- * second.  FLAVOR bits: GKM_F_RARE_BINS takes the two rarest bins (count <= 1 when
- * NB = 4) off the straight-line path (no POPC for them; a loop entered for ~1 % of
- * the warp steps), GKM_F_IMAD_ACC accumulates the counters through IMAD.
+ * second.  The unweighted NB = 4 kernel therefore takes its two rarest bins (count
+ * <= 1) off the straight-line path (no POPC for them; a loop entered for ~1 % of the
+ * warp steps), and so does the unweighted NB = 8 kernel for d = 4 (D4, counts <= 2).
  */
 #ifndef GKM_BITSLICE_H_INCLUDED
 #define GKM_BITSLICE_H_INCLUDED
 
 #include <stdint.h>
+#include <type_traits>
 
 #if defined(__CUDACC__)
 #define GKM_HD __host__ __device__ __forceinline__
@@ -55,12 +56,19 @@
 #define GKM_HDM inline
 #endif
 
-enum { GKM_F_ONE_BODY = 1, GKM_F_RARE_BINS = 2, GKM_F_IMAD_ACC = 4 };
+/* The instance of the lane code that serves a problem with d mismatches: NB = gkm_diag_nb(d) bins; one instance per
+ * (L, NB, WEIGHTED), and for the unweighted NB = 8 problems with d = 4 (the top of the BASELINE sweep) a second one with
+ * D4 set.  gkm_diag_instance<NB, WEIGHTED>(d, f) calls f(std::bool_constant<D4>()).  The kernel launcher
+ * (gkm_diag_inst.cu) and the CPU emulator both choose through these, so the emulator runs what the device runs. */
+constexpr int gkm_diag_nb(int d) { return d < 4 ? 4 : d < 8 ? 8 : 16; }
 
-#if defined(__CUDACC__)
-/* the constant 1 behind a constant-bank load, so that ptxas keeps IMAD for the accumulation */
-static __constant__ uint32_t gkm_one_c[1] = { 1u };
-#endif
+template <int NB, bool WEIGHTED, class F>
+auto gkm_diag_instance(int d, F f)
+{
+    if constexpr (NB == 8 && !WEIGHTED)
+        if (d == 4) return f(std::true_type());
+    return f(std::false_type());
+}
 
 /* query-side records of a PAIR of queries for one position e (two 16-byte broadcast loads) */
 struct alignas(16) gkm_apos2 {
@@ -98,18 +106,6 @@ GKM_HD int gkm_ffs0(uint32_t x) /* index of lowest set bit, x != 0 */
 #else
     return __builtin_ctz(x);
 #endif
-}
-
-template <int FLAVOR>
-GKM_HD void gkm_acc_add(int32_t &acc, int v)
-{
-#if defined(__CUDA_ARCH__)
-    if constexpr ((FLAVOR & GKM_F_IMAD_ACC) != 0) {
-        acc = (int32_t) ((uint32_t) v * gkm_one_c[0] + (uint32_t) acc);
-        return;
-    }
-#endif
-    acc += v;
 }
 
 constexpr int gkm_nplanes(int maxv) { return maxv >= 16 ? 5 : maxv >= 8 ? 4 : maxv >= 4 ? 3 : maxv >= 2 ? 2 : 1; }
@@ -175,12 +171,12 @@ GKM_HD uint32_t gkm_bin_mask(const gkm_win_state<L, INV> &st, uint32_t hit)
     return r;
 }
 
-template <int L, int INV, int LB, int FLAVOR, int V0, int V1>
+template <int L, int INV, int LB, int V0, int V1>
 GKM_HD void gkm_bins_popc(const gkm_win_state<L, INV> &st, uint32_t hit, int32_t *acc)
 {
     if constexpr (V0 < V1) {
-        if constexpr (V0 <= L) gkm_acc_add<FLAVOR>(acc[V0], gkm_popc(gkm_bin_mask<L, INV, LB, V0>(st, hit)));
-        gkm_bins_popc<L, INV, LB, FLAVOR, V0 + 1, V1>(st, hit, acc);
+        if constexpr (V0 <= L) acc[V0] += gkm_popc(gkm_bin_mask<L, INV, LB, V0>(st, hit));
+        gkm_bins_popc<L, INV, LB, V0 + 1, V1>(st, hit, acc);
     }
 }
 
@@ -207,15 +203,15 @@ GKM_HD void gkm_bins_weighted(const gkm_win_state<L, INV> &st, uint32_t hit, uin
 }
 
 /* binning of one query at one step */
-template <int L, int INV, int NB, bool WEIGHTED, int FLAVOR>
+template <int L, int INV, int NB, bool WEIGHTED, bool D4>
 GKM_HD void gkm_bins(const gkm_win_state<L, INV> &st, uint32_t hit, uint32_t wa, const uint8_t *wend,
                      int jbase, int P, int32_t *acc)
 {
     constexpr int LB = gkm_log2nb<NB>::v;
     if constexpr (WEIGHTED) {
         gkm_bins_weighted<L, INV, LB>(st, hit, wa, wend, jbase, P, acc);
-    } else if constexpr ((FLAVOR & GKM_F_RARE_BINS) != 0 && NB == 4) {
-        gkm_bins_popc<L, INV, LB, FLAVOR, 2, 4>(st, hit, acc); /* counts 2 and 3: ~99 % of all hits */
+    } else if constexpr (NB == 4) {
+        gkm_bins_popc<L, INV, LB, 2, 4>(st, hit, acc);        /* counts 2 and 3: ~99 % of all hits */
         uint32_t rare = hit & ~st.plane(1);                   /* counts 0 and 1 (plane 1 is stored inverted) */
         if (rare) {
             /* a loop, so that the compiler keeps this off the straight-line path (a real branch,
@@ -226,7 +222,7 @@ GKM_HD void gkm_bins(const gkm_win_state<L, INV> &st, uint32_t hit, uint32_t wa,
                 if (st.plane(0) & low) acc[1] += 1; else acc[0] += 1;
             } while (rare);
         }
-    } else if constexpr ((FLAVOR & GKM_F_RARE_BINS) != 0 && NB == 8 && ((FLAVOR >> 8) & 15) == 4) {
+    } else if constexpr (NB == 8 && D4) {
         /* d = 4 known at compile time: counts 5..7 are not wanted at all, 4 and 3 hold ~99 % of the
          * wanted hits, 0..2 take the rare path.  2 POPC per step instead of 8. */
         const uint32_t p0 = st.plane(0), p1 = st.plane(1), p2 = st.plane(2);
@@ -234,8 +230,8 @@ GKM_HD void gkm_bins(const gkm_win_state<L, INV> &st, uint32_t hit, uint32_t wa,
         const uint32_t low = hit & ~p2;
         const uint32_t b3 = low & p1 & p0;
         uint32_t rare = low & ~(p1 & p0);
-        gkm_acc_add<FLAVOR>(acc[4], gkm_popc(b4));
-        gkm_acc_add<FLAVOR>(acc[3], gkm_popc(b3));
+        acc[4] += gkm_popc(b4);
+        acc[3] += gkm_popc(b3);
         if (rare) {
             do {
                 const uint32_t lowbit = rare & (0u - rare);
@@ -244,16 +240,12 @@ GKM_HD void gkm_bins(const gkm_win_state<L, INV> &st, uint32_t hit, uint32_t wa,
             } while (rare);
         }
     } else {
-        gkm_bins_popc<L, INV, LB, FLAVOR, 0, NB>(st, hit, acc);
+        gkm_bins_popc<L, INV, LB, 0, NB>(st, hit, acc);
     }
 }
 
-/* which plane to keep complemented for a given kernel flavour */
-template <int NB, bool WEIGHTED, int FLAVOR>
-struct gkm_inv_plane { static constexpr int v = (!WEIGHTED && NB == 4 && (FLAVOR & GKM_F_RARE_BINS) != 0) ? 1 : -1; };
-
 /* steps S0..S1-1 of one half chunk (16 positions) for the query pair */
-template <int L, int INV, int NB, bool WEIGHTED, int FLAVOR, bool USE_VA, int S0, int S1>
+template <int L, int INV, int NB, bool WEIGHTED, bool D4, bool USE_VA, int S0, int S1>
 GKM_HD void gkm_diag_steps(gkm_win_state<L, INV> &st0, gkm_win_state<L, INV> &st1,
                            const gkm_apos2 *ap, const gkm_aaux2 *ax,
                            uint32_t lo0, uint32_t hi0, uint32_t lo1, uint32_t hi1, uint32_t loE, uint32_t hiE,
@@ -275,11 +267,11 @@ GKM_HD void gkm_diag_steps(gkm_win_state<L, INV> &st0, gkm_win_state<L, INV> &st
         }
         const uint32_t h0 = gkm_hit_word<L, INV, LB>(st0, v0), h1 = gkm_hit_word<L, INV, LB>(st1, v1);
         if (!WEIGHTED || (h0 | h1) != 0u) { /* weighted: ONE divergent region per step for both queries */
-            gkm_bins<L, INV, NB, WEIGHTED, FLAVOR>(st0, h0, w0, wend, jbase + S0, P, acc0);
-            gkm_bins<L, INV, NB, WEIGHTED, FLAVOR>(st1, h1, w1, wend, jbase + S0, P, acc1);
+            gkm_bins<L, INV, NB, WEIGHTED, D4>(st0, h0, w0, wend, jbase + S0, P, acc0);
+            gkm_bins<L, INV, NB, WEIGHTED, D4>(st1, h1, w1, wend, jbase + S0, P, acc1);
         }
-        gkm_diag_steps<L, INV, NB, WEIGHTED, FLAVOR, USE_VA, S0 + 1, S1>(st0, st1, ap, ax, lo0, hi0, lo1, hi1, loE, hiE,
-                                                                     wend, jbase, P, acc0, acc1);
+        gkm_diag_steps<L, INV, NB, WEIGHTED, D4, USE_VA, S0 + 1, S1>(st0, st1, ap, ax, lo0, hi0, lo1, hi1, loE, hiE,
+                                                                 wend, jbase, P, acc0, acc1);
     }
 }
 
@@ -288,13 +280,14 @@ GKM_HD void gkm_diag_steps(gkm_win_state<L, INV> &st0, gkm_win_state<L, INV> &st
  *              a query of length 0 is a dummy)
  *   C0,C1,E    target bit planes (both strands, circular) and valid-window-end plane, Wc words each
  *   wend       WEIGHTED: target weights by window end position, 32*Wc bytes
- *   acc0/acc1  NB counters per query, added to                                              */
-template <int L, int NB, bool WEIGHTED, int FLAVOR>
+ *   acc0/acc1  NB counters per query, added to
+ *   D4         unweighted NB = 8 only: d = 4, counts above 4 are not wanted (gkm_diag_instance)        */
+template <int L, int NB, bool WEIGHTED, bool D4>
 GKM_HD void gkm_diag_lane(const gkm_apos2 *apos, const gkm_aaux2 *aaux, int len0, int len1,
                           const uint32_t *C0, const uint32_t *C1, const uint32_t *E, int Wc, int q,
                           const uint8_t *wend, int32_t *acc0, int32_t *acc1)
 {
-    constexpr int INV = gkm_inv_plane<NB, WEIGHTED, FLAVOR>::v;
+    constexpr int INV = (!WEIGHTED && NB == 4) ? 1 : -1; /* the rare-bin test of the unweighted NB = 4 kernel wants ~p1 */
     gkm_win_state<L, INV> st0, st1;
     st0.clear();
     st1.clear();
@@ -319,14 +312,13 @@ GKM_HD void gkm_diag_lane(const gkm_apos2 *apos, const gkm_aaux2 *aaux, int len0
             const uint32_t lo0 = half ? gkm_funnel(a0, b0, 16) : a0, hi0 = half ? gkm_funnel(b0, c0, 16) : b0;
             const uint32_t lo1 = half ? gkm_funnel(a1, b1, 16) : a1, hi1 = half ? gkm_funnel(b1, c1, 16) : b1;
             const uint32_t loE = half ? gkm_funnel(aE, bE, 16) : aE, hiE = half ? gkm_funnel(bE, cE, 16) : bE;
-            /* GKM_F_ONE_BODY: a single body that always pays for the AND (half the code, for the I-cache) */
-            const bool need_va = ((FLAVOR & GKM_F_ONE_BODY) != 0) || (e0 < L - 1) || (e0 + 16 > lmin);
+            const bool need_va = (e0 < L - 1) || (e0 + 16 > lmin);
             if (need_va)
-                gkm_diag_steps<L, INV, NB, WEIGHTED, FLAVOR, true, 0, 16>(st0, st1, apos + e0, aaux + e0, lo0, hi0, lo1, hi1, loE, hiE,
-                                                                      wend, jbase, P, acc0, acc1);
+                gkm_diag_steps<L, INV, NB, WEIGHTED, D4, true, 0, 16>(st0, st1, apos + e0, aaux + e0, lo0, hi0, lo1, hi1, loE, hiE,
+                                                                  wend, jbase, P, acc0, acc1);
             else
-                gkm_diag_steps<L, INV, NB, WEIGHTED, FLAVOR, false, 0, 16>(st0, st1, apos + e0, aaux + e0, lo0, hi0, lo1, hi1, loE, hiE,
-                                                                       wend, jbase, P, acc0, acc1);
+                gkm_diag_steps<L, INV, NB, WEIGHTED, D4, false, 0, 16>(st0, st1, apos + e0, aaux + e0, lo0, hi0, lo1, hi1, loE, hiE,
+                                                                   wend, jbase, P, acc0, acc1);
             jbase += 16;
             if (jbase >= P) jbase -= P;
         }

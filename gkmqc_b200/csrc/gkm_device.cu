@@ -42,24 +42,24 @@
     } while (0)
 
 extern "C" {
-const void *gkm_diag_fn_L2(int, int, int, int);  const void *gkm_diag_fn_L3(int, int, int, int);  const void *gkm_diag_fn_L4(int, int, int, int);
-const void *gkm_diag_fn_L5(int, int, int, int);  const void *gkm_diag_fn_L6(int, int, int, int);  const void *gkm_diag_fn_L7(int, int, int, int);
-const void *gkm_diag_fn_L8(int, int, int, int);  const void *gkm_diag_fn_L9(int, int, int, int);  const void *gkm_diag_fn_L10(int, int, int, int);
-const void *gkm_diag_fn_L11(int, int, int, int); const void *gkm_diag_fn_L12(int, int, int, int); const void *gkm_diag_fn_L13(int, int, int, int);
-const void *gkm_diag_fn_L14(int, int, int, int); const void *gkm_diag_fn_L15(int, int, int, int); const void *gkm_diag_fn_L16(int, int, int, int);
+const void *gkm_diag_fn_L2(int, int, int);  const void *gkm_diag_fn_L3(int, int, int);  const void *gkm_diag_fn_L4(int, int, int);
+const void *gkm_diag_fn_L5(int, int, int);  const void *gkm_diag_fn_L6(int, int, int);  const void *gkm_diag_fn_L7(int, int, int);
+const void *gkm_diag_fn_L8(int, int, int);  const void *gkm_diag_fn_L9(int, int, int);  const void *gkm_diag_fn_L10(int, int, int);
+const void *gkm_diag_fn_L11(int, int, int); const void *gkm_diag_fn_L12(int, int, int); const void *gkm_diag_fn_L13(int, int, int);
+const void *gkm_diag_fn_L14(int, int, int); const void *gkm_diag_fn_L15(int, int, int); const void *gkm_diag_fn_L16(int, int, int);
 }
 
-static const void *diag_fn(int L, int nb, int weighted, int d, int flavor)
+static const void *diag_fn(int L, int nb, int weighted, int d)
 {
     switch (L) {
-        case 2: return gkm_diag_fn_L2(nb, weighted, d, flavor);   case 3: return gkm_diag_fn_L3(nb, weighted, d, flavor);
-        case 4: return gkm_diag_fn_L4(nb, weighted, d, flavor);   case 5: return gkm_diag_fn_L5(nb, weighted, d, flavor);
-        case 6: return gkm_diag_fn_L6(nb, weighted, d, flavor);   case 7: return gkm_diag_fn_L7(nb, weighted, d, flavor);
-        case 8: return gkm_diag_fn_L8(nb, weighted, d, flavor);   case 9: return gkm_diag_fn_L9(nb, weighted, d, flavor);
-        case 10: return gkm_diag_fn_L10(nb, weighted, d, flavor); case 11: return gkm_diag_fn_L11(nb, weighted, d, flavor);
-        case 12: return gkm_diag_fn_L12(nb, weighted, d, flavor); case 13: return gkm_diag_fn_L13(nb, weighted, d, flavor);
-        case 14: return gkm_diag_fn_L14(nb, weighted, d, flavor); case 15: return gkm_diag_fn_L15(nb, weighted, d, flavor);
-        case 16: return gkm_diag_fn_L16(nb, weighted, d, flavor);
+        case 2: return gkm_diag_fn_L2(nb, weighted, d);   case 3: return gkm_diag_fn_L3(nb, weighted, d);
+        case 4: return gkm_diag_fn_L4(nb, weighted, d);   case 5: return gkm_diag_fn_L5(nb, weighted, d);
+        case 6: return gkm_diag_fn_L6(nb, weighted, d);   case 7: return gkm_diag_fn_L7(nb, weighted, d);
+        case 8: return gkm_diag_fn_L8(nb, weighted, d);   case 9: return gkm_diag_fn_L9(nb, weighted, d);
+        case 10: return gkm_diag_fn_L10(nb, weighted, d); case 11: return gkm_diag_fn_L11(nb, weighted, d);
+        case 12: return gkm_diag_fn_L12(nb, weighted, d); case 13: return gkm_diag_fn_L13(nb, weighted, d);
+        case 14: return gkm_diag_fn_L14(nb, weighted, d); case 15: return gkm_diag_fn_L15(nb, weighted, d);
+        case 16: return gkm_diag_fn_L16(nb, weighted, d);
         default: return NULL;
     }
 }
@@ -369,19 +369,17 @@ static int launch_hist(const gkmb200_problem *p, const gkm_image *im, gkm_gpu *g
         if (variant_out) *variant_out = variant;
         return launch_index(p, im, g, kp, st);
     }
-    const int forced_ta = gkm_opt_tile_rows();
     const void *fn = NULL;
     unsigned smem = 0;
     if (variant == GKM_KERNEL_DIAG) {
-        const int nb = (p->param.d < 4) ? 4 : (p->param.d < 8) ? 8 : 16;
-        fn = diag_fn(p->param.L, nb, p->weighted, p->param.d, gkm_opt_diag_flavor());
+        const int nb = gkm_diag_nb(p->param.d);
+        fn = diag_fn(p->param.L, nb, p->weighted, p->param.d);
         if (!fn) { gkm_set_error("no diag kernel for L=%d", p->param.L); return 1; }
         /* TB = 32 makes the lane-task count of a uniform-length tile a multiple of the warp size */
         static const int cand[][2] = { {8, 32}, {4, 32}, {4, 16}, {2, 16}, {2, 8}, {2, 4}, {2, 2}, {2, 1} }; /* TA even: queries go in pairs */
         int chosen = -1;
         for (int pass = 0; pass < 2 && chosen < 0; pass++)
             for (unsigned i = 0; i < sizeof(cand) / sizeof(cand[0]); i++) {
-                if (forced_ta && cand[i][0] != forced_ta && pass == 0) continue;
                 unsigned s = gkm_diag_layout(p->Wmax, p->Wa, cand[i][0], cand[i][1], nb, p->weighted).total;
                 if (s <= (pass == 0 ? 74u * 1024u : 220u * 1024u)) { chosen = (int) i; smem = s; break; }
             }
@@ -1291,10 +1289,8 @@ extern "C" int gkm_dev_compute(gkmb200_problem *p, int row0, int nrows, int col0
     p->stats.launches = 0;
     /* Chunks are issued in ascending row order.  Round 1 issued the widest rows first so that the call ends on the smallest
      * copy; that saves < 1 ms at 10k and costs the weighted kernel types dearly (wgkm 10k x 300 bp: device span 59.0
-     * against 47.3 ms; gkmQC's default, 600-bp windows: 312 against 237 ms; unit weights: equal) -- tools/order_ab.py.
-     * GKM_CHUNK_ORDER=desc brings the old order back (A/B knob). */
-    const char *ord = getenv("GKM_CHUNK_ORDER");
-    const int desc = lower && ord && ord[0] == 'd';
+     * against 47.3 ms; gkmQC's default, 600-bp windows: 312 against 237 ms; unit weights: equal) --
+     * profiles/r2_chunk_order_carveout_ab.txt. */
     int rc = upload_locked(p, 0);
     const double t_up = now_ms();
     if (!rc) rc = choose_variant(p, row0, nrows, col0, ncols, lower);
@@ -1317,10 +1313,8 @@ extern "C" int gkm_dev_compute(gkmb200_problem *p, int row0, int nrows, int col0
             gkm_job job;
             memset(&job, 0, sizeof(job));
             job.p = p; job.chunks = chunks; job.owned = owned;
-            for (int i = 0; i < nchunks; i++) {
-                const int c = desc ? nchunks - 1 - i : i;
+            for (int c = 0; c < nchunks; c++)
                 if (gkm_chunk_owner(c, nchunks, p->shard_world) == p->shard_rank) owned[job.nowned++] = c;
-            }
             job.row0 = row0; job.col0 = col0; job.ncols = ncols; job.lower = lower;
             job.out = out; job.ld = ld; job.rows = rows; job.hist = hist;
             /* the host threads that scatter finished chunks are shared by the GPUs of the call: each device thread

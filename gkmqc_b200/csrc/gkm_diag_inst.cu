@@ -1,6 +1,6 @@
 /* gkm_diag_inst.cu -- instantiates the bit-sliced kernel for ONE word length.
  * Compiled once per L = 2..16 with -DGKM_INST_L=<L> (see Makefile) so that the
- * specialisations (15 L x {4,8,16} bins x {plain, weighted}) build in parallel. */
+ * specialisations (15 L x {4,8,16} bins x {plain, weighted}, + d = 4) build in parallel. */
 #include "gkm_diag_kernel.cuh"
 
 #ifndef GKM_INST_L
@@ -10,39 +10,18 @@
 #define GKM_CAT2(a, b) a##b
 #define GKM_CAT(a, b) GKM_CAT2(a, b)
 
-#ifndef GKM_DIAG_DEFAULT_FLAVOR
-#define GKM_DIAG_DEFAULT_FLAVOR 0
-#endif
-
-template <int L, int F>
-static const void *pick(int nb, int weighted, int d)
+template <int NB, bool WEIGHTED>
+static const void *pick(int d)
 {
-    constexpr int FW = F & ~GKM_F_RARE_BINS; /* the rare-bin path exists for the plain kernels only */
-    if (nb == 4) return weighted ? (const void *) gkm_diag_kernel<L, 4, true, FW> : (const void *) gkm_diag_kernel<L, 4, false, F>;
-    if (nb == 8) {
-        if (weighted) return (const void *) gkm_diag_kernel<L, 8, true, FW>;
-        /* d = 4 (the top of the BASELINE sweep) has its own specialisation: flavor bits 8..11 carry d */
-        if (d == 4 && (F & GKM_F_RARE_BINS) != 0 && L >= 4) return (const void *) gkm_diag_kernel<L, 8, false, (F | (4 << 8))>;
-        return (const void *) gkm_diag_kernel<L, 8, false, FW>;
-    }
-    if (nb == 16) return weighted ? (const void *) gkm_diag_kernel<L, 16, true, FW> : (const void *) gkm_diag_kernel<L, 16, false, FW>;
-    return nullptr;
+    return gkm_diag_instance<NB, WEIGHTED>(d, [](auto d4) {
+        return (const void *) gkm_diag_kernel<GKM_INST_L, NB, WEIGHTED, decltype(d4)::value>;
+    });
 }
 
-/* flavor < 0: the default for this build.  Other flavors exist only where GKM_INST_FLAVORS is set
- * (the benchmark word length), for A/B measurements on the device. */
-extern "C" const void *GKM_CAT(gkm_diag_fn_L, GKM_INST_L)(int nb, int weighted, int d, int flavor)
+extern "C" const void *GKM_CAT(gkm_diag_fn_L, GKM_INST_L)(int nb, int weighted, int d)
 {
-    constexpr int L = GKM_INST_L;
-#ifdef GKM_INST_FLAVORS
-    if (flavor >= 0 && nb == 4 && !weighted) {
-        switch (flavor & 7) {
-            case 0: return (const void *) gkm_diag_kernel<L, 4, false, 0>;
-            case 2: return (const void *) gkm_diag_kernel<L, 4, false, 2>;
-            case 6: return (const void *) gkm_diag_kernel<L, 4, false, 6>;
-        }
-    }
-#endif
-    (void) flavor;
-    return pick<L, GKM_DIAG_DEFAULT_FLAVOR>(nb, weighted, d);
+    if (nb == 4) return weighted ? pick<4, true>(d) : pick<4, false>(d);
+    if (nb == 8) return weighted ? pick<8, true>(d) : pick<8, false>(d);
+    if (nb == 16) return weighted ? pick<16, true>(d) : pick<16, false>(d);
+    return nullptr;
 }

@@ -77,7 +77,7 @@ __device__ __forceinline__ void gkm_emit_entry(const gkm_kparams &p, int a_g, in
     if (p.decision) atomicAdd(p.decision + (a_g - p.row_base), p.alpha[b_g - p.col_base] * v);
 }
 
-template <int L, int NB, bool WEIGHTED, int FLAVOR>
+template <int L, int NB, bool WEIGHTED, bool D4>
 __global__ void __launch_bounds__(GKM_DIAG_THREADS)
 gkm_diag_kernel(const __grid_constant__ gkm_kparams p)
 {
@@ -196,8 +196,8 @@ gkm_diag_kernel(const __grid_constant__ gkm_kparams p)
         int32_t acc0[NB], acc1[NB];
 #pragma unroll
         for (int m = 0; m < NB; m++) { acc0[m] = 0; acc1[m] = 0; }
-        gkm_diag_lane<L, NB, WEIGHTED, FLAVOR>(sAp + (size_t) pi * 32 * WA, sAx + (size_t) pi * 32 * WA, len0, len1,
-                                               C0, C1, E, Wc, active ? q : 0, wendp, acc0, acc1);
+        gkm_diag_lane<L, NB, WEIGHTED, D4>(sAp + (size_t) pi * 32 * WA, sAx + (size_t) pi * 32 * WA, len0, len1,
+                                           C0, C1, E, Wc, active ? q : 0, wendp, acc0, acc1);
         if (active) {
             int32_t *h0 = sH + ((2 * pi) * TB + b_l) * NB;
             int32_t *h1 = sH + ((2 * pi + 1) * TB + b_l) * NB;

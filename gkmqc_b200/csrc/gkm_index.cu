@@ -13,7 +13,6 @@
  *                         (ascending-m sum, one division, no FMA; libgkm.c:576-582,1169-1179).
  */
 #include <cuda_runtime.h>
-#include <stdlib.h>
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
 
@@ -773,7 +772,6 @@ int gkm_idx_rows(const gkm_kparams *kp, const gkm_idx_rowargs *ra, int weighted,
     /* weighted types on input with repeats (long-tailed rows): one CTA per SM (everything-mixed workload of
      * tools/nonuniform.py: 80 against 95 ms; uniform input: 50.4 against 47.4 ms the other way round) */
     if (weighted && ra->skew > GKM_IDX_SKEW_ONE_CTA) two = false;
-    { const char *e = getenv("GKM_IDX_MINB"); if (e) two = atoi(e) == 2; } /* A/B knob */
     if ((ra->fmt == GKM_IDX_FMT_C16 && weighted) || (ra->fmt == GKM_IDX_FMT_W20 && !weighted)) { gkm_set_error("index slot format does not match the kernel type"); return 1; }
     const void *fn;
 #define GKM_IDX_PICK(W, F) (range ? (two ? (const void *) gkm_index_rows_kernel<W, true, F, 2> : (const void *) gkm_index_rows_kernel<W, true, F, 1>) \
@@ -784,17 +782,14 @@ int gkm_idx_rows(const gkm_kparams *kp, const gkm_idx_rowargs *ra, int weighted,
     else fn = GKM_IDX_PICK(false, GKM_IDX_FMT_P32);
 #undef GKM_IDX_PICK
     cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
-    {   /* Ask for no more shared memory per SM than this launch's CTAs need: what is left is L1, where the in-flight slot
-         * probes live.  Without the hint the split of an earlier, larger launch can stay in force (rows issued widest
-         * first ran the weighted build 25 % slower than ascending: tools/order_ab.py).  GKM_IDX_CARVEOUT=0: no hint. */
-        static int use = -1;
-        if (use < 0) { const char *c = getenv("GKM_IDX_CARVEOUT"); use = !(c && c[0] == '0'); }
-        if (use && e == cudaSuccess) {
-            const unsigned per_sm = (two ? 2u : 1u) * (smem + 1280u);
-            int pct = (int) ((per_sm * 100u + 228u * 1024u - 1u) / (228u * 1024u));
-            if (pct > 100) pct = 100;
-            e = cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
-        }
+    /* Ask for no more shared memory per SM than this launch's CTAs need: what is left is L1, where the in-flight slot
+     * probes live.  Without the hint the split of an earlier, larger launch can stay in force (rows issued widest first
+     * ran the weighted build 25 % slower than ascending: profiles/r2_chunk_order_carveout_ab.txt). */
+    if (e == cudaSuccess) {
+        const unsigned per_sm = (two ? 2u : 1u) * (smem + 1280u);
+        int pct = (int) ((per_sm * 100u + 228u * 1024u - 1u) / (228u * 1024u));
+        if (pct > 100) pct = 100;
+        e = cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
     }
     if (e == cudaSuccess) {
         void *args[] = { (void *) kp, (void *) ra };

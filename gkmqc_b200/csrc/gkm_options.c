@@ -20,8 +20,6 @@ static int g_loaded = 0;
 static int g_kernel = GKM_KERNEL_AUTO;
 static int g_max_L = 12;
 static int g_chunk_mb = 128; /* 50k x 50k: 686 ms per pass with 64 MB chunks (one wave of 148 rows each), 671 with 128, 669 with 256 */
-static int g_tile_rows = 0;
-static int g_diag_flavor = -1;
 static int g_index_cols = 0;
 static int g_index_wide = 0;
 static int g_pack_host = 0;
@@ -46,19 +44,15 @@ static void load_env(void)
     if ((v = getenv("GKM_KERNEL")) != NULL) parse_kernel(v, &g_kernel);
     if ((v = getenv("GKM_MAX_L")) != NULL) { int x = atoi(v); if (x == 12 || x == 16) g_max_L = x; }
     if ((v = getenv("GKM_CHUNK_MB")) != NULL) { int x = atoi(v); if (x >= 1 && x <= 4096) g_chunk_mb = x; }
-    if ((v = getenv("GKM_DIAG_FLAVOR")) != NULL) { int x = atoi(v); if (x >= -1 && x <= 7) g_diag_flavor = x; }
     if ((v = getenv("GKM_INDEX_COLS")) != NULL) { int x = atoi(v); if (x >= 32) g_index_cols = x & ~31; }
     if ((v = getenv("GKM_INDEX_WIDE")) != NULL) g_index_wide = atoi(v) != 0;
     if ((v = getenv("GKM_PACK")) != NULL) g_pack_host = !strcmp(v, "host");
     if ((v = getenv("GKM_INDEX_SPLIT")) != NULL) g_index_greedy = !strcmp(v, "greedy") ? 1 : !strcmp(v, "equal") ? 0 : -1;
-    if ((v = getenv("GKM_TILE_ROWS")) != NULL) { int x = atoi(v); if (x >= 1 && x <= 16) g_tile_rows = x; }
 }
 
 int gkm_opt_kernel(void) { load_env(); return g_kernel; }
 int gkm_opt_max_L(void) { load_env(); return g_max_L; }
 int gkm_opt_chunk_mb(void) { load_env(); return g_chunk_mb; }
-int gkm_opt_tile_rows(void) { load_env(); return g_tile_rows; }
-int gkm_opt_diag_flavor(void) { load_env(); return g_diag_flavor; }
 int gkm_opt_index_cols(void) { load_env(); return g_index_cols; }
 int gkm_opt_index_wide(void) { load_env(); return g_index_wide; }
 int gkm_opt_pack_host(void) { load_env(); return g_pack_host; }
@@ -83,11 +77,6 @@ int gkmb200_set_option(const char *key, const char *value)
         g_chunk_mb = x;
         return 0;
     }
-    if (!strcmp(key, "diag_flavor")) { /* A/B switch for the pipe-balancing variants of the diag kernel */
-        if (x < -1 || x > 7) { gkm_set_error("diag_flavor out of range"); return 1; }
-        g_diag_flavor = x;
-        return 0;
-    }
     if (!strcmp(key, "index_cols")) { /* upper bound of the columns of one index block (0 = what fits shared memory) */
         if (x != 0 && x < 32) { gkm_set_error("index_cols must be 0 or >= 32"); return 1; }
         g_index_cols = x & ~31;
@@ -105,11 +94,6 @@ int gkmb200_set_option(const char *key, const char *value)
     if (!strcmp(key, "index_split")) { /* equal: blocks of equal size; greedy: full blocks first, the rest last; auto: per call */
         if (strcmp(value, "equal") && strcmp(value, "greedy") && strcmp(value, "auto")) { gkm_set_error("index_split must be equal, greedy or auto"); return 1; }
         g_index_greedy = !strcmp(value, "greedy") ? 1 : !strcmp(value, "equal") ? 0 : -1;
-        return 0;
-    }
-    if (!strcmp(key, "tile_rows")) {
-        if (x < 0 || x > 16) { gkm_set_error("tile_rows out of range"); return 1; }
-        g_tile_rows = x;
         return 0;
     }
     gkm_set_error("unknown option %s", key);

@@ -7,8 +7,6 @@ enum { GKM_KERNEL_AUTO = 0, GKM_KERNEL_LMER = 1, GKM_KERNEL_DIAG = 2, GKM_KERNEL
 int gkm_opt_kernel(void);
 int gkm_opt_max_L(void);
 int gkm_opt_chunk_mb(void);
-int gkm_opt_tile_rows(void);
-int gkm_opt_diag_flavor(void);
 int gkm_opt_index_cols(void);
 int gkm_opt_index_wide(void);
 int gkm_opt_pack_host(void);

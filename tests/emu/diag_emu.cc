@@ -45,7 +45,7 @@ static void build_records(const gkmb200_problem *p, int L, int a0, int a1,
     }
 }
 
-template <int L, int NB, bool WEIGHTED, int FLAVOR>
+template <int L, int NB, bool WEIGHTED, bool D4>
 static void emu_pair(const gkmb200_problem *p, int a0, int a1, int b, int32_t *H0, int32_t *H1)
 {
     const int W = p->Wmax;
@@ -66,29 +66,25 @@ static void emu_pair(const gkmb200_problem *p, int a0, int a1, int b, int32_t *H
         we = wext.data();
     }
     for (int q = 0; q < Wc; q++)
-        gkm_diag_lane<L, NB, WEIGHTED, FLAVOR>(apos.data(), aaux.data(), len[0], len[1], pb, pb + W, pb + 2 * W, Wc, q, we, acc0, acc1);
+        gkm_diag_lane<L, NB, WEIGHTED, D4>(apos.data(), aaux.data(), len[0], len[1], pb, pb + W, pb + 2 * W, Wc, q, we, acc0, acc1);
     for (int m = 0; m <= p->param.d; m++) { H0[m] = acc0[m]; if (H1) H1[m] = acc1[m]; }
 }
 
-static int g_flavor = 0;
-extern "C" void gkm_emu_set_flavor(int f) { g_flavor = f; }
-
-template <int L, int NB>
-static void emu_dispatch_w(const gkmb200_problem *p, int a0, int a1, int b, int32_t *H0, int32_t *H1)
+/* the instance the kernel launcher picks for the problem (gkm_diag_nb, gkm_diag_instance) */
+template <int L, int NB, bool WEIGHTED>
+static int emu_run(const gkmb200_problem *p, int a0, int a1, int b, int32_t *H0, int32_t *H1)
 {
-    if (p->weighted) emu_pair<L, NB, true, 0>(p, a0, a1, b, H0, H1);
-    else if (g_flavor & GKM_F_RARE_BINS) emu_pair<L, NB, false, GKM_F_RARE_BINS>(p, a0, a1, b, H0, H1);
-    else emu_pair<L, NB, false, 0>(p, a0, a1, b, H0, H1);
+    gkm_diag_instance<NB, WEIGHTED>(p->param.d, [&](auto d4) { emu_pair<L, NB, WEIGHTED, decltype(d4)::value>(p, a0, a1, b, H0, H1); });
+    return 0;
 }
 
 template <int L>
-static int emu_dispatch_nb(const gkmb200_problem *p, int a0, int a1, int b, int32_t *H0, int32_t *H1)
+static int emu_dispatch(const gkmb200_problem *p, int a0, int a1, int b, int32_t *H0, int32_t *H1)
 {
-    const int d = p->param.d;
-    if (d < 4) emu_dispatch_w<L, 4>(p, a0, a1, b, H0, H1);
-    else if (d < 8) emu_dispatch_w<L, 8>(p, a0, a1, b, H0, H1);
-    else emu_dispatch_w<L, 16>(p, a0, a1, b, H0, H1);
-    return 0;
+    const int nb = gkm_diag_nb(p->param.d);
+    if (nb == 4) return p->weighted ? emu_run<L, 4, true>(p, a0, a1, b, H0, H1) : emu_run<L, 4, false>(p, a0, a1, b, H0, H1);
+    if (nb == 8) return p->weighted ? emu_run<L, 8, true>(p, a0, a1, b, H0, H1) : emu_run<L, 8, false>(p, a0, a1, b, H0, H1);
+    return p->weighted ? emu_run<L, 16, true>(p, a0, a1, b, H0, H1) : emu_run<L, 16, false>(p, a0, a1, b, H0, H1);
 }
 
 /* histograms of the query pair (a0, a1) against target b; a1 < 0: single query */
@@ -96,7 +92,7 @@ extern "C" int gkm_emu_hist_pair(gkmb200_problem *p, int a0, int a1, int b, int3
 {
     if (gkm_pack_problem(p)) return 1;
     switch (p->param.L) {
-#define CASE(x) case x: return emu_dispatch_nb<x>(p, a0, a1, b, H0, H1);
+#define CASE(x) case x: return emu_dispatch<x>(p, a0, a1, b, H0, H1);
         CASE(2) CASE(3) CASE(4) CASE(5) CASE(6) CASE(7) CASE(8) CASE(9)
         CASE(10) CASE(11) CASE(12) CASE(13) CASE(14) CASE(15) CASE(16)
 #undef CASE

@@ -16,18 +16,14 @@ sizes = [int(a) for a in sys.argv[1:]] or [20000, 28288, 50000]
 res = {}
 
 
-def timed(n, split, cols=0, minb=None, kt=2, L=11, k=7, d=3):
+def timed(n, split, cols=0, kt=2, L=11, k=7, d=3):
     capi.set_option("index_split", split)
     capi.set_option("index_cols", cols)
-    if minb is None:
-        os.environ.pop("GKM_IDX_MINB", None)
-    else:
-        os.environ["GKM_IDX_MINB"] = str(minb)
     with capi.Problem(kt, L, k, d) as P:
         P.add_block(bench.synth(n))
         ms = P.bench_lower_resident(2, 1, True)
         out = {"ms": float(ms.mean()), "launches": P.stats()["launches"], "layout": P.index_layout()}
-    key = "n%d_t%d_%s_cols%d_minb%s" % (n, kt, split, cols, minb)
+    key = "n%d_t%d_%s_cols%d" % (n, kt, split, cols)
     res[key] = out
     print(key, out, flush=True)
     with open("gpurun_out/split_ab.json", "w") as f:
@@ -54,10 +50,8 @@ res["same_bits_20k"] = bool(same)
 for n in sizes:
     timed(n, "equal")
     timed(n, "greedy")
-    timed(n, "greedy", minb=1)
     if n >= 40000:
         timed(n, "greedy", cols=14336)
-        timed(n, "greedy", cols=13312, minb=1)
 # gkmQC's weighted default kernel type at 20k x 300 bp (two blocks either way; W20 slots hold 16 352 columns at most)
 timed(20000, "equal", kt=4, L=10, k=6, d=3)
 timed(20000, "greedy", kt=4, L=10, k=6, d=3)
