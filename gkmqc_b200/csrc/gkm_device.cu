@@ -14,7 +14,6 @@
 #include <cuda_runtime.h>
 #include <pthread.h>
 #include <semaphore.h>
-#include <sys/mman.h>
 #include <unistd.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -31,6 +30,7 @@
 #define GKM_MAX_DEV 16
 #define GKM_NBUF 4 /* chunks in flight per GPU: kernels run ahead while the host scatters finished ones */
 #define GKM_FLUSH_BYTES ((size_t) 256 << 20) /* > 126 MB L2 */
+#define GKM_WAVE_ROWS 148 /* rows of one wave of the index variant's row kernel: one CTA per row and SM */
 
 #define CK(call)                                                                              \
     do {                                                                                      \
@@ -247,6 +247,33 @@ static int gpu_prepare(gkm_gpu *g, int id, size_t band_bytes, size_t stage_bytes
     return 0;
 }
 
+/* body(slot) for every GPU slot of ds side by side, with that slot's device current: slot 0 on the caller's thread, the
+ * others on threads of their own (on the caller's thread too if one cannot start).  The error text is per thread
+ * (gkm_log.c), so a failing slot's is handed over to the caller's. */
+template <class F>
+static int for_each_gpu(const gkm_devstate *ds, const F &body)
+{
+    struct slot_run { const F *body; int dev, slot, rc; char err[256]; } run[GKM_MAX_DEV];
+    void *(*go)(void *) = [](void *a) -> void * {
+        slot_run *r = (slot_run *) a;
+        r->rc = 1;
+        if (cudaSetDevice(r->dev) != cudaSuccess) gkm_set_error("CUDA: cannot select device %d", r->dev);
+        else r->rc = (*r->body)(r->slot);
+        if (r->rc) snprintf(r->err, sizeof(r->err), "%s", gkmb200_last_error());
+        return NULL;
+    };
+    pthread_t th[GKM_MAX_DEV];
+    int started[GKM_MAX_DEV];
+    for (int i = 0; i < ds->ndev; i++) {
+        run[i].body = &body; run[i].dev = ds->dev[i]; run[i].slot = i; run[i].rc = 0;
+        started[i] = i > 0 && pthread_create(&th[i], NULL, go, &run[i]) == 0;
+    }
+    go(&run[0]);
+    for (int i = 1; i < ds->ndev; i++) { if (started[i]) pthread_join(th[i], NULL); else go(&run[i]); }
+    for (int i = 0; i < ds->ndev; i++) if (run[i].rc) { gkm_set_error("%s", run[i].err); return 1; }
+    return 0;
+}
+
 /* ------------------------------------------------------------------ */
 /* one launch of a histogram kernel over the block described by kp     */
 /* ------------------------------------------------------------------ */
@@ -360,6 +387,20 @@ static int ensure_mma(const gkmb200_problem *p, gkm_image *im, gkm_gpu *g, cudaS
     return 0;
 }
 
+/* the tile shape (TA, TB) of a bit-sliced or lmer launch: the first candidate, in order, whose shared memory
+ * bytes(TA, TB) fit `lim`, else the first that fits 220 KB */
+template <int N, class F>
+static int pick_tile(const int (&cand)[N][2], unsigned lim, const F &bytes, gkm_kparams *kp, unsigned *smem)
+{
+    for (int pass = 0; pass < 2; pass++)
+        for (int i = 0; i < N; i++) {
+            const unsigned s = bytes(cand[i][0], cand[i][1]);
+            if (s <= (pass == 0 ? lim : 220u * 1024u)) { kp->TA = cand[i][0]; kp->TB = cand[i][1]; *smem = s; return 0; }
+        }
+    gkm_set_error("sequence too long for shared memory");
+    return 1;
+}
+
 static int launch_hist(const gkmb200_problem *p, const gkm_image *im, gkm_gpu *g, gkm_kparams kp, cudaStream_t st, int *variant_out)
 {
     const int variant = pick_variant(p, kp.mode);
@@ -370,22 +411,16 @@ static int launch_hist(const gkmb200_problem *p, const gkm_image *im, gkm_gpu *g
         return launch_index(p, im, g, kp, st);
     }
     const void *fn = NULL;
-    unsigned smem = 0;
+    unsigned smem = 0, threads = 256;
+    void *args[3] = { &kp }; /* each kernel reads the leading entries it takes */
     if (variant == GKM_KERNEL_DIAG) {
         const int nb = gkm_diag_nb(p->param.d);
         fn = diag_fn(p->param.L, nb, p->weighted, p->param.d);
         if (!fn) { gkm_set_error("no diag kernel for L=%d", p->param.L); return 1; }
         /* TB = 32 makes the lane-task count of a uniform-length tile a multiple of the warp size */
         static const int cand[][2] = { {8, 32}, {4, 32}, {4, 16}, {2, 16}, {2, 8}, {2, 4}, {2, 2}, {2, 1} }; /* TA even: queries go in pairs */
-        int chosen = -1;
-        for (int pass = 0; pass < 2 && chosen < 0; pass++)
-            for (unsigned i = 0; i < sizeof(cand) / sizeof(cand[0]); i++) {
-                unsigned s = gkm_diag_layout(p->Wmax, p->Wa, cand[i][0], cand[i][1], nb, p->weighted).total;
-                if (s <= (pass == 0 ? 74u * 1024u : 220u * 1024u)) { chosen = (int) i; smem = s; break; }
-            }
-        if (chosen < 0) { gkm_set_error("sequence too long for shared memory"); return 1; }
-        kp.TA = cand[chosen][0];
-        kp.TB = cand[chosen][1];
+        if (pick_tile(cand, 74u * 1024u, [&](int ta, int tb) { return gkm_diag_layout(p->Wmax, p->Wa, ta, tb, nb, p->weighted).total; },
+                      &kp, &smem)) return 1;
     } else if (variant == GKM_KERNEL_MMA) {
         gkm_image *imw = const_cast<gkm_image *>(im);
         if (ensure_mma(p, imw, g, st)) return 1;
@@ -397,42 +432,30 @@ static int launch_hist(const gkmb200_problem *p, const gkm_image *im, gkm_gpu *g
         if (smem > 227u * 1024u) { gkm_set_error("sequence too long for the mma kernel"); return 1; }
         kp.TA = im->mma.QA;
         kp.TB = GKM_MMA_TB;
-        CK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
-        dim3 grid((unsigned) ((cols + kp.TB - 1) / kp.TB), (unsigned) ((rows + kp.TA - 1) / kp.TA), 1);
-        if (grid.y > 65535u) { gkm_set_error("chunk has too many row tiles"); return 1; }
-        void *args[] = { &kp, (void *) &im->mma, (void *) &im->tmap };
-        CK(cudaLaunchKernel(fn, grid, dim3(GKM_MMA_THREADS, 1, 1), args, smem, st));
-        g->nkernels++;
-        if (variant_out) *variant_out = variant;
-        return 0;
+        threads = GKM_MMA_THREADS;
+        args[1] = (void *) &im->mma;
+        args[2] = (void *) &im->tmap;
     } else {
         fn = p->weighted ? (const void *) gkm_lmer_kernel<true> : (const void *) gkm_lmer_kernel<false>;
         static const int cand[][2] = { {8, 8}, {4, 4}, {2, 2}, {1, 1} };
-        int chosen = -1;
-        for (int pass = 0; pass < 2 && chosen < 0; pass++)
-            for (unsigned i = 0; i < sizeof(cand) / sizeof(cand[0]); i++) {
-                unsigned s = gkm_lmer_smem_bytes(p->Wa, cand[i][0], cand[i][1], p->nbins, p->weighted);
-                if (s <= (pass == 0 ? 100u * 1024u : 220u * 1024u)) { chosen = (int) i; smem = s; break; }
-            }
-        if (chosen < 0) { gkm_set_error("sequence too long for shared memory"); return 1; }
-        kp.TA = cand[chosen][0];
-        kp.TB = cand[chosen][1];
+        if (pick_tile(cand, 100u * 1024u, [&](int ta, int tb) { return gkm_lmer_smem_bytes(p->Wa, ta, tb, p->nbins, p->weighted); },
+                      &kp, &smem)) return 1;
     }
     CK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
     dim3 grid((unsigned) ((cols + kp.TB - 1) / kp.TB), (unsigned) ((rows + kp.TA - 1) / kp.TA), 1);
     /* the diagonal: one CTA per row tile (it finds its own column tile), where the tile shapes allow it */
     if (kp.mode == GKM_MODE_DIAG && variant == GKM_KERNEL_DIAG && kp.TB % kp.TA == 0 && kp.row_begin == kp.col_begin) grid.x = 1;
     if (grid.y > 65535u) { gkm_set_error("chunk has too many row tiles"); return 1; }
-    void *args[] = { &kp };
-    CK(cudaLaunchKernel(fn, grid, dim3(256, 1, 1), args, smem, st));
+    CK(cudaLaunchKernel(fn, grid, dim3(threads, 1, 1), args, smem, st));
     g->nkernels++;
     if (variant_out) *variant_out = variant;
     return 0;
 }
 
-static void fill_kparams(const gkmb200_problem *p, const gkm_image *im, gkm_kparams *kp)
+static void fill_kparams(const gkmb200_problem *p, const gkm_image *im, int mode, gkm_kparams *kp)
 {
     memset(kp, 0, sizeof(*kp));
+    kp->mode = mode;
     kp->planes = im->planes;
     kp->lens = im->lens;
     kp->wend = im->wend;
@@ -660,28 +683,13 @@ static int choose_variant(gkmb200_problem *p, int row0, int nrows, int col0, int
     if (v == GKM_KERNEL_INDEX) {
         /* every GPU builds its own copy of the (cheap) index: side by side, one host thread per GPU -- in turn the
          * builds of an 8-GPU call at 50k (4 column blocks each, a stream sync per block) were ~25 ms of host time */
-        struct idx_job { gkmb200_problem *p; int slot, col0, col1, greedy, strict, rc; char err[256]; };
-        idx_job jobs[GKM_MAX_DEV];
-        pthread_t th[GKM_MAX_DEV];
-        int started[GKM_MAX_DEV];
-        auto body = [](void *a) -> void * {
-            idx_job *j = (idx_job *) a;
-            gkm_devstate *d = j->p->dev;
-            gkm_gpu *g = &g_gpu[d->dev[j->slot]];
-            j->rc = 1;
-            if (cudaSetDevice(d->dev[j->slot]) != cudaSuccess) { gkm_set_error("CUDA: cannot select device %d", d->dev[j->slot]); }
-            else if (!ensure_index(j->p, g, &d->img[j->slot], j->col0, j->col1, j->greedy, j->strict) &&
-                     cudaEventRecord(g->join, g->sc) == cudaSuccess && cudaStreamWaitEvent(g->sc2, g->join, 0) == cudaSuccess) j->rc = 0;
-            if (j->rc) snprintf(j->err, sizeof(j->err), "%s", gkmb200_last_error());
-            return NULL;
-        };
-        for (int i = 0; i < ds->ndev; i++) {
-            jobs[i].p = p; jobs[i].slot = i; jobs[i].col0 = col0; jobs[i].col1 = col0 + ncols; jobs[i].greedy = greedy; jobs[i].strict = gopt >= 0; jobs[i].rc = 0; jobs[i].err[0] = 0;
-            started[i] = (i > 0) && pthread_create(&th[i], NULL, body, &jobs[i]) == 0;
-        }
-        body(&jobs[0]);
-        for (int i = 1; i < ds->ndev; i++) { if (started[i]) pthread_join(th[i], NULL); else body(&jobs[i]); }
-        for (int i = 0; i < ds->ndev; i++) if (jobs[i].rc) { gkm_set_error("%s", jobs[i].err[0] ? jobs[i].err : "index build failed"); return 1; }
+        if (for_each_gpu(ds, [&](int slot) {
+                gkm_gpu *g = &g_gpu[ds->dev[slot]];
+                if (ensure_index(p, g, &ds->img[slot], col0, col0 + ncols, greedy, gopt >= 0)) return 1;
+                CK(cudaEventRecord(g->join, g->sc));
+                CK(cudaStreamWaitEvent(g->sc2, g->join, 0));
+                return 0;
+            })) return 1;
         /* kernel = auto, second look: the cost model above assumes random sequences.  The index build knows better:
          * a list of l postings is met by ~l/2 query L-mers of the same problem, l^2/4 exact-match hits in the lower
          * triangle.  Low-complexity input (thousands of poly-A sequences) makes that term seconds; the bit-sliced
@@ -886,8 +894,7 @@ static int upload_locked(gkmb200_problem *p, int need_host)
         }
         /* sqnorm: Kraw(a,a) by the same kernel in diagonal mode, in blocks of 1024 rows */
         gkm_kparams kp;
-        fill_kparams(p, im, &kp);
-        kp.mode = GKM_MODE_DIAG;
+        fill_kparams(p, im, GKM_MODE_DIAG, &kp);
         kp.sqnorm_out = im->sqnorm;
         /* the bit-sliced kernel covers the diagonal with one column of CTAs, 8 rows each: one launch for up to
          * 131 070 rows (grid.y <= 65 535 row tiles of at least 2 rows; it was 10 launches of 32 x 128 CTAs at 10k,
@@ -935,9 +942,6 @@ struct gkm_job {
     double **rows;          /* ... or row pointers (absolute column index) */
     int32_t *hist;          /* dense histogram destination (tests) */
     int copy_threads;
-    double thp_cover;       /* advise_chunk: least covered fraction of a chunk's row span that earns the huge-page hint; 0 = never */
-    int failed;
-    char err[256];
 };
 
 struct gkm_scatter {
@@ -1044,39 +1048,6 @@ static void scatter_chunk(gkm_team *tm, const gkm_job *job, const gkm_chunk *c, 
     if (nt > 1) while (sem_wait(&tm->done) != 0) { /* EINTR */ }
 }
 
-/* The caller's matrix is fresh, never-touched memory (np.zeros of 15000 x 15000, gkmsvm.py:75): every 4 KB page the
- * scatter writes first takes a page fault (~2 us; 1.4-1.8 GB/s per thread).  With transparent huge pages in "madvise"
- * mode a 2 MB page is zeroed in one fault at ~5 GB/s per thread -- but the WHOLE page, the upper triangle included.
- * Round 1 hinted the whole matrix and measured no gain: the triangle covers half of it.  The hint is now given per
- * chunk, only to the whole huge pages inside that chunk's own row span, and only where the chunk's entries cover
- * at least `thp_cover` of that span (break-even 0.37 on this host: 400 us per huge page against 512 x 2.1 us).
- * A hint only: it changes no contents and no ownership -- but it makes the untouched part of a huge page resident, and it
- * bought nothing measurable (gkm_dev_compute), so it is off unless GKM_THP_COVER sets a bar. */
-static int advise_chunk(const gkm_job *job, const gkm_chunk *c)
-{
-    const int nr = c->row_end - c->row_begin;
-    if (job->thp_cover <= 0.0 || nr < 2 || c->col_end <= c->col_begin) return 0;
-    const char *first;
-    ptrdiff_t stride;
-    if (job->rows) {
-        first = (const char *) (job->rows[c->row_begin] + c->col_begin);
-        stride = (const char *) job->rows[c->row_begin + 1] - (const char *) job->rows[c->row_begin];
-        for (int r = c->row_begin; r + 1 < c->row_end; r++) /* one array with evenly spaced rows, or no hint */
-            if ((const char *) job->rows[r + 1] - (const char *) job->rows[r] != stride) return 0;
-    } else if (job->out) {
-        stride = (ptrdiff_t) job->ld * (ptrdiff_t) sizeof(double);
-        first = (const char *) (job->out + (size_t) (c->row_begin - job->row0) * (size_t) job->ld + (size_t) (c->col_begin - job->col0));
-    } else return 0;
-    if (stride <= 0) return 0;
-    const double span = (double) stride * (double) nr;
-    if ((double) c->entries * 8.0 < job->thp_cover * span) return 0;
-    const uintptr_t huge = (uintptr_t) 2 << 20;
-    uintptr_t lo = ((uintptr_t) first + huge - 1) & ~(huge - 1);
-    uintptr_t hi = ((uintptr_t) first + (uintptr_t) stride * (uintptr_t) (nr - 1) + (uintptr_t) (c->col_end - c->col_begin) * sizeof(double)) & ~(huge - 1);
-    if (hi <= lo) return 0;
-    return madvise((void *) lo, (size_t) (hi - lo), MADV_HUGEPAGE) == 0;
-}
-
 struct gkm_devthread {
     gkm_job *job;
     int slot;          /* index into devstate */
@@ -1084,15 +1055,13 @@ struct gkm_devthread {
     double scatter_ms, wait_ms; /* host time of this device thread spent copying into caller rows / waiting for the GPU */
     long long launches, d2h_bytes, entries;
     int variant;
-    int thp_chunks;    /* chunks whose destination got the huge-page hint */
 };
 
 static int dev_issue(gkm_devthread *dt, gkm_gpu *g, const gkm_image *im, const gkm_chunk *c, int buf, int32_t *d_hist)
 {
     gkm_job *job = dt->job;
     gkm_kparams kp;
-    fill_kparams(job->p, im, &kp);
-    kp.mode = job->lower ? GKM_MODE_LOWER : GKM_MODE_RECT;
+    fill_kparams(job->p, im, job->lower ? GKM_MODE_LOWER : GKM_MODE_RECT, &kp);
     kp.row_begin = kp.row_base = c->row_begin;
     kp.row_end = c->row_end;
     kp.col_begin = kp.col_base = c->col_begin;
@@ -1103,7 +1072,6 @@ static int dev_issue(gkm_devthread *dt, gkm_gpu *g, const gkm_image *im, const g
     kp.hist = d_hist;
     kp.hist_cols = width;
     cudaStream_t st = (buf & 1) ? g->sc2 : g->sc;
-    dt->thp_chunks += advise_chunk(job, c); /* ahead of the kernel: off the critical path of the copy-out */
     CK(cudaEventRecord(g->k0[buf], st));
     const long long k_before = g->nkernels;
     if (launch_hist(job->p, im, g, kp, st, &dt->variant)) return 1;
@@ -1206,33 +1174,14 @@ static int dev_thread_run(gkm_devthread *dt, gkm_team *team_p)
         }
     }
     dt->scatter_ms = t_scatter; dt->wait_ms = t_wait;
-    gkm_log(GKM_LOG_DEBUG, "GPU %d: %.2f ms in all: issue %.2f, waiting for chunks %.2f, scatter %.2f = %.1f GB/s with %d threads, %d chunks "
-            "hinted huge (after the last chunk arrived: %.2f)",
+    gkm_log(GKM_LOG_DEBUG, "GPU %d: %.2f ms in all: issue %.2f, waiting for chunks %.2f, scatter %.2f = %.1f GB/s with %d threads "
+            "(after the last chunk arrived: %.2f)",
             ds->dev[dt->slot], now_ms() - tb0, t_issue, t_wait, t_scatter, t_scatter > 0 ? (double) dt->entries * 8e-6 / t_scatter : 0.0,
-            team.nthreads, dt->thp_chunks, now_ms() - t_lastsync);
+            team.nthreads, now_ms() - t_lastsync);
     if (rc) cudaDeviceSynchronize();
     if (d_hist) cudaFree(d_hist);
     free(h_hist);
     return rc;
-}
-
-static int dev_thread_body(gkm_devthread *dt)
-{
-    gkm_team team;
-    team_start(&team, (dt->job->out || dt->job->rows) ? dt->job->copy_threads : 1);
-    const int rc = dev_thread_run(dt, &team);
-    team_stop(&team);
-    return rc;
-}
-
-static void *dev_thread(void *arg)
-{
-    gkm_devthread *dt = (gkm_devthread *) arg;
-    if (dev_thread_body(dt)) {
-        dt->job->failed = 1;
-        snprintf(dt->job->err, sizeof(dt->job->err), "%s", gkmb200_last_error());
-    }
-    return NULL;
 }
 
 static long long plan_budget(const gkmb200_problem *p, long long total_cells, int ndev)
@@ -1241,6 +1190,21 @@ static long long plan_budget(const gkmb200_problem *p, long long total_cells, in
     long long want = total_cells * 8 / (16LL * ndev * p->shard_world);
     if (want < (4LL << 20)) want = 4LL << 20;
     return want < cap ? want : cap;
+}
+
+/* The chunks of rows [row0, +nrows) x columns [col0, +ncols) in *out (malloc'd; the caller frees it), for nshare GPUs.
+ * The index variant costs the same for every row, so its chunks are whole waves of rows, at most 4 of them; the
+ * others take 16-row tiles, at most 65 520 rows (grid.y <= 65 535 row tiles).  Returns the count, or -1. */
+static int plan_chunks(const gkmb200_problem *p, int row0, int nrows, int col0, int ncols, int lower, int nshare, gkm_chunk **out)
+{
+    const int by_rows = (p->dev->variant == GKM_KERNEL_INDEX);
+    const int maxc = nrows / 16 + 2;
+    const long long total_cells = (long long) nrows * ncols / (lower ? 2 : 1);
+    *out = (gkm_chunk *) malloc(sizeof(gkm_chunk) * (size_t) maxc);
+    const int nchunks = *out ? gkm_plan_chunks_rows(row0, nrows, col0, ncols, lower, by_rows ? GKM_WAVE_ROWS : 16, plan_budget(p, total_cells, nshare),
+                                                    by_rows ? 4 * GKM_WAVE_ROWS : 65520, *out, maxc) : -1;
+    if (nchunks < 0) gkm_set_error("chunk planning failed");
+    return nchunks;
 }
 
 /* Host threads that scatter finished chunks into the caller's rows.  The reference's `nthreads` (default 1 in
@@ -1299,16 +1263,9 @@ extern "C" int gkm_dev_compute(gkmb200_problem *p, int row0, int nrows, int col0
     int *owned = NULL;
     if (!rc) {
         gkm_devstate *ds = p->dev;
-        const long long total_cells = (long long) nrows * ncols / (lower ? 2 : 1);
-        /* index variant: every row costs the same, so chunks are whole waves of rows (one CTA per row and SM) */
-        const int by_rows = (ds->variant == GKM_KERNEL_INDEX);
-        const int tile_rows = by_rows ? 148 : 16;
-        const int maxc = nrows / tile_rows + 2;
-        chunks = (gkm_chunk *) malloc(sizeof(gkm_chunk) * (size_t) maxc);
-        owned = (int *) malloc(sizeof(int) * (size_t) maxc);
-        int nchunks = (chunks && owned) ? gkm_plan_chunks_rows(row0, nrows, col0, ncols, lower, tile_rows,
-                                                               plan_budget(p, total_cells, ds->ndev), by_rows ? 4 * 148 : 65520 /* grid.y <= 65535 row tiles */, chunks, maxc) : -1;
-        if (nchunks < 0) { gkm_set_error("chunk planning failed"); rc = 1; }
+        const int nchunks = plan_chunks(p, row0, nrows, col0, ncols, lower, ds->ndev, &chunks);
+        if (nchunks < 0) rc = 1;
+        else if (!(owned = (int *) malloc(sizeof(int) * (size_t) (nchunks + 1)))) { gkm_set_error("out of memory"); rc = 1; }
         if (!rc) {
             gkm_job job;
             memset(&job, 0, sizeof(job));
@@ -1320,35 +1277,22 @@ extern "C" int gkm_dev_compute(gkmb200_problem *p, int row0, int nrows, int col0
             /* the host threads that scatter finished chunks are shared by the GPUs of the call: each device thread
              * leads a team of its share of them (different chunks, so different 2 MB regions of the destination) */
             job.copy_threads = copy_threads / ds->ndev > 1 ? copy_threads / ds->ndev : 1;
-            /* huge-page hint on the destination: OFF unless asked for (GKM_THP_COVER=<least covered share of a chunk's row
-             * span>, e.g. 0.4).  Round 2 measured no gain at any GPU count (16 threads first-touch 23 GB/s with 2 MB pages
-             * against 19 with 4 KB ones in the probe, 0.427 s per 50k call on 2 GPUs either way) and the hint makes the
-             * caller's untouched upper triangle resident. */
-            if ((rows || out) && !hist && !getenv("GKM_NO_THP")) {
-                const char *tc = getenv("GKM_THP_COVER");
-                job.thp_cover = tc ? atof(tc) : 0.0;
-            }
             gkm_devthread dts[GKM_MAX_DEV];
-            pthread_t th[GKM_MAX_DEV];
-            int started[GKM_MAX_DEV];
             memset(dts, 0, sizeof(dts));
-            for (int i = 0; i < ds->ndev; i++) {
-                dts[i].job = &job; dts[i].slot = i;
-                started[i] = 0;
-                if (i > 0) started[i] = (pthread_create(&th[i], NULL, dev_thread, &dts[i]) == 0);
-            }
-            dev_thread(&dts[0]);
-            for (int i = 1; i < ds->ndev; i++) {
-                if (started[i]) pthread_join(th[i], NULL);
-                else dev_thread(&dts[i]);
-            }
+            for (int i = 0; i < ds->ndev; i++) { dts[i].job = &job; dts[i].slot = i; }
+            rc = for_each_gpu(ds, [&](int slot) {
+                gkm_team team;
+                team_start(&team, (out || rows) ? job.copy_threads : 1);
+                const int r = dev_thread_run(&dts[slot], &team);
+                team_stop(&team);
+                return r;
+            });
             p->stats.kernel_ms = 0; p->stats.d2h_bytes = 0; p->stats.entries = 0;
-            p->stats.scatter_ms = 0; p->stats.wait_ms = 0; p->stats.thp_chunks = 0;
+            p->stats.scatter_ms = 0; p->stats.wait_ms = 0;
             p->stats.copy_threads = job.copy_threads * ds->ndev;
             for (int i = 0; i < ds->ndev; i++) {
                 if (dts[i].scatter_ms > p->stats.scatter_ms) p->stats.scatter_ms = (float) dts[i].scatter_ms;
                 if (dts[i].wait_ms > p->stats.wait_ms) p->stats.wait_ms = (float) dts[i].wait_ms;
-                p->stats.thp_chunks += dts[i].thp_chunks;
                 if (dts[i].kernel_ms > p->stats.kernel_ms) p->stats.kernel_ms = dts[i].kernel_ms;
                 p->stats.launches += dts[i].launches;
                 p->stats.d2h_bytes += dts[i].d2h_bytes;
@@ -1357,7 +1301,6 @@ extern "C" int gkm_dev_compute(gkmb200_problem *p, int row0, int nrows, int col0
             }
             p->stats.devices = ds->ndev;
             p->stats.shard_rank = p->shard_rank; p->stats.shard_world = p->shard_world;
-            if (job.failed) { gkm_set_error("%s", job.err); rc = 1; }
         }
     }
     free(chunks);
@@ -1372,66 +1315,46 @@ extern "C" int gkm_dev_compute(gkmb200_problem *p, int row0, int nrows, int col0
 /* ------------------------------------------------------------------ */
 /* fused decision values (SURVEY.md 8f/f1)                              */
 /* ------------------------------------------------------------------ */
-struct gkm_decjob {
-    gkmb200_problem *p;
-    int slot, row0, nrows, col0, ncols;
-    const double *alpha;
-    double bias;
-    double *out;     /* out[0] = first row of this slice */
-    int rc;
-    char err[256];
-};
-
 /* one GPU's slice of the test rows: out[r] = bias + sum_c alpha[c] K(row0 + r, col0 + c) */
-static int decision_slice(gkm_decjob *j)
+static int decision_slice(gkmb200_problem *p, int slot, int row0, int nrows, int col0, int ncols, const double *alpha, double bias, double *out)
 {
-    gkmb200_problem *p = j->p;
+    if (nrows <= 0) return 0;
     gkm_devstate *ds = p->dev;
-    gkm_gpu *g = &g_gpu[ds->dev[j->slot]];
+    gkm_gpu *g = &g_gpu[ds->dev[slot]];
     double *d_alpha = NULL, *d_dec = NULL;
     int rc = 0;
     do {
-        if (cudaSetDevice(ds->dev[j->slot]) != cudaSuccess) { rc = 1; break; }
-        if (cudaMalloc(&d_alpha, sizeof(double) * (size_t) (j->ncols ? j->ncols : 1)) != cudaSuccess) { rc = 1; break; }
-        if (cudaMalloc(&d_dec, sizeof(double) * (size_t) (j->nrows ? j->nrows : 1)) != cudaSuccess) { rc = 1; break; }
-        if (cudaMemcpyAsync(d_alpha, j->alpha, sizeof(double) * (size_t) j->ncols, cudaMemcpyHostToDevice, g->sc) != cudaSuccess) { rc = 1; break; }
-        if (cudaMemsetAsync(d_dec, 0, sizeof(double) * (size_t) j->nrows, g->sc) != cudaSuccess) { rc = 1; break; }
+        if (cudaMalloc(&d_alpha, sizeof(double) * (size_t) (ncols ? ncols : 1)) != cudaSuccess) { rc = 1; break; }
+        if (cudaMalloc(&d_dec, sizeof(double) * (size_t) nrows) != cudaSuccess) { rc = 1; break; }
+        if (cudaMemcpyAsync(d_alpha, alpha, sizeof(double) * (size_t) ncols, cudaMemcpyHostToDevice, g->sc) != cudaSuccess) { rc = 1; break; }
+        if (cudaMemsetAsync(d_dec, 0, sizeof(double) * (size_t) nrows, g->sc) != cudaSuccess) { rc = 1; break; }
         /* the second compute stream must see alpha and the zeroed accumulator too */
         if (cudaEventRecord(g->join, g->sc) != cudaSuccess || cudaStreamWaitEvent(g->sc2, g->join, 0) != cudaSuccess) { rc = 1; break; }
     } while (0);
     if (rc) gkm_set_error("CUDA: decision-value buffers: %s", cudaGetErrorString(cudaGetLastError()));
     gkm_kparams kp;
-    fill_kparams(p, &ds->img[j->slot], &kp);
-    kp.mode = GKM_MODE_RECT;
+    fill_kparams(p, &ds->img[slot], GKM_MODE_RECT, &kp);
     kp.alpha = d_alpha; kp.decision = d_dec;
-    kp.col_begin = kp.col_base = j->col0; kp.col_end = j->col0 + j->ncols;
-    kp.row_base = j->row0;
+    kp.col_begin = kp.col_base = col0; kp.col_end = col0 + ncols;
+    kp.row_base = row0;
     int launches = 0;
     /* index variant: whole waves of rows per launch, and a bounded cold-bin scratch */
-    const int rows_per_launch = (ds->variant == GKM_KERNEL_INDEX) ? 16 * 148 : 8192;
-    for (int r = j->row0; !rc && r < j->row0 + j->nrows; r += rows_per_launch) {
+    const int rows_per_launch = (ds->variant == GKM_KERNEL_INDEX) ? 16 * GKM_WAVE_ROWS : 8192;
+    for (int r = row0; !rc && r < row0 + nrows; r += rows_per_launch) {
         kp.row_begin = r;
-        kp.row_end = (r + rows_per_launch < j->row0 + j->nrows) ? r + rows_per_launch : j->row0 + j->nrows;
-        rc = launch_hist(p, &ds->img[j->slot], g, kp, (launches++ & 1) ? g->sc2 : g->sc, NULL);
+        kp.row_end = (r + rows_per_launch < row0 + nrows) ? r + rows_per_launch : row0 + nrows;
+        rc = launch_hist(p, &ds->img[slot], g, kp, (launches++ & 1) ? g->sc2 : g->sc, NULL);
     }
     if (!rc) {
         rc = (cudaStreamSynchronize(g->sc2) != cudaSuccess) ||
-             (cudaMemcpyAsync(j->out, d_dec, sizeof(double) * (size_t) j->nrows, cudaMemcpyDeviceToHost, g->sc) != cudaSuccess) ||
+             (cudaMemcpyAsync(out, d_dec, sizeof(double) * (size_t) nrows, cudaMemcpyDeviceToHost, g->sc) != cudaSuccess) ||
              (cudaStreamSynchronize(g->sc) != cudaSuccess);
         if (rc) gkm_set_error("CUDA: decision values failed: %s", cudaGetErrorString(cudaGetLastError()));
     }
-    if (!rc) for (int i = 0; i < j->nrows; i++) j->out[i] += j->bias;
+    if (!rc) for (int i = 0; i < nrows; i++) out[i] += bias;
     cudaFree(d_alpha);
     cudaFree(d_dec);
     return rc;
-}
-
-static void *decision_thread(void *arg)
-{
-    gkm_decjob *j = (gkm_decjob *) arg;
-    j->rc = decision_slice(j);
-    if (j->rc) snprintf(j->err, sizeof(j->err), "%s", gkmb200_last_error());
-    return NULL;
 }
 
 /* the test rows are cut into one contiguous slice per selected GPU; every GPU holds all columns (SVs) */
@@ -1447,28 +1370,13 @@ extern "C" int gkm_dev_decision(gkmb200_problem *p, int row0, int nrows, int col
     int rc = upload_locked(p, 0);
     if (!rc) rc = choose_variant(p, row0, nrows, col0, ncols, 0);
     if (!rc) {
-        gkm_devstate *ds = p->dev;
-        const int nd = ds->ndev;
-        gkm_decjob jobs[GKM_MAX_DEV];
-        pthread_t th[GKM_MAX_DEV];
-        int started[GKM_MAX_DEV];
-        const int per = ((nrows + nd - 1) / nd + 7) & ~7;
-        for (int i = 0; i < nd; i++) {
-            int b = i * per, e = b + per;
+        const int nd = p->dev->ndev, per = ((nrows + nd - 1) / nd + 7) & ~7;
+        rc = for_each_gpu(p->dev, [&](int slot) {
+            int b = slot * per, e = b + per;
             if (b > nrows) b = nrows;
             if (e > nrows) e = nrows;
-            memset(&jobs[i], 0, sizeof(jobs[i]));
-            jobs[i].p = p; jobs[i].slot = i; jobs[i].row0 = row0 + b; jobs[i].nrows = e - b;
-            jobs[i].col0 = col0; jobs[i].ncols = ncols; jobs[i].alpha = alpha; jobs[i].bias = bias; jobs[i].out = out + b;
-            started[i] = 0;
-            if (i > 0 && jobs[i].nrows > 0) started[i] = (pthread_create(&th[i], NULL, decision_thread, &jobs[i]) == 0);
-        }
-        decision_thread(&jobs[0]);
-        for (int i = 1; i < nd; i++) {
-            if (started[i]) pthread_join(th[i], NULL);
-            else if (jobs[i].nrows > 0) decision_thread(&jobs[i]);
-        }
-        for (int i = 0; i < nd; i++) if (jobs[i].rc) { gkm_set_error("%s", jobs[i].err); rc = 1; }
+            return decision_slice(p, slot, row0 + b, e - b, col0, ncols, alpha, bias, out + b);
+        });
     }
     pthread_mutex_unlock(&g_lock);
     return rc;
@@ -1479,13 +1387,12 @@ extern "C" int gkm_dev_decision(gkmb200_problem *p, int row0, int nrows, int col
 /* ------------------------------------------------------------------ */
 /* GPUs of the call that compute chunks of the resident matrix.  The matrix lives on the first selected GPU; the others
  * may help only if they can store into its memory -- peer access over NVLink / NVSwitch, enabled once per process and
- * pair.  All of them or one: GKM_RESIDENT_GPUS=1 keeps the whole pass on the owner (A/B, and boxes whose GPUs are
- * not peers do so by themselves).  Leaves another device current. */
+ * pair.  All of them or one: on boxes whose GPUs are not peers the owner does the whole pass.  Leaves another device
+ * current. */
 static int resident_sharers(const gkm_devstate *ds)
 {
     static signed char peer_ok[GKM_MAX_DEV][GKM_MAX_DEV]; /* [writer][owner]: 0 not asked yet, 1 yes, -1 no */
-    const char *e = getenv("GKM_RESIDENT_GPUS");
-    if (ds->ndev < 2 || (e && atoi(e) == 1)) return 1;
+    if (ds->ndev < 2) return 1;
     const int owner = ds->dev[0];
     for (int i = 1; i < ds->ndev; i++) {
         const int d = ds->dev[i];
@@ -1505,6 +1412,42 @@ static int resident_sharers(const gkm_devstate *ds)
     return ds->ndev;
 }
 
+/* the resident N x full_ld matrix of the first selected GPU (current device must be g's) */
+static int ensure_full(gkm_gpu *g, gkm_image *im, int n)
+{
+    if (im->full) return 0;
+    im->full_ld = ((size_t) n + 15) & ~(size_t) 15;
+    CK(dev_malloc(g, (void **) &im->full, im->full_ld * (size_t) n * sizeof(double)));
+    return 0;
+}
+
+/* Queues the chunks of the lower triangle that shard rank/world owns into im->full of the first selected GPU: chunk c
+ * runs on GPU c % nshare, on sc or sc2 by that GPU's own count of issued chunks.  Adds the kernels launched and the
+ * entries to *kernels / *entries.  With nshare > 1 it leaves another device current. */
+static int lower_pass(gkmb200_problem *p, const gkm_chunk *chunks, int nchunks, int nshare, int rank, int world,
+                      long long *kernels, long long *entries, int *variant_out)
+{
+    gkm_devstate *ds = p->dev;
+    int issued[GKM_MAX_DEV] = { 0 };
+    for (int c = 0; c < nchunks; c++) {
+        if (gkm_chunk_owner(c, nchunks, world) != rank) continue;
+        const int s = c % nshare;
+        gkm_gpu *gs = &g_gpu[ds->dev[s]];
+        if (nshare > 1 && cudaSetDevice(ds->dev[s]) != cudaSuccess) { gkm_set_error("CUDA: cannot select device %d", ds->dev[s]); return 1; }
+        gkm_kparams kp;
+        fill_kparams(p, &ds->img[s], GKM_MODE_LOWER, &kp);
+        kp.row_begin = chunks[c].row_begin; kp.row_end = chunks[c].row_end;
+        kp.col_begin = chunks[c].col_begin; kp.col_end = chunks[c].col_end;
+        kp.out = ds->img[0].full; kp.ld = (long long) ds->img[0].full_ld; /* the owner's block, whichever GPU runs the chunk */
+        const long long k_before = gs->nkernels;
+        const int rc = launch_hist(p, &ds->img[s], gs, kp, (issued[s]++ & 1) ? gs->sc2 : gs->sc, variant_out);
+        *kernels += gs->nkernels - k_before; /* kernels, not chunks: the index variant launches one per column block */
+        *entries += chunks[c].entries;
+        if (rc) return 1;
+    }
+    return 0;
+}
+
 /* One pass of the lower triangle into im->full on the first selected GPU, then mirrored there: the matrix never leaves
  * the devices.  With several GPUs in the call (one process, GKM_DEVICES) the chunks go round-robin over all of them
  * and every GPU writes its entries straight into the owner's matrix -- the epilogue's streaming stores travel over
@@ -1520,34 +1463,11 @@ static int resident_symmetric(gkmb200_problem *p)
     if (im->full && im->full_sym) return 0;
     const int nshare = resident_sharers(ds);
     CK(cudaSetDevice(ds->dev[0]));
-    if (!im->full) {
-        im->full_ld = ((size_t) n + 15) & ~(size_t) 15;
-        CK(dev_malloc(g, (void **) &im->full, im->full_ld * (size_t) n * sizeof(double)));
-    }
-    const int by_rows = (ds->variant == GKM_KERNEL_INDEX);
-    const int maxc = n / 16 + 2;
-    gkm_chunk *chunks = (gkm_chunk *) malloc(sizeof(gkm_chunk) * (size_t) maxc);
-    const int nchunks = chunks ? gkm_plan_chunks_rows(0, n, 0, n, 1, by_rows ? 148 : 16, plan_budget(p, (long long) n * n / 2, nshare),
-                                                      by_rows ? 4 * 148 : 65520 /* grid.y */, chunks, maxc) : -1;
-    if (nchunks < 0) { free(chunks); gkm_set_error("chunk planning failed"); return 1; }
-    int rc = 0, issued[GKM_MAX_DEV];
-    long long kernels = 0;
-    for (int s = 0; s < GKM_MAX_DEV; s++) issued[s] = 0;
-    for (int c = 0; !rc && c < nchunks; c++) {
-        const int s = c % nshare;
-        gkm_gpu *gs = &g_gpu[ds->dev[s]];
-        if (nshare > 1 && cudaSetDevice(ds->dev[s]) != cudaSuccess) { gkm_set_error("CUDA: cannot select device %d", ds->dev[s]); rc = 1; break; }
-        gkm_kparams kp;
-        fill_kparams(p, &ds->img[s], &kp);
-        kp.mode = GKM_MODE_LOWER;
-        kp.row_begin = chunks[c].row_begin; kp.row_end = chunks[c].row_end;
-        kp.col_begin = chunks[c].col_begin; kp.col_end = chunks[c].col_end;
-        kp.row_base = 0; kp.col_base = 0;
-        kp.out = im->full; kp.ld = (long long) im->full_ld; /* the owner's block, whichever GPU runs the chunk */
-        const long long k_before = gs->nkernels;
-        rc = launch_hist(p, &ds->img[s], gs, kp, (issued[s]++ & 1) ? gs->sc2 : gs->sc, NULL);
-        kernels += gs->nkernels - k_before;
-    }
+    if (ensure_full(g, im, n)) return 1;
+    gkm_chunk *chunks = NULL;
+    const int nchunks = plan_chunks(p, 0, n, 0, n, 1, nshare, &chunks);
+    long long kernels = 0, entries = 0;
+    int rc = nchunks < 0 || lower_pass(p, chunks, nchunks, nshare, 0, 1, &kernels, &entries, NULL);
     free(chunks);
     /* the stores of the other GPUs have landed once their streams have drained; the owner mirrors the triangle after that */
     for (int s = 1; s < nshare; s++) {
@@ -1652,50 +1572,24 @@ extern "C" int gkm_dev_bench_lower(gkmb200_problem *p, int steps, int warmup, in
         gkm_devstate *ds = p->dev;
         gkm_gpu *g = &g_gpu[ds->dev[0]];
         gkm_image *im = &ds->img[0];
-        const int n = p->n;
-        do {
-            if (cudaSetDevice(ds->dev[0]) != cudaSuccess) { rc = 1; break; }
-            if (!im->full) {
-                im->full_ld = ((size_t) n + 15) & ~(size_t) 15;
-                if (dev_malloc(g, (void **) &im->full, im->full_ld * (size_t) n * sizeof(double)) != cudaSuccess) { rc = 1; break; }
-            }
-            if (flush_l2 && !g->d_flush && cudaMalloc(&g->d_flush, GKM_FLUSH_BYTES) != cudaSuccess) { rc = 1; break; }
-        } while (0);
-        if (rc) gkm_set_error("CUDA: bench buffers: %s", cudaGetErrorString(cudaGetLastError()));
-        const int maxc = n / 16 + 2;
-        int nchunks = -1;
-        if (!rc) {
-            const int by_rows = (ds->variant == GKM_KERNEL_INDEX);
-            chunks = (gkm_chunk *) malloc(sizeof(gkm_chunk) * (size_t) maxc);
-            nchunks = chunks ? gkm_plan_chunks_rows(0, n, 0, n, 1, by_rows ? 148 : 16, plan_budget(p, (long long) n * n / 2, 1),
-                                                    by_rows ? 4 * 148 : 65520 /* grid.y */, chunks, maxc) : -1;
-            if (nchunks < 0) { gkm_set_error("chunk planning failed"); rc = 1; }
+        if (cudaSetDevice(ds->dev[0]) != cudaSuccess || ensure_full(g, im, p->n) ||
+            (flush_l2 && !g->d_flush && cudaMalloc(&g->d_flush, GKM_FLUSH_BYTES) != cudaSuccess)) {
+            gkm_set_error("CUDA: bench buffers: %s", cudaGetErrorString(cudaGetLastError()));
+            rc = 1;
         }
+        const int nchunks = rc ? -1 : plan_chunks(p, 0, p->n, 0, p->n, 1, 1, &chunks);
+        if (nchunks < 0) rc = 1;
         cudaEvent_t e0 = NULL, e1 = NULL;
         if (!rc) rc = (cudaEventCreate(&e0) != cudaSuccess) || (cudaEventCreate(&e1) != cudaSuccess);
         long long launches = 0, entries = 0;
         int variant = 0;
+        im->full_sym = 0; /* the pass writes the lower triangle only: the consumer mirrors it again */
         for (int it = 0; !rc && it < warmup + steps; it++) {
             if (flush_l2) cudaMemsetAsync(g->d_flush, it & 0xff, GKM_FLUSH_BYTES, g->sc);
             cudaEventRecord(e0, g->sc);
             cudaStreamWaitEvent(g->sc2, e0, 0);
             launches = 0; entries = 0;
-            int nchunk_issued = 0;
-            for (int c = 0; !rc && c < nchunks; c++) {
-                if (gkm_chunk_owner(c, nchunks, p->shard_world) != p->shard_rank) continue;
-                gkm_kparams kp;
-                fill_kparams(p, im, &kp);
-                kp.mode = GKM_MODE_LOWER;
-                kp.row_begin = chunks[c].row_begin; kp.row_end = chunks[c].row_end;
-                kp.col_begin = chunks[c].col_begin; kp.col_end = chunks[c].col_end;
-                kp.row_base = 0; kp.col_base = 0;
-                kp.out = im->full; kp.ld = (long long) im->full_ld;
-                im->full_sym = 0;
-                const long long k_before = g->nkernels;
-                rc = launch_hist(p, im, g, kp, (nchunk_issued++ & 1) ? g->sc2 : g->sc, &variant);
-                launches += g->nkernels - k_before; /* kernels of this pass (one per chunk and column block) */
-                entries += chunks[c].entries;
-            }
+            rc = lower_pass(p, chunks, nchunks, 1, p->shard_rank, p->shard_world, &launches, &entries, &variant);
             cudaEventRecord(g->join, g->sc2);
             cudaStreamWaitEvent(g->sc, g->join, 0);
             cudaEventRecord(e1, g->sc);
@@ -1801,38 +1695,45 @@ __global__ void __launch_bounds__(1024, 2) gkm_mb_atoms_kernel(int iters, uint32
     if ((threadIdx.x & 31u) == 0u) atomicAdd(total, (unsigned long long) cnt + (mbH[threadIdx.x % ncols] < 0 ? 1ull : 0ull));
 }
 
-static int microbench_atoms(gkm_gpu *g, uint32_t active, double *result)
+/* device time of launch(rep) on g->sc: the best of repetitions 1..3 (repetition 0 warms up) */
+template <class F>
+static int best_ms(gkm_gpu *g, const F &launch, float *best)
 {
-    unsigned long long *d = NULL, h = 0;
-    if (cudaMalloc(&d, sizeof(*d)) != cudaSuccess) { gkm_set_error("CUDA: microbench buffers: %s", cudaGetErrorString(cudaGetLastError())); return 1; }
-    int sms = 148;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, g->id);
-    const uint32_t ncols = 20000;
-    const unsigned smem = ncols * 4;
-    const int iters = 4096;
-    cudaFuncSetAttribute(gkm_mb_atoms_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
     cudaEvent_t e0, e1;
     cudaEventCreate(&e0); cudaEventCreate(&e1);
-    float best = 1e30f;
+    *best = 1e30f;
     int rc = 0;
     for (int rep = 0; rep < 4; rep++) {
-        cudaMemsetAsync(d, 0, sizeof(*d), g->sc);
         cudaEventRecord(e0, g->sc);
-        gkm_mb_atoms_kernel<<<2 * sms, 1024, smem, g->sc>>>(iters, ncols, active, d);
+        launch(rep);
         cudaEventRecord(e1, g->sc);
         if (cudaEventSynchronize(e1) != cudaSuccess) { gkm_set_error("CUDA: microbench failed: %s", cudaGetErrorString(cudaGetLastError())); rc = 1; break; }
         float ms = 0.f;
         cudaEventElapsedTime(&ms, e0, e1);
-        if (rep > 0 && ms < best) best = ms;
-        cudaMemcpy(&h, d, sizeof(h), cudaMemcpyDeviceToHost);
+        if (rep > 0 && ms < *best) *best = ms;
     }
     cudaEventDestroy(e0); cudaEventDestroy(e1);
+    return rc;
+}
+
+static int microbench_atoms(gkm_gpu *g, int sms, uint32_t active, double *result)
+{
+    unsigned long long *d = NULL, h = 0; /* one counter per repetition */
+    if (cudaMalloc(&d, 4 * sizeof(*d)) != cudaSuccess) { gkm_set_error("CUDA: microbench buffers: %s", cudaGetErrorString(cudaGetLastError())); return 1; }
+    cudaMemsetAsync(d, 0, 4 * sizeof(*d), g->sc);
+    const uint32_t ncols = 20000;
+    const unsigned smem = ncols * 4;
+    const int iters = 4096;
+    cudaFuncSetAttribute(gkm_mb_atoms_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
+    float best;
+    const int rc = best_ms(g, [&](int rep) { gkm_mb_atoms_kernel<<<2 * sms, 1024, smem, g->sc>>>(iters, ncols, active, d + rep); }, &best);
+    if (!rc) cudaMemcpy(&h, d + 3, sizeof(h), cudaMemcpyDeviceToHost);
     cudaFree(d);
     if (!rc) *result = (double) h / ((double) best * 1e-3) / 1e9;
     return rc;
 }
 
-static int microbench_gather(gkm_gpu *g, double *result)
+static int microbench_gather(gkm_gpu *g, int sms, double *result)
 {
     const size_t slots = (size_t) 1 << 22; /* 4 Mi x 16 B = 64 MB, the size of the L = 11 slot table */
     uint4 *tab = NULL;
@@ -1843,23 +1744,9 @@ static int microbench_gather(gkm_gpu *g, double *result)
         return 1;
     }
     cudaMemsetAsync(tab, 0x5A, slots * sizeof(uint4), g->sc);
-    int sms = 148;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, g->id);
     const int iters = 2048;
-    cudaEvent_t e0, e1;
-    cudaEventCreate(&e0); cudaEventCreate(&e1);
-    float best = 1e30f;
-    int rc = 0;
-    for (int rep = 0; rep < 4; rep++) {
-        cudaEventRecord(e0, g->sc);
-        gkm_mb_gather_kernel<<<sms, 1024, 0, g->sc>>>(tab, (uint32_t) (slots - 1), iters, d);
-        cudaEventRecord(e1, g->sc);
-        if (cudaEventSynchronize(e1) != cudaSuccess) { gkm_set_error("CUDA: microbench failed"); rc = 1; break; }
-        float ms = 0.f;
-        cudaEventElapsedTime(&ms, e0, e1);
-        if (rep > 0 && ms < best) best = ms;
-    }
-    cudaEventDestroy(e0); cudaEventDestroy(e1);
+    float best;
+    const int rc = best_ms(g, [&](int) { gkm_mb_gather_kernel<<<sms, 1024, 0, g->sc>>>(tab, (uint32_t) (slots - 1), iters, d); }, &best);
     cudaFree(tab); cudaFree(d);
     if (!rc) *result = (double) sms * 1024.0 * (double) iters * 4.0 / ((double) best * 1e-3) / 1e9; /* 1e9 gathers (sectors) per second */
     return rc;
@@ -1868,46 +1755,33 @@ static int microbench_gather(gkm_gpu *g, double *result)
 extern "C" int gkm_dev_microbench(const char *what, double *result)
 {
     if (!what || !result) { gkm_set_error("null argument"); return 1; }
+    static const struct { const char *name; void (*fn)(uint32_t *, int, uint32_t); } ops[] = {
+        { "lop3", gkm_mb_kernel<0> }, { "shf", gkm_mb_kernel<1> }, { "popc", gkm_mb_kernel<2> }, { "iadd3", gkm_mb_kernel<3> },
+        { "imad", gkm_mb_kernel<4> }, { "imadhi", gkm_mb_kernel<5> }, { "lop3+imad", gkm_mb_kernel<6> },
+        { "lop3+popc", gkm_mb_kernel<7> }, { "lop3+imad+popc", gkm_mb_kernel<8> } };
     pthread_mutex_lock(&g_lock);
     int rc = ensure_selected();
+    gkm_gpu *g = rc ? NULL : &g_gpu[g_sel[0]];
+    if (!rc) rc = gpu_prepare(g, g_sel[0], 0, 0);
     if (!rc) {
-        do {
-            gkm_gpu *g = &g_gpu[g_sel[0]];
-            if (gpu_prepare(g, g_sel[0], 0, 0)) { rc = 1; break; }
-            if (!strcmp(what, "gather16")) { rc = microbench_gather(g, result); break; }
-            if (!strcmp(what, "atoms7")) { rc = microbench_atoms(g, 7u, result); break; }
-            if (!strcmp(what, "atoms14")) { rc = microbench_atoms(g, 14u, result); break; }
-            if (!strcmp(what, "atoms32")) { rc = microbench_atoms(g, 32u, result); break; }
+        int sms = 148;
+        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, g->id);
+        int op = -1;
+        for (int i = 0; i < (int) (sizeof(ops) / sizeof(ops[0])); i++) if (!strcmp(what, ops[i].name)) op = i;
+        if (!strcmp(what, "gather16")) rc = microbench_gather(g, sms, result);
+        else if (!strcmp(what, "atoms7")) rc = microbench_atoms(g, sms, 7u, result);
+        else if (!strcmp(what, "atoms14")) rc = microbench_atoms(g, sms, 14u, result);
+        else if (!strcmp(what, "atoms32")) rc = microbench_atoms(g, sms, 32u, result);
+        else if (op < 0) { gkm_set_error("unknown microbench %s", what); rc = 1; }
+        else {
             uint32_t *d = NULL;
-            if (cudaMalloc(&d, 64) != cudaSuccess) { rc = 1; break; }
-            int sms = 148;
-            cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, g_sel[0]);
             const int iters = 4096, blocks = sms * 8;
-            cudaEvent_t e0, e1;
-            cudaEventCreate(&e0); cudaEventCreate(&e1);
-            float best = 1e30f;
-            for (int rep = 0; rep < 4; rep++) {
-                cudaEventRecord(e0, g->sc);
-                if (!strcmp(what, "lop3")) gkm_mb_kernel<0><<<blocks, 256, 0, g->sc>>>(d, iters, 12345u + rep);
-                else if (!strcmp(what, "shf")) gkm_mb_kernel<1><<<blocks, 256, 0, g->sc>>>(d, iters, 12345u + rep);
-                else if (!strcmp(what, "popc")) gkm_mb_kernel<2><<<blocks, 256, 0, g->sc>>>(d, iters, 12345u + rep);
-                else if (!strcmp(what, "iadd3")) gkm_mb_kernel<3><<<blocks, 256, 0, g->sc>>>(d, iters, 12345u + rep);
-                else if (!strcmp(what, "imad")) gkm_mb_kernel<4><<<blocks, 256, 0, g->sc>>>(d, iters, 12345u + rep);
-                else if (!strcmp(what, "imadhi")) gkm_mb_kernel<5><<<blocks, 256, 0, g->sc>>>(d, iters, 12345u + rep);
-                else if (!strcmp(what, "lop3+imad")) gkm_mb_kernel<6><<<blocks, 256, 0, g->sc>>>(d, iters, 12345u + rep);
-                else if (!strcmp(what, "lop3+popc")) gkm_mb_kernel<7><<<blocks, 256, 0, g->sc>>>(d, iters, 12345u + rep);
-                else if (!strcmp(what, "lop3+imad+popc")) gkm_mb_kernel<8><<<blocks, 256, 0, g->sc>>>(d, iters, 12345u + rep);
-                else { gkm_set_error("unknown microbench %s", what); rc = 1; break; }
-                cudaEventRecord(e1, g->sc);
-                if (cudaEventSynchronize(e1) != cudaSuccess) { gkm_set_error("CUDA: microbench failed"); rc = 1; break; }
-                float ms = 0.f;
-                cudaEventElapsedTime(&ms, e0, e1);
-                if (rep > 0 && ms < best) best = ms;
-            }
-            cudaEventDestroy(e0); cudaEventDestroy(e1);
+            float best;
+            if (cudaMalloc(&d, 64) != cudaSuccess) { gkm_set_error("CUDA: microbench buffers: %s", cudaGetErrorString(cudaGetLastError())); rc = 1; }
+            else rc = best_ms(g, [&](int rep) { ops[op].fn<<<blocks, 256, 0, g->sc>>>(d, iters, 12345u + rep); }, &best);
             cudaFree(d);
             if (!rc) *result = (double) blocks * 256.0 * (double) iters * 32.0 / ((double) best * 1e-3) / 1e9;
-        } while (0);
+        }
     }
     pthread_mutex_unlock(&g_lock);
     return rc;

@@ -36,7 +36,7 @@ typedef struct gkmb200_stats {
     int kernel_variant;      /* 1 = lmer (XOR/LOP3/POPC per pair), 2 = diag (bit-sliced diagonals), 3 = mma (tcgen05), 4 = index */
     int shard_rank, shard_world; /* the call computed only the chunks of shard rank/world (1 = everything) */
     int copy_threads;        /* host threads that copied finished chunks into the caller's rows */
-    int thp_chunks;          /* chunks whose destination rows got the transparent-huge-page hint */
+    int thp_chunks;          /* always 0: the transparent-huge-page hint on the destination rows is retired (no gain measured) */
     float scatter_ms;        /* host time spent in that copy (page faults of a fresh matrix included), slowest GPU thread */
     float wait_ms;           /* host time spent waiting for the GPU, slowest GPU thread */
 } gkmb200_stats;

@@ -374,19 +374,35 @@ def test_properties_at_scale():
 
 
 def test_multi_gpu_in_one_process_if_available():
+    """all GPUs of the box in one process against one GPU: the kernel matrix (index forced: every GPU builds its own
+    index) and fused decision values (one slice of the test rows per GPU)"""
     ndev = capi.device_count()
     if ndev < 2:
         pytest.skip("single GPU box")
+    lib = capi.load()
+    ids = (capi.ctypes.c_int * ndev)(*range(ndev))
     seqs = random_seqs(700, 300, seed=77)
-    with capi.Problem(2, 11, 7, 3) as P:
-        P.add_many(seqs)
-        K = P.kernel_lower()
-        assert P.stats()["devices"] == ndev
-    ids = (capi.ctypes.c_int * 1)(0)
-    assert capi.load().gkmb200_set_devices(ids, 1) == 0
-    with capi.Problem(2, 11, 7, 3) as P:
-        P.add_many(seqs)
-        assert np.array_equal(P.kernel_lower(), K)
+    alpha = np.random.default_rng(3).standard_normal(500)
+    try:
+        for kernel in ("auto", "index"):
+            capi.set_option("kernel", kernel)
+            assert lib.gkmb200_set_devices(ids, ndev) == 0
+            with capi.Problem(2, 11, 7, 3) as P:
+                P.add_many(seqs)
+                K = P.kernel_lower()
+                st = P.stats()
+                dv = P.decision_values(500, 200, 0, 500, alpha, bias=0.25)
+            assert st["devices"] == ndev
+            assert kernel == "auto" or st["kernel_variant"] == 4
+            np.testing.assert_allclose(dv, K[500:, :500] @ alpha + 0.25, rtol=1e-9, atol=1e-12)
+            assert lib.gkmb200_set_devices(ids, 1) == 0
+            with capi.Problem(2, 11, 7, 3) as P:
+                P.add_many(seqs)
+                assert np.array_equal(P.kernel_lower(), K)
+                np.testing.assert_allclose(P.decision_values(500, 200, 0, 500, alpha, bias=0.25), dv, rtol=1e-9, atol=1e-12)
+    finally:
+        capi.set_option("kernel", "auto")
+        lib.gkmb200_set_devices(ids, 1)
 
 
 def test_sharded_ranks_cover_the_matrix():

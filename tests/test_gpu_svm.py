@@ -112,6 +112,31 @@ def test_resident_matrix_equals_host_matrix(problem):
     assert [f["n_iter"] for f in f_host] == [f["n_iter"] for f in f_dev]
 
 
+def test_bench_pass_is_the_resident_pass():
+    """the benchmark's timed pass (bench_lower_resident) issues the chunks of the pass that fills the consumer's matrix:
+    the entries of two shards add up to those of an unsharded pass, n(n-1)/2; a bench pass writes the lower triangle
+    only, so the consumer's next read mirrors the matrix again.  2000 sequences: the 16 MB triangle makes several chunks
+    (at least 4 MB each), so both shards own some"""
+    with capi.Problem(4, 10, 6, 3, 50, 50.0, 1.0) as P:
+        P.add_many(planted_seqs(1000, 1000, 200))
+        n = P.n
+        low = np.tril(P.kernel_lower(), -1)
+        K = low + low.T + np.eye(n)
+        assert np.array_equal(P.resident_matrix(), K)
+        P.bench_lower_resident(1, 0, flush_l2=False)
+        total = P.stats()["entries"]
+        assert total == n * (n - 1) // 2
+        parts = []
+        for rank in range(2):
+            P.set_shard(rank, 2)
+            P.bench_lower_resident(1, 0, flush_l2=False)
+            parts.append(P.stats()["entries"])
+        P.set_shard(0, 1)
+        assert min(parts) > 0 and sum(parts) == total, parts
+        assert np.array_equal(P.resident_matrix(), K)
+        assert P.stats()["launches"] > 0, "the resident matrix was not mirrored again after the bench pass"
+
+
 def test_driver_crossValidate_matches_the_reference_flow(problem):
     """gkmsvm.crossValidate (gkmsvm.py:126-176) restated with sklearn fits, against the driver mirror"""
     P, K, y = problem

@@ -65,14 +65,14 @@ def e2e(n, tag, env=None, reps=3, seqlen=300, **kw):
 
 if "e2e50" in what:
     res["e2e50"] = {}
-    for tag, env in (("default", {}), ("no_thp", {"GKM_NO_THP": "1"}), ("thp_all", {"GKM_THP_COVER": "0.01"}), ("threads8", {"GKM_COPY_THREADS": "8"}),
-                     ("threads16", {"GKM_COPY_THREADS": "16"}), ("threads32", {"GKM_COPY_THREADS": "32"})):
+    for tag, env in (("default", {}), ("threads8", {"GKM_COPY_THREADS": "8"}), ("threads16", {"GKM_COPY_THREADS": "16"}),
+                     ("threads32", {"GKM_COPY_THREADS": "32"})):
         res["e2e50"][tag] = e2e(50000, "50k", env, reps=2, kernel_type=2, L=11, k=7, d=3)
         print(tag, res["e2e50"][tag]["walls_s"], res["e2e50"][tag]["stats"], flush=True); save()
 
 if "e2e10" in what:
     res["e2e10"] = {}
-    for tag, env in (("default", {}), ("no_thp", {"GKM_NO_THP": "1"}), ("threads8", {"GKM_COPY_THREADS": "8"})):
+    for tag, env in (("default", {}), ("threads8", {"GKM_COPY_THREADS": "8"})):
         res["e2e10"][tag] = e2e(10000, "10k", env, reps=3, kernel_type=2, L=11, k=7, d=3)
         print(tag, res["e2e10"][tag]["walls_s"], res["e2e10"][tag]["stats"], flush=True); save()
 
