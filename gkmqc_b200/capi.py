@@ -118,6 +118,7 @@ def _declare(lib):
         ("gkmb200_decision_values", [P, I, I, I, I, c_dbl_p, ctypes.c_double, c_dbl_p]),
         ("gkmb200_get_stats", [P, ctypes.POINTER(gkmb200_stats)]),
         ("gkmb200_problem_index_layout", [P, c_int_p]),
+        ("gkmb200_problem_launch_shape", [P, c_int_p]),
         ("gkmb200_problem_image", [P, ctypes.c_void_p, ctypes.c_void_p, c_int_p]),
         ("gkmb200_resident_rows", [P, I, I, c_dbl_p, ctypes.c_long]),
         ("gkmb200_trim", []),
@@ -336,6 +337,13 @@ class Problem:
         """(column blocks, columns per block, first column) of the index variant's last call; (0, 0, 0) otherwise"""
         out = (ctypes.c_int * 3)()
         _check(self.lib.gkmb200_problem_index_layout(self.h, out), self.lib)
+        return tuple(out)
+
+    def launch_shape(self):
+        """(variant, TA, TB, dynamic shared memory bytes) of the last bit-sliced, lmer or mma launch for this problem on its
+        first GPU (variant 1 lmer, 2 diag, 3 mma; mma: TA = queries per CTA, TB = 8); (0, 0, 0, 0) if none"""
+        out = (ctypes.c_int * 4)()
+        _check(self.lib.gkmb200_problem_launch_shape(self.h, out), self.lib)
         return tuple(out)
 
     def bench_lower_resident(self, steps, warmup, flush_l2=True):

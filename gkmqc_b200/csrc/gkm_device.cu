@@ -118,6 +118,7 @@ struct gkm_image {
     int nblk, blk_cols;
     int blk_greedy;       /* the blocks were cut full-size first (index_split) */
     int part_lo, part_hi; /* the column range the blocks partition (that of the call that created them) */
+    int shape[4];         /* {variant, TA, TB, dynamic shared memory bytes} of the last bit-sliced, lmer or mma launch (slot 0) */
 };
 
 struct gkm_devstate {
@@ -448,6 +449,10 @@ static int launch_hist(const gkmb200_problem *p, const gkm_image *im, gkm_gpu *g
     if (grid.y > 65535u) { gkm_set_error("chunk has too many row tiles"); return 1; }
     CK(cudaLaunchKernel(fn, grid, dim3(threads, 1, 1), args, smem, st));
     g->nkernels++;
+    if (im == &p->dev->img[0]) { /* what gkmb200_problem_launch_shape reports */
+        int *s = const_cast<gkm_image *>(im)->shape;
+        s[0] = variant; s[1] = kp.TA; s[2] = kp.TB; s[3] = (int) smem;
+    }
     if (variant_out) *variant_out = variant;
     return 0;
 }
@@ -746,6 +751,19 @@ extern "C" int gkmb200_problem_index_layout(const gkmb200_problem *p, int *out)
     if (p->dev && p->dev->variant == GKM_KERNEL_INDEX && p->dev->img[0].blk) {
         out[0] = p->dev->img[0].nblk; out[1] = p->dev->img[0].blk_cols; out[2] = p->dev->img[0].part_lo;
     }
+    pthread_mutex_unlock(&g_lock);
+    return 0;
+}
+
+/* {variant, TA, TB, dynamic shared memory bytes} of the last bit-sliced, lmer or mma launch made for this problem on its
+ * first GPU (mma: TA = queries per CTA, TB = 8); zeros if none.  For tests: which tile shape a problem ran. */
+extern "C" int gkmb200_problem_launch_shape(const gkmb200_problem *p, int *out)
+{
+    if (!p || !out) { gkm_set_error("null argument"); return 1; }
+    out[0] = out[1] = out[2] = out[3] = 0;
+    pthread_mutex_lock(&g_lock);
+    if (p->dev)
+        for (int i = 0; i < 4; i++) out[i] = p->dev->img[0].shape[i];
     pthread_mutex_unlock(&g_lock);
     return 0;
 }

@@ -131,6 +131,9 @@ int gkmb200_problem_image(gkmb200_problem *p, uint32_t *planes, uint8_t *wend, i
 /* ---- measurement ---- */
 /* out[3] = {column blocks, columns per block, first column} of the index variant's last compute call on p (zeros: another variant ran) */
 int gkmb200_problem_index_layout(const gkmb200_problem *p, int *out);
+/* out[4] = {variant (1 lmer, 2 diag, 3 mma), TA, TB, dynamic shared memory bytes} of the last bit-sliced, lmer or mma launch
+ * made for p on its first GPU (mma: TA = queries per CTA, TB = targets per CTA); zeros if none */
+int gkmb200_problem_launch_shape(const gkmb200_problem *p, int *out);
 int gkmb200_get_stats(const gkmb200_problem *p, gkmb200_stats *out);
 /* `steps` timed passes over the full lower triangle with inputs and outputs resident in HBM;
  * ms_each[steps] = CUDA-event time of each pass; flush_l2 != 0 rewrites a >L2-sized buffer between passes */
