@@ -600,15 +600,8 @@ static int ensure_index(gkmb200_problem *p, gkm_gpu *g, gkm_image *im, int col_b
         const size_t sbytes = gkm_idx_scratch_bytes(P, L, &cub_bytes);
         void *scratch = NULL, *d_offs = NULL;
         size_t scratch_got = 0, offs_got = 0;
-        /* unit-weight kernel types get the compact slots with 15-bit columns (index_block_cap keeps the blocks below that) */
-        b->fmt = GKM_IDX_FMT_P32;
-        if (!gkm_opt_index_wide()) {
-            if (!p->weighted && nc <= GKM_IDX_C16_MAX_COLS) b->fmt = GKM_IDX_FMT_C16;
-            /* weighted types: 8-byte slots of three 20-bit postings where weights, columns and the overflow offsets fit
-             * (worst case 4/3 overflow entries per posting + padding) */
-            if (p->weighted && nc <= GKM_IDX_W20_MAX_COLS && p->param.M <= GKM_IDX_W20_MAX_WEIGHT &&
-                (4 * P) / 3 + 64 < 4 * (size_t) GKM_IDX_W20_MAX_UNITS) b->fmt = GKM_IDX_FMT_W20;
-        }
+        /* compact slots unless a limit of theirs is crossed (index_block_cap keeps the blocks below their column limits) */
+        b->fmt = gkm_idx_block_fmt(p->weighted, p->param.M, nc, P, gkm_opt_index_wide());
         int rc = pool_alloc(g, (void **) &b->tab, &b->tab_bytes, gkm_idx_tab_bytes(L, b->fmt)) ||
                  pool_alloc(g, (void **) &b->ovf, &b->ovf_bytes, gkm_idx_ovf_bytes(P, b->fmt)) ||
                  pool_alloc(g, &scratch, &scratch_got, sbytes) ||

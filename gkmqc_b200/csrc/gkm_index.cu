@@ -6,44 +6,33 @@
  *   cub radix sort        by code, stable: columns stay ascending   [library call, set-up only]
  *   gkm_idx_runs_kernel   run length of every distinct code; overflow demand of runs >= 5
  *   cub exclusive scan    overflow offsets             [library call, set-up only]
- *   gkm_idx_fill_kernel   slots {posting 0, 1, 2, posting 3 | pointer} and overflow lists
+ *   gkm_idx_fill_kernel   slots and overflow lists, one posting per thread (formats: gkm_index_slot.h)
  * Hot loop:
  *   gkm_index_rows_kernel one CTA of 1024 threads per query row; histogram row in shared
  *                         memory; fused fp64 epilogue identical to the other variants
  *                         (ascending-m sum, one division, no FMA; libgkm.c:576-582,1169-1179).
  */
 #include <cuda_runtime.h>
+#include <type_traits>
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
 
 #include "gkm_index_dev.h"
+#include "gkm_index_slot.h"
 #include "gkm_internal.h"
 
-#ifndef GKM_MAX_BINS
-#define GKM_MAX_BINS 16
-#endif
-
 #define GKM_IDX_THREADS 1024
-#ifndef GKM_IDX_UNROLL
 #define GKM_IDX_UNROLL 4
-#endif
-#ifndef GKM_IDX_WUNR
 #define GKM_IDX_WUNR 2 /* slot loads in flight per thread of the weighted two-CTA build (A/B: 3, 4) */
-#endif
 #define GKM_IDX_QCAP 64 /* queued overflow walks per warp: < 32 waiting + <= 32 new */
 #define GKM_IDX_LQCAP 32 /* long lists waiting for a whole-warp walk, per warp */
 /* Problems of several column blocks run two CTAs per SM only while both fit the 196 KB step of the L1/shared split
  * (blocks up to ~10 700 columns): beyond it L1 shrinks to 28 KB, and the two-CTA build then measured 2x SLOWER than
  * one CTA per SM (50k x 50k, 4 blocks of 12 512 columns: 1 300-1 590 ms against 704 ms).  A single block profits from
  * two CTAs up to the 227 KB limit (12 000 columns: 54.9 against 59.6 ms). */
-#ifndef GKM_IDX_TWO_SMEM
 #define GKM_IDX_TWO_SMEM (196u * 1024u)
-#endif
 #define GKM_IDX_SKEW_ONE_CTA 10.0 /* sum len^2 / P of the block: 2.4 on uniform 10k x 300 bp (L = 11), 3 on AT-rich, 6.5 at L = 10, 12.3 at L = 10 with 600-bp
                                       * windows (gkmQC's default: one CTA 220.6 ms, two 227.0), > 100 with 10 % poly-A */
-#ifndef GKM_IDX_W20_TWO
-#define GKM_IDX_W20_TWO 1 /* weighted compact slots: two CTAs per SM where the histogram rows fit (A/B: 0) */
-#endif
 /* queue entry: (list, bin row, weight).  Compact slots: 4 bytes; 16-byte slots: 8 bytes.  The queues are kept small on
  * purpose: at 10 000 columns two CTAs per SM need 2 x (80 KB histogram + queues + query) of shared memory, and
  * every KB beyond 196 KB per SM moves the L1/shared split to its last step (28 KB of L1 instead of 60), which
@@ -129,146 +118,41 @@ gkm_idx_runs_kernel(const unsigned long long *__restrict__ keys, uint32_t P, int
     }
     if (i >= P) return;
     runlen[i] = len;
-    /* overflow entries of a run of 5 or more: P32 keeps postings 3.. (32-bit entries, quads), C16 columns 2..
-     * (16-bit entries, octets); both padded with at least one end marker */
-    if (fmt == GKM_IDX_FMT_C16) {
-        const uint32_t units = (len >= 5) ? GKM_IDX_C16_UNITS(len) : 0u;
-        need[i] = 8u * (units + (units >= GKM_IDX_LONG_UNITS ? 1u : 0u)); /* long lists carry a header unit */
-    } else if (fmt == GKM_IDX_FMT_W20) {
-        const uint32_t units = (len >= 4) ? GKM_IDX_W20_UNITS(len) : 0u;
-        need[i] = 4u * (units + (units >= GKM_IDX_LONG_UNITS ? 1u : 0u));
-    } else {
-        const uint32_t units = (len >= 5) ? GKM_IDX_P32_UNITS(len) : 0u;
-        need[i] = 4u * (units + (units >= GKM_IDX_LONG_UNITS ? 1u : 0u));
-    }
+    need[i] = gkm_idx_ovf_need(fmt, len);
 }
 
+/* the head of the run that holds posting i: gallop back, then bisect */
+__device__ __forceinline__ uint32_t idx_run_head(const unsigned long long *keys, const uint32_t *runlen, uint32_t i, uint32_t code)
+{
+    if (runlen[i] != 0) return i;
+    uint32_t hi = i, lo = 0, step = 1; /* [hi, i] holds `code` */
+    for (;;) {
+        if (hi < step) { lo = 0; break; }
+        const uint32_t probe = hi - step;
+        if ((uint32_t) (keys[probe] >> 32) != code) { lo = probe + 1; break; }
+        hi = probe;
+        step <<= 1;
+    }
+    return idx_lower(keys, lo, hi, code);
+}
+
+/* plain stores; the three 20-bit fields of a W20 slot are written by three threads into two 32-bit words: AND */
+struct idx_store {
+    template <class T> static __device__ __forceinline__ void st(T *p, T v) { *p = v; }
+    static __device__ __forceinline__ void and_(uint32_t *p, uint32_t v) { atomicAnd(p, v); }
+};
+
+template <int FMT>
 __global__ void __launch_bounds__(256)
 gkm_idx_fill_kernel(const unsigned long long *__restrict__ keys, uint32_t P, const uint32_t *__restrict__ runlen,
-                    const uint32_t *__restrict__ ovfofs, uint4 *__restrict__ tab, uint32_t *__restrict__ ovf)
+                    const uint32_t *__restrict__ ovfofs, void *__restrict__ tab, uint32_t *__restrict__ ovf)
 {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= P) return;
     const unsigned long long key = keys[i];
-    const uint32_t code = (uint32_t) (key >> 32);
-    uint32_t lb = i;
-    if (runlen[i] == 0) {
-        /* not a head: gallop back, then bisect */
-        uint32_t hi = i, lo = 0, step = 1; /* [hi, i] holds `code` */
-        for (;;) {
-            if (hi < step) { lo = 0; break; }
-            const uint32_t probe = hi - step;
-            if ((uint32_t) (keys[probe] >> 32) != code) { lo = probe + 1; break; }
-            hi = probe;
-            step <<= 1;
-        }
-        lb = idx_lower(keys, lo, hi, code);
-    }
-    const uint32_t len = runlen[lb], r = i - lb;
-    const uint32_t posting = gkm_idx_posting((uint32_t) (key >> 8) & GKM_IDX_COL_MASK, (uint32_t) key & 0xFFu);
-    uint32_t *slot = reinterpret_cast<uint32_t *>(tab + code);
-    const uint32_t units = (len >= 5) ? GKM_IDX_P32_UNITS(len) : 0u;
-    const bool lng = units >= GKM_IDX_LONG_UNITS;
-    const uint32_t data = ovfofs[lb] + (lng ? 4u : 0u); /* behind the header unit */
-    if (r < 3 || (r == 3 && len == 4)) {
-        slot[r] = posting;
-    } else {
-        ovf[data + r - 3] = posting;
-    }
-    if (r == 0 && len >= 5) {
-        slot[3] = GKM_IDX_PTR | ovfofs[lb] | (lng ? GKM_IDX_LONG : 0u);
-        if (lng) { ovf[ovfofs[lb]] = units; ovf[ovfofs[lb] + 1] = 0; ovf[ovfofs[lb] + 2] = 0; ovf[ovfofs[lb] + 3] = 0; }
-        for (uint32_t t = len - 3; t < 4u * units; t++) ovf[data + t] = GKM_IDX_EMPTY; /* lists are read 16 bytes at a time */
-    }
-}
-
-__global__ void __launch_bounds__(256)
-gkm_idx_fill_c16_kernel(const unsigned long long *__restrict__ keys, uint32_t P, const uint32_t *__restrict__ runlen,
-                        const uint32_t *__restrict__ ovfofs, uint2 *__restrict__ tab, uint16_t *__restrict__ ovf)
-{
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= P) return;
-    const unsigned long long key = keys[i];
-    const uint32_t code = (uint32_t) (key >> 32);
-    uint32_t lb = i;
-    if (runlen[i] == 0) {
-        uint32_t hi = i, lo = 0, step = 1;
-        for (;;) {
-            if (hi < step) { lo = 0; break; }
-            const uint32_t probe = hi - step;
-            if ((uint32_t) (keys[probe] >> 32) != code) { lo = probe + 1; break; }
-            hi = probe;
-            step <<= 1;
-        }
-        lb = idx_lower(keys, lo, hi, code);
-    }
-    const uint32_t len = runlen[lb], r = i - lb;
-    const uint16_t col = (uint16_t) ((key >> 8) & 0x7FFFu);
-    uint16_t *slot = reinterpret_cast<uint16_t *>(tab + code);
-    if (len <= 4) {
-        slot[r] = col;
-    } else {
-        const uint32_t units = GKM_IDX_C16_UNITS(len);
-        const bool lng = units >= GKM_IDX_LONG_UNITS;
-        const uint32_t data = ovfofs[lb] + (lng ? 8u : 0u); /* behind the header unit */
-        if (r < 2) slot[r] = col;
-        else ovf[data + r - 2] = col;
-        if (r == 0) {
-            reinterpret_cast<uint32_t *>(tab + code)[1] = GKM_IDX_PTR | ovfofs[lb] | (lng ? GKM_IDX_LONG : 0u);
-            if (lng) {
-                uint32_t *h = reinterpret_cast<uint32_t *>(ovf + ovfofs[lb]);
-                h[0] = units; h[1] = 0; h[2] = 0; h[3] = 0;
-            }
-            for (uint32_t t = len - 2; t < 8u * units; t++) ovf[data + t] = GKM_IDX_C16_NONE;
-        }
-    }
-}
-
-/* W20: the three 20-bit fields of a slot are written by three different threads into two shared 32-bit words that
- * start as all ones: each thread ANDs its own bits in */
-__global__ void __launch_bounds__(256)
-gkm_idx_fill_w20_kernel(const unsigned long long *__restrict__ keys, uint32_t P, const uint32_t *__restrict__ runlen,
-                        const uint32_t *__restrict__ ovfofs, uint2 *__restrict__ tab, uint32_t *__restrict__ ovf)
-{
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= P) return;
-    const unsigned long long key = keys[i];
-    const uint32_t code = (uint32_t) (key >> 32);
-    uint32_t lb = i;
-    if (runlen[i] == 0) {
-        uint32_t hi = i, lo = 0, step = 1;
-        for (;;) {
-            if (hi < step) { lo = 0; break; }
-            const uint32_t probe = hi - step;
-            if ((uint32_t) (keys[probe] >> 32) != code) { lo = probe + 1; break; }
-            hi = probe;
-            step <<= 1;
-        }
-        lb = idx_lower(keys, lo, hi, code);
-    }
-    const uint32_t len = runlen[lb], r = i - lb;
-    const uint32_t col = (uint32_t) (key >> 8) & GKM_IDX_W20_COL_MASK, wt = (uint32_t) key & 0xFFu;
-    const uint32_t p20 = col | (wt << GKM_IDX_W20_COL_BITS);
-    uint32_t *slot = reinterpret_cast<uint32_t *>(tab + code);
-    const uint32_t units = (len >= 4) ? GKM_IDX_W20_UNITS(len) : 0u;
-    const bool lng = units >= GKM_IDX_LONG_UNITS;
-    const uint32_t data = ovfofs[lb] + (lng ? 4u : 0u); /* behind the header unit */
-    if (r == 0) {
-        atomicAnd(slot, p20 | ~0xFFFFFu);
-        if (len <= 3) atomicAnd(slot + 1, ~GKM_IDX_PTR);
-        else {
-            atomicAnd(slot + 1, GKM_IDX_PTR | ((ovfofs[lb] >> 2) << 9) | (lng ? (GKM_IDX_LONG << 8) : 0u) | 0xFFu);
-            if (lng) { ovf[ovfofs[lb]] = units; ovf[ovfofs[lb] + 1] = 0; ovf[ovfofs[lb] + 2] = 0; ovf[ovfofs[lb] + 3] = 0; }
-            for (uint32_t t = len - 2; t < 4u * units; t++) ovf[data + t] = GKM_IDX_EMPTY;
-        }
-    } else if (r == 1) {
-        atomicAnd(slot, (p20 << 20) | 0xFFFFFu);
-        atomicAnd(slot + 1, (p20 >> 12) | ~0xFFu);
-    } else if (len == 3) {
-        atomicAnd(slot + 1, (p20 << 8) | ~(0xFFFFFu << 8));
-    } else {
-        ovf[data + r - 2] = gkm_idx_posting(col, wt);
-    }
+    const uint32_t code = (uint32_t) (key >> 32), lb = idx_run_head(keys, runlen, i, code);
+    uint32_t *slot = reinterpret_cast<uint32_t *>(tab) + (size_t) code * (FMT == GKM_IDX_FMT_P32 ? 4 : 2);
+    gkm_idx_place<FMT, idx_store>(i - lb, runlen[lb], ovfofs[lb], (uint32_t) (key >> 8) & GKM_IDX_COL_MASK, (uint32_t) key & 0xFFu, slot, ovf);
 }
 
 /* 4^L slots and one spare, always empty: where the probes of lanes that ran out of query L-mers go */
@@ -317,9 +201,9 @@ int gkm_idx_build(const gkm_idx_build_args *a, cudaStream_t st)
         uint32_t *ovfofs = (uint32_t *) keys_a; /* the unsorted keys are dead now */
         cub_bytes = a->cub_bytes;
         if ((e = cub::DeviceScan::ExclusiveSum(cub_tmp, cub_bytes, need, ovfofs, (int) P, st)) != cudaSuccess) goto fail;
-        if (a->fmt == GKM_IDX_FMT_C16) gkm_idx_fill_c16_kernel<<<blocks, 256, 0, st>>>(keys_b, (uint32_t) P, runlen, ovfofs, (uint2 *) a->tab, (uint16_t *) a->ovf);
-        else if (a->fmt == GKM_IDX_FMT_W20) gkm_idx_fill_w20_kernel<<<blocks, 256, 0, st>>>(keys_b, (uint32_t) P, runlen, ovfofs, (uint2 *) a->tab, a->ovf);
-        else gkm_idx_fill_kernel<<<blocks, 256, 0, st>>>(keys_b, (uint32_t) P, runlen, ovfofs, (uint4 *) a->tab, a->ovf);
+        if (a->fmt == GKM_IDX_FMT_C16) gkm_idx_fill_kernel<GKM_IDX_FMT_C16><<<blocks, 256, 0, st>>>(keys_b, (uint32_t) P, runlen, ovfofs, a->tab, a->ovf);
+        else if (a->fmt == GKM_IDX_FMT_W20) gkm_idx_fill_kernel<GKM_IDX_FMT_W20><<<blocks, 256, 0, st>>>(keys_b, (uint32_t) P, runlen, ovfofs, a->tab, a->ovf);
+        else gkm_idx_fill_kernel<GKM_IDX_FMT_P32><<<blocks, 256, 0, st>>>(keys_b, (uint32_t) P, runlen, ovfofs, a->tab, a->ovf);
     }
     if ((e = cudaGetLastError()) != cudaSuccess) goto fail;
     return 0;
@@ -331,138 +215,51 @@ fail:
 /* ------------------------------------------------------------------ */
 /* hot loop                                                             */
 /* ------------------------------------------------------------------ */
-/* One posting against the wanted column range [blo, bhi): H[b] += v iff blo <= b < bhi.  The column field of an
- * empty word / end marker is all ones, so the range test is the validity test as well.  (ptxas turns a
- * predicated red.shared back into a branch around ATOMS, so this is plain C++.) */
-template <bool RANGE>
-__device__ __forceinline__ void idx_red(int32_t *Hm, uint32_t b, uint32_t blo, uint32_t bhi, int v)
+/* the hit callback of the row kernel: a shared (hot bins) or global (cold bins) atomic into the bin row Hm */
+struct idx_add {
+    int32_t *Hm;
+    __device__ __forceinline__ void operator()(uint32_t i, int v) const { atomicAdd(Hm + i, v); }
+};
+
+template <int FMT> using idx_slot_t = std::conditional_t<FMT == GKM_IDX_FMT_P32, uint4, uint2>;
+
+/* inline postings of one slot; returns the offset of the overflow list that still has to be walked, or ~0u */
+template <bool WEIGHTED, bool RANGE, int FMT>
+__device__ __forceinline__ uint32_t idx_slot(const idx_slot_t<FMT> sl, int32_t *Hm, uint32_t blo, uint32_t bhi, int w)
 {
-    bool ok = b < bhi;
-    if (RANGE) ok = ok && b >= blo;
-    if (ok) atomicAdd(Hm + (RANGE ? b - blo : b), v);
+    if constexpr (FMT == GKM_IDX_FMT_P32) return gkm_idx_slot<FMT, WEIGHTED, RANGE>(sl.x, sl.y, sl.z, sl.w, blo, bhi, w, idx_add{Hm});
+    else return gkm_idx_slot<FMT, WEIGHTED, RANGE>(sl.x, sl.y, 0u, 0u, blo, bhi, w, idx_add{Hm});
 }
 
-template <bool WEIGHTED, bool RANGE>
-__device__ __forceinline__ void idx_hit(int32_t *Hm, uint32_t e, uint32_t blo, uint32_t bhi, int w)
+/* the first 16-byte unit of the overflow list at entry ofs (16-bit entries for C16, 32-bit ones otherwise) */
+template <int FMT>
+__device__ __forceinline__ const uint4 *idx_units(const uint32_t *ovf, uint32_t ofs)
 {
-    idx_red<RANGE>(Hm, e & GKM_IDX_COL_MASK, blo, bhi, WEIGHTED ? w * (int) (e >> GKM_IDX_COL_BITS) : 1);
+    return FMT == GKM_IDX_FMT_C16 ? reinterpret_cast<const uint4 *>(reinterpret_cast<const uint16_t *>(ovf) + ofs)
+                                  : reinterpret_cast<const uint4 *>(ovf + ofs);
 }
 
-/* ---- 16-byte slots (GKM_IDX_FMT_P32) ---- */
-/* inline postings of one slot; returns the offset of the overflow list that still has to be walked, or ~0u.
- * Lists are sorted by column, so a list whose third posting is behind the range needs no walk. */
-template <bool WEIGHTED, bool RANGE>
-__device__ __forceinline__ uint32_t idx_slot(const uint4 sl, int32_t *Hm, uint32_t blo, uint32_t bhi, int w)
+/* one overflow list (lists of five or more: 1.7 % of the slots at 10k x 300 bp) by one lane, 16 bytes at a time; a
+ * long one from behind its header unit */
+template <bool WEIGHTED, bool RANGE, int FMT>
+__device__ __forceinline__ void idx_walk(const gkm_idx_rowargs &r, uint32_t ofs, bool lng, int32_t *Hm, uint32_t blo, uint32_t bhi, int w)
 {
-    idx_hit<WEIGHTED, RANGE>(Hm, sl.x, blo, bhi, w);
-    idx_hit<WEIGHTED, RANGE>(Hm, sl.y, blo, bhi, w);
-    idx_hit<WEIGHTED, RANGE>(Hm, sl.z, blo, bhi, w);
-    if (!(sl.w & GKM_IDX_PTR)) { idx_hit<WEIGHTED, RANGE>(Hm, sl.w, blo, bhi, w); return ~0u; }
-    return (sl.w != GKM_IDX_EMPTY && (sl.z & GKM_IDX_COL_MASK) < bhi) ? (sl.w & ~GKM_IDX_PTR) : ~0u;
-}
-
-/* postings 3.. of a list of five or more (1.7 % of the slots at 10k x 300 bp), 16 bytes at a time */
-template <bool WEIGHTED, bool RANGE>
-__device__ __forceinline__ void idx_walk(const uint32_t *__restrict__ ovf, uint32_t ofs, int32_t *Hm, uint32_t blo, uint32_t bhi, int w)
-{
-    const uint4 *q = reinterpret_cast<const uint4 *>(ovf + ofs);
+    const uint4 *q = idx_units<FMT>(r.ovf, ofs + (lng ? gkm_idx_unit_entries(FMT) : 0u));
     for (;;) {
         const uint4 v = __ldg(q++);
-        idx_hit<WEIGHTED, RANGE>(Hm, v.x, blo, bhi, w);
-        idx_hit<WEIGHTED, RANGE>(Hm, v.y, blo, bhi, w);
-        idx_hit<WEIGHTED, RANGE>(Hm, v.z, blo, bhi, w);
-        idx_hit<WEIGHTED, RANGE>(Hm, v.w, blo, bhi, w);
-        if ((v.w & GKM_IDX_COL_MASK) >= bhi) break;
+        if (!gkm_idx_unit<FMT, WEIGHTED, RANGE>(v.x, v.y, v.z, v.w, blo, bhi, w, idx_add{Hm})) break;
     }
 }
 
-/* ---- compact slots (GKM_IDX_FMT_C16): unit weights, 16-bit columns; 0xFFFF (none) fails the range test ---- */
-template <bool RANGE>
-__device__ __forceinline__ uint32_t idx_slot16(const uint2 sl, int32_t *Hm, uint32_t blo, uint32_t bhi)
-{
-    const uint32_t c1 = sl.x >> 16, c3 = sl.y >> 16;
-    idx_red<RANGE>(Hm, sl.x & 0xFFFFu, blo, bhi, 1);
-    idx_red<RANGE>(Hm, c1, blo, bhi, 1);
-    if (!(sl.y & GKM_IDX_PTR) || c3 == GKM_IDX_C16_NONE) {
-        idx_red<RANGE>(Hm, sl.y & 0xFFFFu, blo, bhi, 1);
-        idx_red<RANGE>(Hm, c3, blo, bhi, 1);
-        return ~0u;
-    }
-    return (c1 < bhi) ? (sl.y & ~GKM_IDX_PTR) : ~0u;
-}
-
-/* columns 2.. of a list of five or more, eight at a time */
-template <bool RANGE>
-__device__ __forceinline__ void idx_walk16(const uint32_t *__restrict__ ovf, uint32_t ofs, int32_t *Hm, uint32_t blo, uint32_t bhi)
-{
-    const uint4 *q = reinterpret_cast<const uint4 *>(reinterpret_cast<const uint16_t *>(ovf) + ofs);
-    for (;;) {
-        const uint4 v = __ldg(q++);
-        idx_red<RANGE>(Hm, v.x & 0xFFFFu, blo, bhi, 1); idx_red<RANGE>(Hm, v.x >> 16, blo, bhi, 1);
-        idx_red<RANGE>(Hm, v.y & 0xFFFFu, blo, bhi, 1); idx_red<RANGE>(Hm, v.y >> 16, blo, bhi, 1);
-        idx_red<RANGE>(Hm, v.z & 0xFFFFu, blo, bhi, 1); idx_red<RANGE>(Hm, v.z >> 16, blo, bhi, 1);
-        idx_red<RANGE>(Hm, v.w & 0xFFFFu, blo, bhi, 1); idx_red<RANGE>(Hm, v.w >> 16, blo, bhi, 1);
-        if ((v.w >> 16) >= bhi) break;
-    }
-}
-
-/* ---- compact slots with weights (GKM_IDX_FMT_W20): three 20-bit postings (column : 14 | weight : 6) in 8 bytes ----
- * x = p0 | p1 << 20, y = p1 >> 12 | p2 << 8 | flags << 28.  Four or more postings: p0 and p1 inline, y bit 31 set, y bits
- * 9..30 = offset of postings 2.. in the overflow array in 16-byte units (entries there are the 32-bit postings of the
- * P32 format: the walks are shared), y bit 8 = GKM_IDX_LONG.  A column field of all ones (0x3FFF: blocks hold at most
- * 16 352 columns) fails the range test; an empty slot is all ones and is told from a pointer by its first column. */
-template <bool RANGE>
-__device__ __forceinline__ uint32_t idx_slot20(const uint2 sl, int32_t *Hm, uint32_t blo, uint32_t bhi, int w)
-{
-    const uint32_t p0 = sl.x & 0xFFFFFu, p1 = (sl.x >> 20) | ((sl.y & 0xFFu) << 12);
-    const uint32_t c0 = p0 & GKM_IDX_W20_COL_MASK, c1 = p1 & GKM_IDX_W20_COL_MASK;
-    idx_red<RANGE>(Hm, c0, blo, bhi, w * (int) (p0 >> GKM_IDX_W20_COL_BITS));
-    idx_red<RANGE>(Hm, c1, blo, bhi, w * (int) (p1 >> GKM_IDX_W20_COL_BITS));
-    if (!(sl.y & GKM_IDX_PTR) || c0 == GKM_IDX_W20_COL_MASK) {
-        const uint32_t p2 = (sl.y >> 8) & 0xFFFFFu;
-        idx_red<RANGE>(Hm, p2 & GKM_IDX_W20_COL_MASK, blo, bhi, w * (int) (p2 >> GKM_IDX_W20_COL_BITS));
-        return ~0u;
-    }
-    return (c1 < bhi) ? ((((sl.y >> 9) & 0x3FFFFFu) << 2) | ((sl.y >> 8) & GKM_IDX_LONG)) : ~0u;
-}
-
-/* A long list (GKM_IDX_LONG), walked by the whole warp: lane l takes the units l, l + 32, ...  Equal columns are
- * adjacent in a list (a column with a repeat owns a run of postings): each lane folds the runs inside its unit
- * before it touches the histogram, so a homopolymer costs one atomic per unit instead of eight on one address. */
+/* a long list (GKM_IDX_LONG), walked by the whole warp: lane l takes the units l, l + 32, ... */
 template <bool WEIGHTED, bool RANGE, int FMT>
 __device__ __forceinline__ void idx_walk_long(const uint32_t *__restrict__ ovf, uint32_t ofs, int32_t *Hm, uint32_t blo, uint32_t bhi, int w, int lane)
 {
-    constexpr bool C16 = FMT == GKM_IDX_FMT_C16;
-    const uint4 *q = C16 ? reinterpret_cast<const uint4 *>(reinterpret_cast<const uint16_t *>(ovf) + ofs)
-                         : reinterpret_cast<const uint4 *>(ovf + ofs);
+    const uint4 *q = idx_units<FMT>(ovf, ofs);
     const uint32_t units = __ldg(q).x;
     for (uint32_t u = (uint32_t) lane; u < units; u += 32u) {
         const uint4 v = __ldg(q + 1 + u);
-        if constexpr (C16) {
-            uint32_t cur = v.x & 0xFFFFu;
-            if (cur >= bhi) break; /* sorted by column: nothing wanted in this unit or behind it */
-            int cnt = 1;
-            const uint32_t c[7] = { v.x >> 16, v.y & 0xFFFFu, v.y >> 16, v.z & 0xFFFFu, v.z >> 16, v.w & 0xFFFFu, v.w >> 16 };
-#pragma unroll
-            for (int t = 0; t < 7; t++) {
-                if (c[t] == cur) cnt++;
-                else { idx_red<RANGE>(Hm, cur, blo, bhi, cnt); cur = c[t]; cnt = 1; }
-            }
-            idx_red<RANGE>(Hm, cur, blo, bhi, cnt);
-        } else {
-            uint32_t cur = v.x & GKM_IDX_COL_MASK;
-            if (cur >= bhi) break;
-            int acc = WEIGHTED ? w * (int) (v.x >> GKM_IDX_COL_BITS) : 1;
-            const uint32_t e[3] = { v.y, v.z, v.w };
-#pragma unroll
-            for (int t = 0; t < 3; t++) {
-                const uint32_t col = e[t] & GKM_IDX_COL_MASK;
-                const int val = WEIGHTED ? w * (int) (e[t] >> GKM_IDX_COL_BITS) : 1;
-                if (col == cur) acc += val;
-                else { idx_red<RANGE>(Hm, cur, blo, bhi, acc); cur = col; acc = val; }
-            }
-            idx_red<RANGE>(Hm, cur, blo, bhi, acc);
-        }
+        if (!gkm_idx_unit_folded<FMT, WEIGHTED, RANGE>(v.x, v.y, v.z, v.w, blo, bhi, w, idx_add{Hm})) break;
     }
 }
 
@@ -486,14 +283,6 @@ template <> struct idx_qe<false> {
     static __device__ __forceinline__ int w(type e) { return (int) (e.y >> 8); }
     static __device__ __forceinline__ type none() { return make_uint2(0u, 0u); }
 };
-
-/* one list by the lane that owns the entry; a long one from behind its header unit */
-template <bool WEIGHTED, bool RANGE, int FMT>
-__device__ __forceinline__ void idx_walk_own(const gkm_idx_rowargs &r, uint32_t ofs, bool lng, int32_t *He, uint32_t blo, uint32_t bhi, int w)
-{
-    if constexpr (FMT == GKM_IDX_FMT_C16) idx_walk16<RANGE>(r.ovf, ofs + (lng ? 8u : 0u), He, blo, bhi);
-    else idx_walk<WEIGHTED, RANGE>(r.ovf, ofs + (lng ? 4u : 0u), He, blo, bhi, w);
-}
 
 /* the long queue of a warp, one list after the other, each by all 32 lanes */
 template <bool WEIGHTED, bool RANGE, int FMT>
@@ -535,16 +324,13 @@ __device__ __forceinline__ void idx_probe_cold(const gkm_idx_rowargs &r, int t_b
         for (int xi = ph; xi < nq; xi += nph) {
             const uint32_t y = xq[xi] ^ dx;
             const int w = WEIGHTED ? (int) wq[xi] : 1;
-            uint32_t o;
-            if constexpr (FMT == GKM_IDX_FMT_C16) o = idx_slot16<RANGE>(__ldg(reinterpret_cast<const uint2 *>(r.tab) + y), Hm, blo, bhi);
-            else if constexpr (FMT == GKM_IDX_FMT_W20) o = idx_slot20<RANGE>(__ldg(reinterpret_cast<const uint2 *>(r.tab) + y), Hm, blo, bhi, w);
-            else o = idx_slot<WEIGHTED, RANGE>(__ldg(reinterpret_cast<const uint4 *>(r.tab) + y), Hm, blo, bhi, w);
+            const uint32_t o = idx_slot<WEIGHTED, RANGE, FMT>(__ldg(reinterpret_cast<const idx_slot_t<FMT> *>(r.tab) + y), Hm, blo, bhi, w);
             if (o == ~0u) continue;
             if (o & GKM_IDX_LONG) {
                 const int pos = atomicAdd(lqcnt, 1);
                 if (pos < GKM_IDX_LQCAP) { lq[pos] = QE::make(o, mrow, w); continue; }
             }
-            idx_walk_own<WEIGHTED, RANGE, FMT>(r, o & ~GKM_IDX_LONG, o & GKM_IDX_LONG, Hm, blo, bhi, w);
+            idx_walk<WEIGHTED, RANGE, FMT>(r, o & ~GKM_IDX_LONG, o & GKM_IDX_LONG, Hm, blo, bhi, w);
         }
     }
     __syncwarp();
@@ -570,7 +356,7 @@ __device__ __forceinline__ void idx_drain(const gkm_idx_rowargs &r, typename idx
         lqn += __popc(lm);
         have = have && !lng;
     }
-    if (have) idx_walk_own<WEIGHTED, RANGE, FMT>(r, QE::ofs(e), lng, Hb + (size_t) QE::mrow(e) * (size_t) ldh, blo, bhi, QE::w(e));
+    if (have) idx_walk<WEIGHTED, RANGE, FMT>(r, QE::ofs(e), lng, Hb + (size_t) QE::mrow(e) * (size_t) ldh, blo, bhi, QE::w(e));
 }
 
 /* Probes of the masks [t_begin, t_end) into the HOT bins (shared memory H; bin row 0 of H holds m = mbase).
@@ -588,8 +374,7 @@ __device__ __forceinline__ void idx_probe_hot(const gkm_idx_rowargs &r, int t_be
     typedef idx_qe<FMT == GKM_IDX_FMT_C16> QE;
     const int tid = (int) threadIdx.x, lane = tid & 31;
     const uint32_t lt = (1u << lane) - 1u;
-    const uint4 *__restrict__ tab = reinterpret_cast<const uint4 *>(r.tab);
-    const uint2 *__restrict__ tab16 = reinterpret_cast<const uint2 *>(r.tab);
+    const idx_slot_t<FMT> *__restrict__ tab = reinterpret_cast<const idx_slot_t<FMT> *>(r.tab);
     typename QE::type *lq = queue + GKM_IDX_QCAP; /* long queue of this warp */
     int qn = 0, lqn = 0;                          /* queued walks of this warp (warp-uniform) */
     for (int t0 = t_begin; t0 < t_end; t0 += GKM_IDX_THREADS) {
@@ -608,8 +393,7 @@ __device__ __forceinline__ void idx_probe_hot(const gkm_idx_rowargs &r, int t_be
         const int n_it = (nq + nph - 1) / nph;     /* the same for every lane */
         for (int it = 0; it < n_it; it += UNR) {
             int w[UNR];
-            uint4 sl[UNR];
-            uint2 sc[UNR];
+            idx_slot_t<FMT> sl[UNR];
 #pragma unroll
             for (int u = 0; u < UNR; u++) {
                 const int xi = ph + (it + u) * nph;
@@ -617,14 +401,11 @@ __device__ __forceinline__ void idx_probe_hot(const gkm_idx_rowargs &r, int t_be
                 /* a probe past the last L-mer reads the spare slot behind the table: always empty, never a hit */
                 const uint32_t y = ok ? (xq[xi] ^ dx) : r.nslots;
                 w[u] = (WEIGHTED && ok) ? (int) wq[xi] : 1;
-                if constexpr (FMT != GKM_IDX_FMT_P32) sc[u] = __ldg(tab16 + y); else sl[u] = __ldg(tab + y);
+                sl[u] = __ldg(tab + y);
             }
 #pragma unroll
             for (int u = 0; u < UNR; u++) {
-                uint32_t o;
-                if constexpr (FMT == GKM_IDX_FMT_C16) o = idx_slot16<RANGE>(sc[u], Hm, blo, bhi_l);
-                else if constexpr (FMT == GKM_IDX_FMT_W20) o = idx_slot20<RANGE>(sc[u], Hm, blo, bhi_l, w[u]);
-                else o = idx_slot<WEIGHTED, RANGE>(sl[u], Hm, blo, bhi_l, w[u]);
+                const uint32_t o = idx_slot<WEIGHTED, RANGE, FMT>(sl[u], Hm, blo, bhi_l, w[u]);
                 const uint32_t mk = __ballot_sync(0xFFFFFFFFu, o != ~0u);
                 if (mk) {
                     if (o != ~0u) queue[qn + __popc(mk & lt)] = QE::make(o, mrow, w[u]);
@@ -768,7 +549,7 @@ int gkm_idx_rows(const gkm_kparams *kp, const gkm_idx_rowargs *ra, int weighted,
      * slower (28 288 sequences: 272 ms against 228 ms), and the 16-byte-slot code spills at 32 registers
      * (wgkm at 10k: 70 ms against 49 ms), so that format always runs one CTA per SM. */
     const unsigned pair = 2u * (gkm_idx_row_smem(kp->nbins, (ra->blk_cols + 31) & ~31, ra->maxq, weighted, c16) + 1280u);
-    bool two = ra->fmt != GKM_IDX_FMT_P32 && (!weighted || GKM_IDX_W20_TWO) && pair <= (ra->nblk > 1 ? GKM_IDX_TWO_SMEM : 227u * 1024u);
+    bool two = ra->fmt != GKM_IDX_FMT_P32 && pair <= (ra->nblk > 1 ? GKM_IDX_TWO_SMEM : 227u * 1024u);
     /* weighted types on input with repeats (long-tailed rows): one CTA per SM (everything-mixed workload of
      * tools/nonuniform.py: 80 against 95 ms; uniform input: 50.4 against 47.4 ms the other way round) */
     if (weighted && ra->skew > GKM_IDX_SKEW_ONE_CTA) two = false;

@@ -54,14 +54,14 @@ extern "C" {
 /* compact slots of the weighted kernel types (4, 5): 8 bytes = three 20-bit postings (column : 14 | weight : 6) + 4 flag
  * bits; four or more postings: two inline + pointer to 32-bit postings (the P32 entry format) in the overflow array.
  * Needs weights <= 63 (M <= 63; gkmQC's default is 50), <= 16 352 columns per block and < 2^22 overflow units;
- * otherwise the 16-byte slots are used.  Same table size and sector density as C16 (gkm_index.cu: idx_slot20). */
+ * otherwise the 16-byte slots are used.  Same table size and sector density as C16.  The three formats are written
+ * out in gkm_index_slot.h. */
 #define GKM_IDX_FMT_W20 2
 #define GKM_IDX_W20_COL_BITS 14
 #define GKM_IDX_W20_COL_MASK 0x3FFFu
 #define GKM_IDX_W20_MAX_COLS 16352
 #define GKM_IDX_W20_MAX_WEIGHT 63
 #define GKM_IDX_W20_MAX_UNITS (1u << 22)
-#define GKM_IDX_W20_UNITS(len) ((((len) - 2u + 4u) & ~3u) >> 2)
 /* long lists (repeats, homopolymers): an overflow list of GKM_IDX_LONG_UNITS or more 16-byte units is not walked by
  * the lane that met it (one dependent load per unit: a 20 000-posting poly-A list cost that lane ~1 ms, and every
  * third random row meets it) but by its whole warp, a unit per lane.  Such a list starts with a 16-byte header
@@ -69,9 +69,6 @@ extern "C" {
  * bits of the offset are free). */
 #define GKM_IDX_LONG 1u
 #define GKM_IDX_LONG_UNITS 8u
-/* units (16 bytes = 8 columns / 4 postings) of the overflow part of a list of `len` postings, end marker included */
-#define GKM_IDX_C16_UNITS(len) ((((len) - 2u + 8u) & ~7u) >> 3)
-#define GKM_IDX_P32_UNITS(len) ((((len) - 3u + 4u) & ~3u) >> 2)
 #define GKM_IDX_HOT_BINS 2            /* bins d and d-1 (99 % of the hits) live in shared memory, the others in L2 */
 
 #if defined(__CUDACC__)
@@ -108,6 +105,10 @@ long long gkm_idx_cold_count(int L, int d);
 
 /* is the variant applicable at all (table and masks representable)? */
 int gkm_idx_supported(int L, int d, int nbins);
+
+/* the slot format of a column block of ncols columns and `postings` postings: C16 for unit weights, W20 for weights
+ * where the weights (M), the columns and the overflow units fit, P32 otherwise and whenever `wide` is set */
+int gkm_idx_block_fmt(int weighted, int M, int ncols, size_t postings, int wide);
 
 /* rough cost model used by kernel = auto (DESIGN.md 4.4): estimated device milliseconds */
 double gkm_idx_cost_ms(int L, int d, int weighted, long long rows, double mean_query_lmers, double col_blocks, long long entries,

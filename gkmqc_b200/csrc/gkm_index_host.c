@@ -1,6 +1,6 @@
 /* gkm_index_host.c -- host logic of the "index" kernel variant (gkm_index.h): the list of
- * XOR masks a query L-mer is probed with, applicability, and the cost model behind
- * kernel = auto.  Pure C, no CUDA: covered by the CPU test tier. */
+ * XOR masks a query L-mer is probed with, applicability, the slot format of a column block,
+ * and the cost model behind kernel = auto.  Pure C, no CUDA: covered by the CPU test tier. */
 #include <math.h>
 
 #include "gkm_index.h"
@@ -90,6 +90,16 @@ int gkm_idx_supported(int L, int d, int nbins)
     if (d < 0 || d > 15 || nbins != d + 1) return 0;
     const long long nd = gkm_idx_delta_count(L, d);
     return nd > 0 && nd <= (64LL << 20); /* the mask list itself must stay small (256 MB) */
+}
+
+int gkm_idx_block_fmt(int weighted, int M, int ncols, size_t postings, int wide)
+{
+    if (wide) return GKM_IDX_FMT_P32;
+    if (!weighted) return ncols <= GKM_IDX_C16_MAX_COLS ? GKM_IDX_FMT_C16 : GKM_IDX_FMT_P32;
+    /* the overflow offsets must fit as well: worst case 4/3 overflow entries per posting + padding */
+    if (ncols <= GKM_IDX_W20_MAX_COLS && M <= GKM_IDX_W20_MAX_WEIGHT && (4 * postings) / 3 + 64 < 4 * (size_t) GKM_IDX_W20_MAX_UNITS)
+        return GKM_IDX_FMT_W20;
+    return GKM_IDX_FMT_P32;
 }
 
 /* Device-time estimates, fitted to round-1 measurements on one B200 (DESIGN.md 4.4; 300 bp):

@@ -1,27 +1,37 @@
 /* tests/emu/index_emu.cc -- CPU emulator of the "index" kernel variant (gkm_index.h / gkm_index.cu).
  *
- * TEST INFRASTRUCTURE, not a fallback: nothing in the product links it.  It runs on the host, over
- * the product's own packed image (gkm_seq.c), the same steps the sm_100a code runs:
- *   keys   -> every valid window of both strands, coded by gkm_idx_code()         (gkm_idx_keys_kernel)
- *   sort   -> by (code, column)                                                    (cub radix sort)
- *   slots  -> {posting 0, 1, 2, posting 3 | pointer}, overflow lists padded to     (gkm_idx_runs_kernel,
- *             quads with end markers; long lists with a header unit and a flag      gkm_idx_fill_kernel)
- *   probes -> x ^ mask for every mask of gkm_idx_deltas(), postings walked with    (gkm_index_rows_kernel,
- *             the same sorted-list / end-marker rules                               idx_slot)
- * so that the code layout, the mask list, the slot encoding and the walk rules are checked against
- * the reference's histograms in the CPU-only tier.  The slot "table" is a hash map here: 4^L slots
- * do not fit a test box for L = 14.
+ * TEST INFRASTRUCTURE, not a fallback: nothing in the product links it.  It runs on the host, over the product's own
+ * packed image (gkm_seq.c), the steps of the sm_100a code.  The kernel's own code, shared verbatim:
+ *   the slot format of a block         gkm_idx_block_fmt()          (gkm_index_host.c, as ensure_index calls it)
+ *   overflow demand of a run           gkm_idx_ovf_need()           (gkm_index_slot.h, as gkm_idx_runs_kernel)
+ *   placement of a posting             gkm_idx_place()              (gkm_index_slot.h, as gkm_idx_fill_kernel)
+ *   decoding of a slot / overflow unit gkm_idx_slot(), gkm_idx_unit(), gkm_idx_unit_folded()
+ *                                                                   (gkm_index_slot.h, as gkm_index_rows_kernel)
+ *   the L-mer code and the mask list   gkm_idx_code(), gkm_idx_deltas()
+ * Emulation: the key generation (gkm_idx_keys_kernel), a stable sort by code in place of the CUB radix sort, the
+ * exclusive sum of the demands (the device's overflow layout), one serial loop over the postings in place of the
+ * fill kernel's threads, and serial probes in place of the row kernel's warps and queues, counting into the histogram
+ * instead of shared memory.  The slot table is a hash map (4^L slots do not fit a test box at L = 14); a slot that was
+ * never written reads as all ones, as the device's table after its memset.
  */
 #include <stdint.h>
-#include <stdlib.h>
+#include <string.h>
 #include <algorithm>
 #include <unordered_map>
 #include <vector>
 
 #include "../../gkmqc_b200/csrc/gkm_internal.h"
-#include "../../gkmqc_b200/csrc/gkm_index.h"
+#include "../../gkmqc_b200/csrc/gkm_index_slot.h"
+#include "../../gkmqc_b200/csrc/gkm_options.h"
 
-struct emu_slot { uint32_t v[4]; };
+struct emu_slot { uint32_t v[4] = { ~0u, ~0u, ~0u, ~0u }; };
+
+/* the fill kernel's stores, one thread after the other */
+struct emu_store {
+    static void st(uint32_t *p, uint32_t v) { *p = v; }
+    static void st(uint16_t *p, uint16_t v) { memcpy(p, &v, sizeof v); } /* halves of 32-bit words */
+    static void and_(uint32_t *p, uint32_t v) { *p &= v; }
+};
 
 static uint32_t window(const uint32_t *pl, int W, int lo, uint32_t mask)
 {
@@ -31,11 +41,30 @@ static uint32_t window(const uint32_t *pl, int W, int lo, uint32_t mask)
 }
 
 struct emu_index {
-    int fmt; /* GKM_IDX_FMT_P32: 16-byte slots of 32-bit postings; GKM_IDX_FMT_C16: 8-byte slots of 16-bit columns */
+    int fmt;
     std::unordered_map<uint32_t, emu_slot> tab;
-    std::vector<uint32_t> ovf;     /* P32 */
-    std::vector<uint16_t> ovf16;   /* C16 */
+    std::vector<uint32_t> ovf;
 };
+
+template <int FMT>
+static void fill(const std::vector<uint64_t> &keys, emu_index &ix)
+{
+    const size_t P = keys.size();
+    std::vector<uint32_t> runlen(P, 0), ofs(P);
+    for (size_t i = 0, e; i < P; i = e) {
+        for (e = i + 1; e < P && (keys[e] >> 32) == (keys[i] >> 32); e++) {}
+        runlen[i] = (uint32_t) (e - i);
+    }
+    uint32_t total = 0;
+    for (size_t i = 0; i < P; i++) { ofs[i] = total; total += gkm_idx_ovf_need(FMT, runlen[i]); }
+    /* the device does not clear the overflow array: an entry the placement misses reads as a posting of column 0 */
+    ix.ovf.assign(gkm_idx_unit_word(FMT, total), gkm_idx_posting(0, 1));
+    for (size_t i = 0, lb = 0; i < P; i++) {
+        if (runlen[i]) lb = i;
+        gkm_idx_place<FMT, emu_store>((uint32_t) (i - lb), runlen[lb], ofs[lb], (uint32_t) (keys[i] >> 8) & GKM_IDX_COL_MASK,
+                                      (uint32_t) keys[i] & 0xFFu, ix.tab[(uint32_t) (keys[i] >> 32)].v, ix.ovf.data());
+    }
+}
 
 /* index over the columns [cb, ce) */
 static void build_index(const gkmb200_problem *p, int cb, int ce, emu_index &ix)
@@ -54,113 +83,15 @@ static void build_index(const gkmb200_problem *p, int cb, int ce, emu_index &ix)
             keys.push_back(((uint64_t) code << 32) | ((uint64_t) (uint32_t) (g - cb) << 8) | wt);
         }
     }
-    std::sort(keys.begin(), keys.end(), [](uint64_t a, uint64_t b) { return (a >> 8) < (b >> 8); });
-    size_t i = 0;
-    ix.fmt = GKM_IDX_FMT_P32;
-    if (!getenv("GKM_EMU_INDEX_WIDE")) {
-        if (!p->weighted && ce - cb <= GKM_IDX_C16_MAX_COLS) ix.fmt = GKM_IDX_FMT_C16;
-        if (p->weighted && ce - cb <= GKM_IDX_W20_MAX_COLS && p->param.M <= GKM_IDX_W20_MAX_WEIGHT) ix.fmt = GKM_IDX_FMT_W20;
-    }
-    /* W20: x = p0 | p1 << 20, y = p1 >> 12 | p2 << 8 | flags; >= 4 postings: y = p1 >> 12 | long << 8 | units offset << 9 | PTR,
-     * overflow entries are P32 postings starting with posting 2 */
-    while (ix.fmt == GKM_IDX_FMT_W20 && i < keys.size()) {
-        size_t e = i;
-        while (e < keys.size() && (keys[e] >> 32) == (keys[i] >> 32)) e++;
-        const size_t len = e - i;
-        uint32_t p20[3] = { 0xFFFFFu, 0xFFFFFu, 0xFFFFFu };
-        for (size_t r = 0; r < len && r < 3; r++)
-            p20[r] = ((uint32_t) (keys[i + r] >> 8) & GKM_IDX_W20_COL_MASK) | (((uint32_t) keys[i + r] & 0xFFu) << GKM_IDX_W20_COL_BITS);
-        emu_slot s;
-        s.v[0] = p20[0] | (p20[1] << 20);
-        if (len <= 3) {
-            s.v[1] = (p20[1] >> 12) | (p20[2] << 8) | (0x7u << 28); /* flag bits other than PTR stay as the memset left them */
-        } else {
-            while (ix.ovf.size() & 3) ix.ovf.push_back(GKM_IDX_EMPTY);
-            const uint32_t units = GKM_IDX_W20_UNITS((uint32_t) len);
-            const uint32_t lng = units >= GKM_IDX_LONG_UNITS ? 1u : 0u;
-            s.v[1] = (p20[1] >> 12) | (lng << 8) | ((uint32_t) (ix.ovf.size() >> 2) << 9) | GKM_IDX_PTR;
-            if (lng) { ix.ovf.push_back(units); ix.ovf.push_back(0); ix.ovf.push_back(0); ix.ovf.push_back(0); }
-            for (size_t r = 2; r < len; r++)
-                ix.ovf.push_back(gkm_idx_posting((uint32_t) (keys[i + r] >> 8) & GKM_IDX_COL_MASK, (uint32_t) keys[i + r] & 0xFFu));
-            ix.ovf.push_back(GKM_IDX_EMPTY);
-            while (ix.ovf.size() & 3) ix.ovf.push_back(GKM_IDX_EMPTY);
-        }
-        s.v[2] = s.v[3] = 0;
-        ix.tab[(uint32_t) (keys[i] >> 32)] = s;
-        i = e;
-    }
-    while (ix.fmt == GKM_IDX_FMT_C16 && i < keys.size()) {
-        size_t e = i;
-        while (e < keys.size() && (keys[e] >> 32) == (keys[i] >> 32)) e++;
-        const size_t len = e - i;
-        uint16_t c[4] = { GKM_IDX_C16_NONE, GKM_IDX_C16_NONE, GKM_IDX_C16_NONE, GKM_IDX_C16_NONE };
-        emu_slot s;
-        if (len <= 4) {
-            for (size_t r = 0; r < len; r++) c[r] = (uint16_t) ((keys[i + r] >> 8) & 0x7FFFu);
-            s.v[0] = c[0] | ((uint32_t) c[1] << 16);
-            s.v[1] = c[2] | ((uint32_t) c[3] << 16);
-        } else {
-            for (size_t r = 0; r < 2; r++) c[r] = (uint16_t) ((keys[i + r] >> 8) & 0x7FFFu);
-            while (ix.ovf16.size() & 7) ix.ovf16.push_back(GKM_IDX_C16_NONE); /* lists start on 16 bytes */
-            s.v[0] = c[0] | ((uint32_t) c[1] << 16);
-            s.v[1] = GKM_IDX_PTR | (uint32_t) ix.ovf16.size();
-            const uint32_t units = GKM_IDX_C16_UNITS((uint32_t) len);
-            if (units >= GKM_IDX_LONG_UNITS) { /* long list: header unit {units, 0, 0, 0}, flag in the pointer */
-                s.v[1] |= GKM_IDX_LONG;
-                ix.ovf16.push_back((uint16_t) (units & 0xFFFFu)); ix.ovf16.push_back((uint16_t) (units >> 16));
-                for (int t = 0; t < 6; t++) ix.ovf16.push_back(0);
-            }
-            for (size_t r = 2; r < len; r++) ix.ovf16.push_back((uint16_t) ((keys[i + r] >> 8) & 0x7FFFu));
-            ix.ovf16.push_back(GKM_IDX_C16_NONE);
-            while (ix.ovf16.size() & 7) ix.ovf16.push_back(GKM_IDX_C16_NONE);
-        }
-        s.v[2] = s.v[3] = 0;
-        ix.tab[(uint32_t) (keys[i] >> 32)] = s;
-        i = e;
-    }
-    while (i < keys.size()) {
-        size_t e = i;
-        while (e < keys.size() && (keys[e] >> 32) == (keys[i] >> 32)) e++;
-        const size_t len = e - i;
-        emu_slot s;
-        for (int t = 0; t < 4; t++) s.v[t] = GKM_IDX_EMPTY;
-        for (size_t r = 0; r < len; r++) {
-            const uint32_t posting = gkm_idx_posting((uint32_t) (keys[i + r] >> 8) & GKM_IDX_COL_MASK, (uint32_t) keys[i + r] & 0xFFu);
-            if (r < 3 || (r == 3 && len == 4)) s.v[r] = posting;
-            else {
-                if (r == 3) {
-                    while (ix.ovf.size() & 3) ix.ovf.push_back(GKM_IDX_EMPTY); /* lists start on 16 bytes */
-                    s.v[3] = GKM_IDX_PTR | (uint32_t) ix.ovf.size();
-                    const uint32_t units = GKM_IDX_P32_UNITS((uint32_t) len);
-                    if (units >= GKM_IDX_LONG_UNITS) {
-                        s.v[3] |= GKM_IDX_LONG;
-                        ix.ovf.push_back(units); ix.ovf.push_back(0); ix.ovf.push_back(0); ix.ovf.push_back(0);
-                    }
-                }
-                ix.ovf.push_back(posting);
-            }
-        }
-        if (len >= 5) { /* at least one end marker, up to a multiple of four */
-            ix.ovf.push_back(GKM_IDX_EMPTY);
-            while (ix.ovf.size() & 3) ix.ovf.push_back(GKM_IDX_EMPTY);
-        }
-        ix.tab[(uint32_t) (keys[i] >> 32)] = s;
-        i = e;
-    }
-}
-
-static inline void hit16(int32_t *H, int nb, int m, uint32_t b, uint32_t blo, uint32_t bhi)
-{
-    if (b < bhi && b >= blo) H[(size_t) (b - blo) * nb + m] += 1;
-}
-
-static inline void hit(int32_t *H, int nb, int m, uint32_t e, uint32_t blo, uint32_t bhi, int w)
-{
-    const uint32_t b = e & GKM_IDX_COL_MASK;
-    if (b < bhi && b >= blo) H[(size_t) (b - blo) * nb + m] += w * (int) (e >> GKM_IDX_COL_BITS);
+    std::stable_sort(keys.begin(), keys.end(), [](uint64_t a, uint64_t b) { return (a >> 32) < (b >> 32); });
+    ix.fmt = gkm_idx_block_fmt(p->weighted, p->param.M, ce - cb, keys.size(), gkm_opt_index_wide());
+    if (ix.fmt == GKM_IDX_FMT_C16) fill<GKM_IDX_FMT_C16>(keys, ix);
+    else if (ix.fmt == GKM_IDX_FMT_W20) fill<GKM_IDX_FMT_W20>(keys, ix);
+    else fill<GKM_IDX_FMT_P32>(keys, ix);
 }
 
 /* H[(b - blo) * nbins + m] += ... for row a against the indexed columns [blo, bhi) (relative) */
+template <int FMT, bool WEIGHTED>
 static void probe_row(const gkmb200_problem *p, const emu_index &ix, const std::vector<uint32_t> &deltas, int a,
                       uint32_t blo, uint32_t bhi, int32_t *H)
 {
@@ -168,91 +99,35 @@ static void probe_row(const gkmb200_problem *p, const emu_index &ix, const std::
     const uint32_t mask = (1u << L) - 1u;
     const uint32_t *pl = p->planes + (size_t) a * 3 * W;
     const int nq = p->len[a] - L + 1;
+    const emu_slot empty;
     for (int i = 0; i < nq; i++) {
         const uint32_t x = gkm_idx_code(window(pl, W, i, mask), window(pl + W, W, i, mask), L);
-        const int w = p->weighted ? p->wend[(size_t) a * 32 * W + i + L - 1] : 1;
+        const int w = WEIGHTED ? p->wend[(size_t) a * 32 * W + i + L - 1] : 1;
         for (uint32_t dl : deltas) {
             const int m = (int) (dl >> 28);
-            auto it = ix.tab.find(x ^ (dl & 0x0FFFFFFFu));
-            if (it == ix.tab.end()) continue;
-            const uint32_t *sl = it->second.v;
-            if (ix.fmt == GKM_IDX_FMT_C16) {
-                const uint32_t c1 = sl[0] >> 16, c3 = sl[1] >> 16;
-                hit16(H, nb, m, sl[0] & 0xFFFFu, blo, bhi);
-                hit16(H, nb, m, c1, blo, bhi);
-                if (!(sl[1] & GKM_IDX_PTR) || c3 == GKM_IDX_C16_NONE) {
-                    hit16(H, nb, m, sl[1] & 0xFFFFu, blo, bhi);
-                    hit16(H, nb, m, c3, blo, bhi);
-                } else if (c1 < bhi && (sl[1] & GKM_IDX_LONG)) {
-                    /* long list (idx_walk_long): `units` units behind the header; a unit whose first column is
-                     * behind the range ends the walk of the lane that owns it -- every later unit is behind it too */
-                    const uint16_t *q = ix.ovf16.data() + (sl[1] & ~(GKM_IDX_PTR | GKM_IDX_LONG));
-                    const uint32_t units = q[0] | ((uint32_t) q[1] << 16);
-                    for (uint32_t u = 0; u < units; u++) {
-                        const uint16_t *v = q + 8 + 8 * (size_t) u;
-                        if (v[0] >= bhi) continue;
-                        for (int t = 0; t < 8; t++) hit16(H, nb, m, v[t], blo, bhi);
-                    }
-                } else if (c1 < bhi) {
-                    const uint16_t *q = ix.ovf16.data() + (sl[1] & ~GKM_IDX_PTR);
-                    for (;;) {
-                        for (int t = 0; t < 8; t++) hit16(H, nb, m, q[t], blo, bhi);
-                        if (q[7] >= bhi) break;
-                        q += 8;
-                    }
-                }
-                continue;
-            }
-            if (ix.fmt == GKM_IDX_FMT_W20) {
-                const uint32_t p0 = sl[0] & 0xFFFFFu, p1 = (sl[0] >> 20) | ((sl[1] & 0xFFu) << 12);
-                const uint32_t c0 = p0 & GKM_IDX_W20_COL_MASK, c1 = p1 & GKM_IDX_W20_COL_MASK;
-                if (c0 < bhi && c0 >= blo) H[(size_t) (c0 - blo) * nb + m] += w * (int) (p0 >> GKM_IDX_W20_COL_BITS);
-                if (c1 < bhi && c1 >= blo) H[(size_t) (c1 - blo) * nb + m] += w * (int) (p1 >> GKM_IDX_W20_COL_BITS);
-                if (!(sl[1] & GKM_IDX_PTR) || c0 == GKM_IDX_W20_COL_MASK) {
-                    const uint32_t p2 = (sl[1] >> 8) & 0xFFFFFu, c2 = p2 & GKM_IDX_W20_COL_MASK;
-                    if (c2 < bhi && c2 >= blo) H[(size_t) (c2 - blo) * nb + m] += w * (int) (p2 >> GKM_IDX_W20_COL_BITS);
-                } else if (c1 < bhi) {
-                    const uint32_t *q = ix.ovf.data() + (((sl[1] >> 9) & 0x3FFFFFu) << 2);
-                    if ((sl[1] >> 8) & GKM_IDX_LONG) {
-                        const uint32_t units = q[0];
-                        for (uint32_t u = 0; u < units; u++) {
-                            const uint32_t *v = q + 4 + 4 * (size_t) u;
-                            if ((v[0] & GKM_IDX_COL_MASK) >= bhi) continue;
-                            for (int t = 0; t < 4; t++) hit(H, nb, m, v[t], blo, bhi, w);
-                        }
-                    } else {
-                        for (;;) {
-                            for (int t = 0; t < 4; t++) hit(H, nb, m, q[t], blo, bhi, w);
-                            if ((q[3] & GKM_IDX_COL_MASK) >= bhi) break;
-                            q += 4;
-                        }
-                    }
-                }
-                continue;
-            }
-            hit(H, nb, m, sl[0], blo, bhi, w);
-            hit(H, nb, m, sl[1], blo, bhi, w);
-            hit(H, nb, m, sl[2], blo, bhi, w);
-            if (!(sl[3] & GKM_IDX_PTR)) hit(H, nb, m, sl[3], blo, bhi, w);
-            else if (sl[3] != GKM_IDX_EMPTY && (sl[2] & GKM_IDX_COL_MASK) < bhi && (sl[3] & GKM_IDX_LONG)) {
-                const uint32_t *q = ix.ovf.data() + (sl[3] & ~(GKM_IDX_PTR | GKM_IDX_LONG));
-                const uint32_t units = q[0];
-                for (uint32_t u = 0; u < units; u++) {
-                    const uint32_t *v = q + 4 + 4 * (size_t) u;
-                    if ((v[0] & GKM_IDX_COL_MASK) >= bhi) continue;
-                    for (int t = 0; t < 4; t++) hit(H, nb, m, v[t], blo, bhi, w);
-                }
-            }
-            else if (sl[3] != GKM_IDX_EMPTY && (sl[2] & GKM_IDX_COL_MASK) < bhi) {
-                const uint32_t *q = ix.ovf.data() + (sl[3] & ~GKM_IDX_PTR);
-                for (;;) {
-                    for (int t = 0; t < 4; t++) hit(H, nb, m, q[t], blo, bhi, w);
-                    if ((q[3] & GKM_IDX_COL_MASK) >= bhi) break;
-                    q += 4;
-                }
+            const auto hit = [&](uint32_t b, int v) { H[(size_t) b * nb + m] += v; };
+            const auto it = ix.tab.find(x ^ (dl & 0x0FFFFFFFu));
+            const uint32_t *s = it == ix.tab.end() ? empty.v : it->second.v;
+            const uint32_t o = gkm_idx_slot<FMT, WEIGHTED, true>(s[0], s[1], s[2], s[3], blo, bhi, w, hit);
+            if (o == ~0u) continue;
+            const uint32_t *q = ix.ovf.data() + gkm_idx_unit_word(FMT, o & ~GKM_IDX_LONG);
+            if (o & GKM_IDX_LONG) { /* idx_walk_long: the units behind the header, one per lane */
+                for (uint32_t u = 1; u <= q[0]; u++)
+                    if (!gkm_idx_unit_folded<FMT, WEIGHTED, true>(q[4 * u], q[4 * u + 1], q[4 * u + 2], q[4 * u + 3], blo, bhi, w, hit)) break;
+            } else {
+                while (gkm_idx_unit<FMT, WEIGHTED, true>(q[0], q[1], q[2], q[3], blo, bhi, w, hit)) q += 4;
             }
         }
     }
+}
+
+static void probe(const gkmb200_problem *p, const emu_index &ix, const std::vector<uint32_t> &deltas, int a,
+                  uint32_t blo, uint32_t bhi, int32_t *H)
+{
+    if (ix.fmt == GKM_IDX_FMT_C16) probe_row<GKM_IDX_FMT_C16, false>(p, ix, deltas, a, blo, bhi, H);
+    else if (ix.fmt == GKM_IDX_FMT_W20) probe_row<GKM_IDX_FMT_W20, true>(p, ix, deltas, a, blo, bhi, H);
+    else if (p->weighted) probe_row<GKM_IDX_FMT_P32, true>(p, ix, deltas, a, blo, bhi, H);
+    else probe_row<GKM_IDX_FMT_P32, false>(p, ix, deltas, a, blo, bhi, H);
 }
 
 extern "C" {
@@ -282,7 +157,7 @@ int gkm_emu_index_hist_lower(gkmb200_problem *p, int block_cols, int32_t *H)
         build_index(p, cb, ce, ix);
         for (int a = cb; a < n; a++) {
             const uint32_t bhi = (uint32_t) ((a + 1 < ce ? a + 1 : ce) - cb); /* columns <= a */
-            probe_row(p, ix, deltas, a, 0u, bhi, H + ((size_t) a * n + cb) * nb);
+            probe(p, ix, deltas, a, 0u, bhi, H + ((size_t) a * n + cb) * nb);
         }
     }
     return 0;
@@ -300,7 +175,7 @@ int gkm_emu_index_hist_rect(gkmb200_problem *p, int row0, int nrows, int col0, i
     emu_index ix;
     build_index(p, 0, p->n, ix); /* the whole problem is one block; only [col0, col0 + ncols) is wanted */
     for (int r = 0; r < nrows; r++)
-        probe_row(p, ix, deltas, row0 + r, (uint32_t) col0, (uint32_t) (col0 + ncols), H + (size_t) r * ncols * nb);
+        probe(p, ix, deltas, row0 + r, (uint32_t) col0, (uint32_t) (col0 + ncols), H + (size_t) r * ncols * nb);
     return 0;
 }
 

@@ -95,6 +95,23 @@ def test_supported_and_cost_model(lib):
     assert lib.gkm_idx_cost_ms(14, 4, 0, 20000, 287.0, 2, n20, 2.0 * 287 * 287) > lib.gkm_diag_cost_ms(4, 0, n20, 2.0 * 287 * 287)
 
 
+def test_block_format_choice(lib):
+    P32, C16, W20 = 0, 1, 2
+    lib.gkm_idx_block_fmt.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_size_t, ctypes.c_int]
+    fmt = lib.gkm_idx_block_fmt
+    # unit weights: 16-bit columns below 0x8000
+    assert fmt(0, 50, 0x7FFF, 10 ** 6, 0) == C16 and fmt(0, 50, 0x8000, 10 ** 6, 0) == P32
+    # weights: <= 63, <= 16 352 columns, overflow offsets below 2^22 units (worst case 4/3 entries per posting + 64)
+    assert fmt(1, 63, 16352, 10 ** 6, 0) == W20
+    assert fmt(1, 64, 16352, 10 ** 6, 0) == P32
+    assert fmt(1, 50, 16353, 10 ** 6, 0) == P32
+    p_max = (3 * (4 << 22) - 3 * 64 - 1) // 4  # the most postings with (4 P) / 3 + 64 < 4 * 2^22
+    assert (4 * p_max) // 3 + 64 < 4 << 22 <= (4 * (p_max + 1)) // 3 + 64
+    assert fmt(1, 50, 16352, p_max, 0) == W20 and fmt(1, 50, 16352, p_max + 1, 0) == P32
+    # index_wide: the 16-byte slots whatever fits
+    assert fmt(0, 50, 100, 1000, 1) == P32 and fmt(1, 50, 100, 1000, 1) == P32
+
+
 @pytest.fixture(scope="module")
 def emu(emu_lib):
     emu_lib.gkm_emu_index_cost.restype = ctypes.c_longlong
@@ -127,13 +144,19 @@ def test_emulated_index_matches_reference_histograms(name, emu):
     P.close()
 
 
-@pytest.mark.parametrize("wide", [False, True])
+@pytest.fixture
+def wide(request, emu):
+    """the emulator library's own index_wide option: 16-byte slots (1) instead of the compact ones (C16 / W20)"""
+    assert emu.gkmb200_set_option(b"index_wide", b"1" if request.param else b"0") == 0
+    yield request.param
+    emu.gkmb200_set_option(b"index_wide", b"0")
+
+
+@pytest.mark.parametrize("wide", [False, True], indirect=True)
 @pytest.mark.parametrize("kernel_type,L,d", [(2, 8, 2), (4, 9, 3), (2, 6, 4), (4, 5, 1)])
-def test_emulated_index_long_lists_and_ranges(kernel_type, L, d, wide, emu, monkeypatch):
+def test_emulated_index_long_lists_and_ranges(kernel_type, L, d, wide, emu):
     """few distinct L-mers (short L, repeats): posting lists far beyond the four inline slots, so the overflow
     walk, its end markers and the column-range cut are exercised; plus a rectangular block with col0 > 0"""
-    if wide:
-        monkeypatch.setenv("GKM_EMU_INDEX_WIDE", "1")  # 16-byte slots instead of the compact ones (C16 / W20)
     seqs = random_seqs(40, 90, seed=17 * L + d, ragged=True)
     seqs = [s if len(s) >= L else s + "ACGT" * 4 for s in seqs]
     seqs[7] = seqs[6]
