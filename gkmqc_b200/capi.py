@@ -58,6 +58,19 @@ class gkmb200_svm_fit(ctypes.Structure):
                 ("n_iter", ctypes.c_int), ("n_sv", ctypes.c_int), ("reserved", ctypes.c_longlong)]
 
 
+class gkmb200_svm_options(ctypes.Structure):
+    _fields_ = [("C", ctypes.c_double), ("eps", ctypes.c_double), ("max_iter", ctypes.c_int), ("shrinking", ctypes.c_int),
+                ("reserved", ctypes.c_longlong)]
+
+
+class gkmb200_svm_shrink_stats(ctypes.Structure):
+    _fields_ = [("shrink_passes", ctypes.c_int), ("min_active", ctypes.c_int), ("unshrink_iter", ctypes.c_int),
+                ("recon_a", ctypes.c_int), ("recon_b", ctypes.c_int), ("reserved", ctypes.c_int)]
+
+    def as_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_ if k != "reserved"}
+
+
 class GkmError(RuntimeError):
     pass
 
@@ -127,6 +140,9 @@ def _declare(lib):
         ("gkmb200_svm_cv", [P, ctypes.c_void_p, ctypes.c_long, I, I, ctypes.POINTER(gkmb200_svm_task), c_int_p,
                             ctypes.POINTER(ctypes.c_byte), c_int_p, ctypes.c_double, ctypes.c_double, I,
                             c_dbl_p, ctypes.POINTER(gkmb200_svm_fit), c_dbl_p]),
+        ("gkmb200_svm_cv_ex", [P, ctypes.c_void_p, ctypes.c_long, I, I, ctypes.POINTER(gkmb200_svm_task), c_int_p,
+                               ctypes.POINTER(ctypes.c_byte), c_int_p, ctypes.POINTER(gkmb200_svm_options),
+                               c_dbl_p, ctypes.POINTER(gkmb200_svm_fit), c_dbl_p, ctypes.POINTER(gkmb200_svm_shrink_stats)]),
         ("gkmb200_device_count", []),
         ("gkmb200_set_devices", [c_int_p, I]),
         ("gkmb200_set_option", [ctypes.c_char_p, ctypes.c_char_p]),
@@ -378,10 +394,12 @@ def svm_prepare_tasks(y, splits):
     return tasks, cat(tr, np.int32), cat(ty, np.int8), cat(te, np.int32)
 
 
-def svm_cv(y, splits, kmat=None, problem=None, C=1.0, eps=1e-3, max_iter=-1, lib=None):
+def svm_cv(y, splits, kmat=None, problem=None, C=1.0, eps=1e-3, max_iter=-1, shrinking=0, stats=False, lib=None):
     """cross-validated C-SVC on the GPU (SURVEY.md 8f/f4).  Either `kmat` (dense symmetric host matrix) or `problem`
     (a capi.Problem whose kernel matrix is computed and kept on the device).  Returns (scores per split, fits, alphas):
-    scores are sklearn decision_function values of the test ids, alphas are in the grouped training order."""
+    scores are sklearn decision_function values of the test ids, alphas are in the grouped training order.
+    shrinking = 1: libsvm's shrinking heuristic, SVC(shrinking=True).  stats=True appends a fourth element, per fit what
+    the heuristic did (gkmb200_svm_shrink_stats as a dict)."""
     lib = lib or (problem.lib if problem is not None else load())
     tasks, tr, ty, te = svm_prepare_tasks(y, splits)
     scores = np.zeros(len(te))
@@ -395,14 +413,24 @@ def svm_cv(y, splits, kmat=None, problem=None, C=1.0, eps=1e-3, max_iter=-1, lib
         n, kptr, ld, h = kmat.shape[0], kmat.ctypes.data, kmat.strides[0] // 8, None
     else:
         n, kptr, ld, h = problem.n, None, 0, problem.h
-    _check(lib.gkmb200_svm_cv(h, kptr, ld, n, len(splits), tasks, tr.ctypes.data_as(c_int_p),
-                              ty.ctypes.data_as(ctypes.POINTER(ctypes.c_byte)), te.ctypes.data_as(c_int_p),
-                              C, eps, max_iter, scores.ctypes.data_as(c_dbl_p), fits, alpha.ctypes.data_as(c_dbl_p)), lib)
+    args = (h, kptr, ld, n, len(splits), tasks, tr.ctypes.data_as(c_int_p), ty.ctypes.data_as(ctypes.POINTER(ctypes.c_byte)),
+            te.ctypes.data_as(c_int_p))
+    outs = (scores.ctypes.data_as(c_dbl_p), fits, alpha.ctypes.data_as(c_dbl_p))
+    st = None
+    if shrinking == 0 and not stats:
+        _check(lib.gkmb200_svm_cv(*args, C, eps, max_iter, *outs), lib)
+    else:
+        opt = gkmb200_svm_options(C, eps, max_iter, shrinking, 0)
+        st = (gkmb200_svm_shrink_stats * len(splits))()
+        _check(lib.gkmb200_svm_cv_ex(*args, ctypes.byref(opt), *outs, st), lib)
     out_s, out_a = [], []
     for t in range(len(splits)):
         out_s.append(scores[tasks[t].test_off: tasks[t].test_off + tasks[t].ntest])
         out_a.append(alpha[tasks[t].train_off: tasks[t].train_off + tasks[t].ntrain])
-    return out_s, [dict(rho=f.rho, obj=f.obj, nu=f.nu, n_iter=f.n_iter, n_sv=f.n_sv) for f in fits], out_a
+    out_f = [dict(rho=f.rho, obj=f.obj, nu=f.nu, n_iter=f.n_iter, n_sv=f.n_sv) for f in fits]
+    if stats:
+        return out_s, out_f, out_a, [x.as_dict() for x in st]
+    return out_s, out_f, out_a
 
 
 def main_pywrapper(posfile, negfile, kernel_type=2, L=11, k=7, d=3, M=50, H=50.0, gamma=1.0,

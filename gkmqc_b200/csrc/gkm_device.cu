@@ -1528,12 +1528,13 @@ extern "C" int gkmb200_resident_rows(gkmb200_problem *p, int row0, int nrows, do
     return rc;
 }
 
-extern "C" int gkm_dev_svm_cv(gkmb200_problem *p, const double *kmat, long ld, int n, int ntasks, const gkmb200_svm_task *tasks,
-                              const int *train_idx, const signed char *train_y, const int *test_idx,
-                              double C, double eps, int max_iter, double *scores, gkmb200_svm_fit *fits, double *alpha)
+static int svm_cv(gkmb200_problem *p, const double *kmat, long ld, int n, int ntasks, const gkmb200_svm_task *tasks,
+                  const int *train_idx, const signed char *train_y, const int *test_idx, double C, double eps, int max_iter,
+                  int shrinking, double *scores, gkmb200_svm_fit *fits, double *alpha, gkmb200_svm_shrink_stats *stats)
 {
     if (ntasks < 0 || (ntasks > 0 && (!tasks || !train_idx || !train_y || !test_idx))) { gkm_set_error("null argument"); return 1; }
     if (!(C > 0.0) || !(eps > 0.0)) { gkm_set_error("svm: C and eps must be positive"); return 1; }
+    if (shrinking != 0 && shrinking != 1) { gkm_set_error("svm: shrinking must be 0 or 1, not %d", shrinking); return 1; }
     pthread_mutex_lock(&g_lock);
     int rc = 0;
     const double t0 = now_ms();
@@ -1547,7 +1548,7 @@ extern "C" int gkm_dev_svm_cv(gkmb200_problem *p, const double *kmat, long ld, i
             gkm_devstate *ds = p->dev;
             gkm_gpu *g = &g_gpu[ds->dev[0]];
             rc = gkm_svm_run(ds->img[0].full, (long long) ds->img[0].full_ld, n, ntasks, tasks, train_idx, train_y, test_idx,
-                             C, eps, max_iter, scores, fits, alpha, g->sc);
+                             C, eps, max_iter, shrinking, scores, fits, alpha, stats, g->sc);
             p->stats.launches += 3;
             p->stats.wall_ms = now_ms() - t0;
         }
@@ -1561,12 +1562,29 @@ extern "C" int gkm_dev_svm_cv(gkmb200_problem *p, const double *kmat, long ld, i
             if (!rc && dev_malloc(g, (void **) &d_K, sizeof(double) * (size_t) n * (size_t) n) != cudaSuccess) { gkm_set_error("CUDA: svm matrix: %s", cudaGetErrorString(cudaGetLastError())); rc = 1; }
             if (!rc && cudaMemcpy2DAsync(d_K, sizeof(double) * (size_t) n, kmat, sizeof(double) * (size_t) ld, sizeof(double) * (size_t) n, (size_t) n,
                                          cudaMemcpyHostToDevice, g->sc) != cudaSuccess) { gkm_set_error("CUDA: svm matrix upload: %s", cudaGetErrorString(cudaGetLastError())); rc = 1; }
-            if (!rc) rc = gkm_svm_run(d_K, (long long) n, n, ntasks, tasks, train_idx, train_y, test_idx, C, eps, max_iter, scores, fits, alpha, g->sc);
+            if (!rc) rc = gkm_svm_run(d_K, (long long) n, n, ntasks, tasks, train_idx, train_y, test_idx, C, eps, max_iter, shrinking,
+                                      scores, fits, alpha, stats, g->sc);
             cudaFree(d_K);
         }
     }
     pthread_mutex_unlock(&g_lock);
     return rc;
+}
+
+extern "C" int gkm_dev_svm_cv(gkmb200_problem *p, const double *kmat, long ld, int n, int ntasks, const gkmb200_svm_task *tasks,
+                              const int *train_idx, const signed char *train_y, const int *test_idx,
+                              double C, double eps, int max_iter, double *scores, gkmb200_svm_fit *fits, double *alpha)
+{
+    return svm_cv(p, kmat, ld, n, ntasks, tasks, train_idx, train_y, test_idx, C, eps, max_iter, 0, scores, fits, alpha, NULL);
+}
+
+extern "C" int gkmb200_svm_cv_ex(gkmb200_problem *p, const double *kmat, long ld, int n, int ntasks, const gkmb200_svm_task *tasks,
+                                 const int *train_idx, const signed char *train_y, const int *test_idx, const gkmb200_svm_options *opt,
+                                 double *scores, gkmb200_svm_fit *fits, double *alpha, gkmb200_svm_shrink_stats *stats)
+{
+    if (!opt) { gkm_set_error("null argument"); return 1; }
+    return svm_cv(p, kmat, ld, n, ntasks, tasks, train_idx, train_y, test_idx, opt->C, opt->eps, opt->max_iter, opt->shrinking,
+                  scores, fits, alpha, stats);
 }
 
 /* ------------------------------------------------------------------ */

@@ -35,12 +35,12 @@ def computeGkmKernel(args_gkm, max_seqs=MAX_SEQS):
 def crossValidate(args_svm, _kmat, n_pseqs, n_nseqs, problem=None):
     """args_svm = [regularization, precision, shrinking, cache_size, ncv, repeats, fast_estimation, random_seeds, p]
     (gkmsvm.py:198-208).  Same splits as the reference (StratifiedKFold per repeat, gkmsvm.py:146-150), same
-    (mean AUC, std AUC) result; the 5 x 10 C-SVC fits run concurrently on the GPU through gkmb200_svm_cv.
+    (mean AUC, std AUC) result; the 5 x 10 C-SVC fits run concurrently on the GPU through gkmb200_svm_cv_ex.
     _kmat = the symmetric host matrix, or None with `problem` given: the matrix then never leaves the device.
-    shrinking is accepted and ignored: the heuristic changes libsvm's path, not its optimum."""
+    shrinking != 0 runs libsvm's shrinking heuristic, as the reference's SVC(shrinking=...) does."""
     from sklearn.metrics import roc_auc_score
     from sklearn.model_selection import StratifiedKFold
-    regularization, precision, _shrinking, _cache_size, ncv, repeats, fast_estimation, random_seeds, _p = args_svm
+    regularization, precision, shrinking, _cache_size, ncv, repeats, fast_estimation, random_seeds, _p = args_svm
     if random_seeds < 0:
         random_seeds = None
     seqids = ["p%4d" % x for x in range(n_pseqs)] + ["n%4d" % x for x in range(n_nseqs)]
@@ -51,7 +51,8 @@ def crossValidate(args_svm, _kmat, n_pseqs, n_nseqs, problem=None):
     for _ in range(repeats):
         kf = StratifiedKFold(n_splits=ncv, shuffle=True, random_state=random_seeds)
         splits.extend(kf.split(seqids, y))
-    scores, fits, _ = capi.svm_cv(y, splits, kmat=_kmat, problem=problem, C=regularization, eps=precision)
+    scores, fits, _ = capi.svm_cv(y, splits, kmat=_kmat, problem=problem, C=regularization, eps=precision,
+                                  shrinking=int(bool(shrinking)))
     aucs = []
     for (_, test), s, f in zip(splits, scores, fits):
         aucs.append(roc_auc_score(y[test], s))
@@ -112,7 +113,7 @@ def main(argv=None):
     s = ap.add_argument_group("SVM training")
     s.add_argument("-C", "--regularization", type=float, default=1.0, help="regularization parameter C (default: 1.0)")
     s.add_argument("-e", "--precision", type=float, default=0.001, help="precision parameter epsilon (default: 0.001)")
-    s.add_argument("-u", "--shrinking", type=int, default=0, help="accepted for compatibility; the GPU solver does not shrink (default: 0)")
+    s.add_argument("-u", "--shrinking", type=int, default=0, help="use the shrinking heuristic of libsvm, 0 or 1 (default: 0)")
     s.add_argument("-c", "--cache-size", type=int, default=512, help="accepted for compatibility (the matrix is resident)")
     s.add_argument("-x", "--ncv", type=int, default=5, help="x-fold cross validation (default: 5)")
     s.add_argument("-r", "--repeats", type=int, default=1, help="number of repeats of CV training (default: 1)")

@@ -114,10 +114,36 @@ typedef struct gkmb200_svm_fit {
  * scores[test_off + r] = sklearn's decision_function value (positive = label 1).
  * kmat != NULL: dense symmetric n x n host matrix with ld doubles per row (what computeGkmKernel returns).
  * kmat == NULL: the kernel matrix of problem p is computed on the device and never leaves it (n = problem size).
- * fits[ntasks] and alpha[sum of ntrain] (in training order) may be NULL. */
+ * fits[ntasks] and alpha[sum of ntrain] (in training order) may be NULL.
+ * = gkmb200_svm_cv_ex with shrinking = 0. */
 int gkmb200_svm_cv(gkmb200_problem *p, const double *kmat, long ld, int n, int ntasks, const gkmb200_svm_task *tasks,
                    const int *train_idx, const signed char *train_y, const int *test_idx,
                    double C, double eps, int max_iter, double *scores, gkmb200_svm_fit *fits, double *alpha);
+
+typedef struct gkmb200_svm_options {
+    double C;          /* SVC's C */
+    double eps;        /* SVC's tol */
+    int max_iter;      /* SVC's max_iter; < 0: libsvm's own ceiling */
+    int shrinking;     /* SVC's shrinking: 0 or 1 (anything else is rejected) */
+    long long reserved;
+} gkmb200_svm_options;
+
+/* what the shrinking heuristic did in one fit (shrinking = 0: {0, ntrain, -1, 0, 0}) */
+typedef struct gkmb200_svm_shrink_stats {
+    int shrink_passes;   /* calls of libsvm's do_shrinking */
+    int min_active;      /* smallest active set those passes left */
+    int unshrink_iter;   /* iterations done when the whole gradient was rebuilt near the optimum (Gmax1 + Gmax2 <= 10 eps), or -1 */
+    int recon_a;         /* gradient reconstructions looping over the inactive points outside, the free active ones inside */
+    int recon_b;         /* gradient reconstructions looping over the free active points outside */
+    int reserved;
+} gkmb200_svm_shrink_stats;
+
+/* gkmb200_svm_cv with the options of SVC: shrinking = 1 follows sklearn's SVC(shrinking=True) iterate for iterate
+ * (libsvm's do_shrinking every min(ntrain, 1000) iterations, its unshrink and gradient reconstructions, the same
+ * iteration count, support vectors, dual_coef_ and intercept_).  stats[ntasks] may be NULL. */
+int gkmb200_svm_cv_ex(gkmb200_problem *p, const double *kmat, long ld, int n, int ntasks, const gkmb200_svm_task *tasks,
+                      const int *train_idx, const signed char *train_y, const int *test_idx, const gkmb200_svm_options *opt,
+                      double *scores, gkmb200_svm_fit *fits, double *alpha, gkmb200_svm_shrink_stats *stats);
 
 /* rows [row0, row0 + nrows) of the resident symmetric matrix of p (all n columns, unit diagonal; ld >= n doubles per row),
  * computed on first use and kept on the device for gkmb200_svm_cv; nrows = 0 only makes it resident.  With several
