@@ -143,6 +143,9 @@ def _declare(lib):
         ("gkmb200_svm_cv_ex", [P, ctypes.c_void_p, ctypes.c_long, I, I, ctypes.POINTER(gkmb200_svm_task), c_int_p,
                                ctypes.POINTER(ctypes.c_byte), c_int_p, ctypes.POINTER(gkmb200_svm_options),
                                c_dbl_p, ctypes.POINTER(gkmb200_svm_fit), c_dbl_p, ctypes.POINTER(gkmb200_svm_shrink_stats)]),
+        ("gkmb200_lmer_table_get", [P, c_dbl_p]),
+        ("gkmb200_lmer_table_scores", [P, P, I, I, ctypes.c_double, c_dbl_p]),
+        ("gkmb200_lmer_table_build_ms", [P, c_dbl_p]),
         ("gkmb200_device_count", []),
         ("gkmb200_set_devices", [c_int_p, I]),
         ("gkmb200_set_option", [ctypes.c_char_p, ctypes.c_char_p]),
@@ -153,6 +156,11 @@ def _declare(lib):
         if hasattr(lib, name):
             getattr(lib, name).argtypes = args
             getattr(lib, name).restype = ctypes.c_int
+    if hasattr(lib, "gkmb200_lmer_table_new"):
+        lib.gkmb200_lmer_table_new.argtypes = [P, I, I, c_dbl_p]
+        lib.gkmb200_lmer_table_new.restype = P
+        lib.gkmb200_lmer_table_free.argtypes = [P]
+        lib.gkmb200_lmer_table_free.restype = None
 
 
 def last_error(lib=None):
@@ -326,6 +334,11 @@ class Problem:
                                                 out.ctypes.data_as(c_dbl_p)), self.lib)
         return out
 
+    def lmer_table(self, col0, ncols, alpha):
+        """the model sum_c alpha[c - col0] K(., c), c in [col0, col0 + ncols), folded into one weight per L-mer
+        (kernel types 0, 1, 2, 4): an LmerTable, built on every GPU of this problem"""
+        return LmerTable(self, col0, ncols, alpha)
+
     def stats(self):
         st = gkmb200_stats()
         _check(self.lib.gkmb200_get_stats(self.h, ctypes.byref(st)), self.lib)
@@ -366,6 +379,52 @@ class Problem:
         ms = np.zeros(steps)
         _check(self.lib.gkmb200_bench_lower_resident(self.h, steps, warmup, int(flush_l2), ms.ctypes.data_as(c_dbl_p)), self.lib)
         return ms
+
+
+class LmerTable:
+    """a linear gkm-SVM model as 4^L L-mer weights T (gkmb200_lmer_table_new): score(r) = bias + sum over the forward
+    L-mers x of r of wt_r(x) T[x] / |r|, at a cost independent of the number of support vectors"""
+
+    def __init__(self, problem, col0, ncols, alpha):
+        self.lib, self.L = problem.lib, problem.L
+        alpha = np.ascontiguousarray(alpha, np.float64)
+        if alpha.shape != (ncols,):
+            raise ValueError("alpha must hold ncols = %d values" % ncols)
+        self.h = self.lib.gkmb200_lmer_table_new(problem.h, col0, ncols, alpha.ctypes.data_as(c_dbl_p))
+        if not self.h:
+            raise GkmError(last_error(self.lib))
+
+    def close(self):
+        if getattr(self, "h", None):
+            self.lib.gkmb200_lmer_table_free(self.h)
+            self.h = None
+
+    def __del__(self):
+        self.close()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
+
+    def weights(self):
+        """T as 4^L float64 values in lexicographic L-mer order (A, C, G, T = 0..3, first base most significant)"""
+        out = np.zeros(4 ** self.L)
+        _check(self.lib.gkmb200_lmer_table_get(self.h, out.ctypes.data_as(c_dbl_p)), self.lib)
+        return out
+
+    def scores(self, problem, row0, nrows, bias=0.0):
+        """bias + sum_c alpha[c] K(r, c) for the rows [row0, row0 + nrows) of `problem` (same parameters and GPUs)"""
+        out = np.zeros(nrows)
+        _check(self.lib.gkmb200_lmer_table_scores(self.h, problem.h, row0, nrows, bias, out.ctypes.data_as(c_dbl_p)), self.lib)
+        return out
+
+    def build_ms(self):
+        """device milliseconds of the build on the first GPU: (S, transform, combine)"""
+        out = np.zeros(3)
+        _check(self.lib.gkmb200_lmer_table_build_ms(self.h, out.ctypes.data_as(c_dbl_p)), self.lib)
+        return tuple(out)
 
 
 def svm_prepare_tasks(y, splits):

@@ -25,6 +25,8 @@
 #include "gkm_lmer_kernel.cuh"
 #include "gkm_mma_kernel.cuh"
 #include "gkm_index_dev.h"
+#include "gkm_lmer_table.h"
+#include "gkm_lmer_table_dev.h"
 #include "gkm_svm.h"
 
 #define GKM_MAX_DEV 16
@@ -1387,6 +1389,204 @@ extern "C" int gkm_dev_decision(gkmb200_problem *p, int row0, int nrows, int col
             if (b > nrows) b = nrows;
             if (e > nrows) e = nrows;
             return decision_slice(p, slot, row0 + b, e - b, col0, ncols, alpha, bias, out + b);
+        });
+    }
+    pthread_mutex_unlock(&g_lock);
+    return rc;
+}
+
+/* ------------------------------------------------------------------ */
+/* the L-mer table: the model folded into one weight per L-mer (DESIGN.md 4.5) */
+/* ------------------------------------------------------------------ */
+/* the folded model: one copy of T on every GPU of the problem it was built from */
+struct gkmb200_lmer_table {
+    gkm_parameter param;       /* of that problem: scoring needs the same (type, L, k, d, M, H) */
+    int ndev;
+    int dev[GKM_MAX_DEV];      /* the problem's GPUs, in its slot order */
+    double *T[GKM_MAX_DEV];    /* 4^L doubles per GPU, in code order (gkm_idx_code) */
+    double build_ms[3];        /* device time of S, the transform and the combine on the first GPU (CUDA events) */
+};
+
+/* one GPU's copy: sorted keys of the columns -> S -> transform -> T.  Everything but T is freed before returning. */
+static int lmer_table_slice(gkmb200_lmer_table *t, gkmb200_problem *p, int slot, int col0, int ncols, const double *alpha)
+{
+    gkm_devstate *ds = p->dev;
+    gkm_gpu *g = &g_gpu[ds->dev[slot]];
+    const gkm_image *im = &ds->img[slot];
+    const int L = p->param.L, d = p->param.d;
+    const size_t n = (size_t) 1 << (2 * L);
+    uint32_t *offs = (uint32_t *) malloc((size_t) ncols * 4);
+    if (!offs) { gkm_set_error("out of memory"); return 1; }
+    size_t P = 0;
+    for (int i = 0; i < ncols; i++) { offs[i] = (uint32_t) P; P += 2 * (size_t) (p->len[col0 + i] - L + 1); }
+    if (P > 0x7FFFFFF0u) { free(offs); gkm_set_error("L-mer table: %zu postings, at most %u", P, 0x7FFFFFF0u); return 1; }
+    size_t cub_bytes = 0;
+    const size_t sbytes = gkm_idx_scratch_bytes(P, L, &cub_bytes);
+    void *scratch = NULL, *d_offs = NULL;
+    double *d_alpha = NULL, *beta = NULL, *A = NULL, *T = NULL;
+    cudaEvent_t ev[4] = { NULL, NULL, NULL, NULL };
+    int rc = 0;
+    cudaError_t e = dev_malloc(g, &scratch, sbytes);
+    if (e == cudaSuccess) e = dev_malloc(g, &d_offs, (size_t) ncols * 4);
+    if (e == cudaSuccess) e = dev_malloc(g, (void **) &d_alpha, (size_t) ncols * sizeof(double));
+    if (e == cudaSuccess) e = dev_malloc(g, (void **) &beta, (size_t) ncols * sizeof(double));
+    if (e == cudaSuccess) e = dev_malloc(g, (void **) &A, (size_t) (d + 1) * n * sizeof(double));
+    if (e == cudaSuccess) e = dev_malloc(g, (void **) &T, n * sizeof(double));
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d_offs, offs, (size_t) ncols * 4, cudaMemcpyHostToDevice, g->sc);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d_alpha, alpha, (size_t) ncols * sizeof(double), cudaMemcpyHostToDevice, g->sc);
+    for (int i = 0; i < 4 && e == cudaSuccess && slot == 0; i++) e = cudaEventCreate(&ev[i]);
+    if (e != cudaSuccess) { gkm_set_error("CUDA: L-mer table buffers (%zu bytes of planes): %s", (size_t) (d + 2) * n * sizeof(double), cudaGetErrorString(e)); rc = 1; }
+    if (!rc) {
+        gkm_lt_build_args a;
+        memset(&a, 0, sizeof(a));
+        a.keys.planes = im->planes; a.keys.lens = im->lens; a.keys.wend = p->weighted ? im->wend : NULL;
+        a.keys.W = p->Wmax; a.keys.L = L; a.keys.cb = col0; a.keys.ce = col0 + ncols;
+        a.keys.offs = (const uint32_t *) d_offs; a.keys.P = P; a.keys.scratch = scratch; a.keys.cub_bytes = cub_bytes;
+        a.d = d; a.alpha = d_alpha; a.norm = im->sqnorm + col0; a.beta = beta; a.A = A; a.T = T; a.w = p->w;
+        rc = gkm_lt_build(&a, g->sc, slot == 0 ? ev : NULL);
+    }
+    /* pageable sources: wait for the build before letting go of them */
+    e = cudaStreamSynchronize(g->sc);
+    if (e != cudaSuccess && !rc) { gkm_set_error("CUDA: L-mer table build failed: %s", cudaGetErrorString(e)); rc = 1; }
+    if (!rc && slot == 0) {
+        for (int i = 0; i < 3; i++) {
+            float ms = 0.f;
+            cudaEventElapsedTime(&ms, ev[i], ev[i + 1]);
+            t->build_ms[i] = ms;
+        }
+    }
+    for (int i = 0; i < 4; i++) if (ev[i]) cudaEventDestroy(ev[i]);
+    free(offs);
+    cudaFree(scratch); cudaFree(d_offs); cudaFree(d_alpha); cudaFree(beta); cudaFree(A);
+    if (rc) { cudaFree(T); return 1; }
+    t->T[slot] = T;
+    return 0;
+}
+
+static void lmer_table_release(gkmb200_lmer_table *t)
+{
+    for (int i = 0; i < t->ndev; i++) {
+        if (!t->T[i]) continue;
+        if (cudaSetDevice(t->dev[i]) == cudaSuccess) cudaFree(t->T[i]);
+        else cudaGetLastError();
+        t->T[i] = NULL;
+    }
+}
+
+extern "C" gkmb200_lmer_table *gkmb200_lmer_table_new(gkmb200_problem *p, int col0, int ncols, const double *alpha)
+{
+    if (!p || !alpha) { gkm_set_error("null argument"); return NULL; }
+    const gkm_parameter *pa = &p->param;
+    if (pa->kernel_type == 3 || pa->kernel_type == 5) {
+        gkm_set_error("kernel type %d is an RBF kernel, not linear in the gkm features: it has no L-mer table", pa->kernel_type);
+        return NULL;
+    }
+    if (col0 < 0 || ncols < 1 || col0 > p->n - ncols) { gkm_set_error("columns [%d,+%d) outside the problem (n=%d)", col0, ncols, p->n); return NULL; }
+    if (ncols > GKM_LT_MAX_COLS) { gkm_set_error("L-mer table of %d columns: at most %d", ncols, GKM_LT_MAX_COLS); return NULL; }
+    if (gkm_lt_bytes(pa->L, pa->d) > GKM_LT_MAX_BYTES) {
+        gkm_set_error("L-mer table at L=%d d=%d needs %llu bytes per GPU, more than %llu", pa->L, pa->d, gkm_lt_bytes(pa->L, pa->d), GKM_LT_MAX_BYTES);
+        return NULL;
+    }
+    gkmb200_lmer_table *t = (gkmb200_lmer_table *) calloc(1, sizeof(*t));
+    if (!t) { gkm_set_error("out of memory"); return NULL; }
+    t->param = *pa;
+    pthread_mutex_lock(&g_lock);
+    int rc = upload_locked(p, 0);
+    if (!rc) {
+        t->ndev = p->dev->ndev;
+        for (int i = 0; i < t->ndev; i++) t->dev[i] = p->dev->dev[i];
+        rc = for_each_gpu(p->dev, [&](int slot) { return lmer_table_slice(t, p, slot, col0, ncols, alpha); });
+    }
+    if (rc) lmer_table_release(t);
+    pthread_mutex_unlock(&g_lock);
+    if (rc) { free(t); return NULL; }
+    return t;
+}
+
+extern "C" void gkmb200_lmer_table_free(gkmb200_lmer_table *t)
+{
+    if (!t) return;
+    pthread_mutex_lock(&g_lock);
+    lmer_table_release(t);
+    pthread_mutex_unlock(&g_lock);
+    free(t);
+}
+
+extern "C" int gkmb200_lmer_table_build_ms(const gkmb200_lmer_table *t, double *out)
+{
+    if (!t || !out) { gkm_set_error("null argument"); return 1; }
+    memcpy(out, t->build_ms, sizeof(t->build_ms));
+    return 0;
+}
+
+extern "C" int gkmb200_lmer_table_get(gkmb200_lmer_table *t, double *out)
+{
+    if (!t || !out) { gkm_set_error("null argument"); return 1; }
+    const size_t n = (size_t) 1 << (2 * t->param.L);
+    pthread_mutex_lock(&g_lock);
+    gkm_gpu *g = &g_gpu[t->dev[0]];
+    double *d_out = NULL;
+    int rc = 0;
+    cudaError_t e = cudaSetDevice(t->dev[0]);
+    if (e == cudaSuccess) e = dev_malloc(g, (void **) &d_out, n * sizeof(double));
+    if (e != cudaSuccess) { gkm_set_error("CUDA: L-mer table export: %s", cudaGetErrorString(e)); rc = 1; }
+    if (!rc) rc = gkm_lt_export(t->T[0], t->param.L, d_out, g->sc);
+    if (!rc) {
+        e = cudaMemcpyAsync(out, d_out, n * sizeof(double), cudaMemcpyDeviceToHost, g->sc);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(g->sc);
+        if (e != cudaSuccess) { gkm_set_error("CUDA: L-mer table export: %s", cudaGetErrorString(e)); rc = 1; }
+    }
+    cudaFree(d_out);
+    pthread_mutex_unlock(&g_lock);
+    return rc;
+}
+
+/* one GPU's slice of the rows of q */
+static int lmer_scores_slice(const gkmb200_lmer_table *t, gkmb200_problem *q, int slot, int row0, int nrows, double bias, double *out)
+{
+    if (nrows <= 0) return 0;
+    gkm_gpu *g = &g_gpu[q->dev->dev[slot]];
+    const gkm_image *im = &q->dev->img[slot];
+    double *d_out = NULL;
+    int rc = 0;
+    cudaError_t e = dev_malloc(g, (void **) &d_out, (size_t) nrows * sizeof(double));
+    if (e != cudaSuccess) { gkm_set_error("CUDA: L-mer table scores: %s", cudaGetErrorString(e)); return 1; }
+    rc = gkm_lt_score(t->T[slot], im->planes, im->lens, q->weighted ? im->wend : NULL, q->Wmax, q->param.L, im->sqnorm, row0, nrows, d_out, g->sc);
+    if (!rc) {
+        e = cudaMemcpyAsync(out, d_out, (size_t) nrows * sizeof(double), cudaMemcpyDeviceToHost, g->sc);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(g->sc);
+        if (e != cudaSuccess) { gkm_set_error("CUDA: L-mer table scores: %s", cudaGetErrorString(e)); rc = 1; }
+    }
+    cudaFree(d_out);
+    if (!rc) for (int i = 0; i < nrows; i++) out[i] += bias; /* as decision_slice adds it */
+    return rc;
+}
+
+extern "C" int gkmb200_lmer_table_scores(gkmb200_lmer_table *t, gkmb200_problem *q, int row0, int nrows, double bias, double *out)
+{
+    if (!t || !q || !out) { gkm_set_error("null argument"); return 1; }
+    const gkm_parameter *a = &t->param, *b = &q->param;
+    if (a->kernel_type != b->kernel_type || a->L != b->L || a->k != b->k || a->d != b->d || a->M != b->M || a->H != b->H) {
+        gkm_set_error("problem (type %d, L=%d, k=%d, d=%d, M=%d, H=%g) does not match the L-mer table (type %d, L=%d, k=%d, d=%d, M=%d, H=%g)",
+                      b->kernel_type, b->L, b->k, b->d, b->M, b->H, a->kernel_type, a->L, a->k, a->d, a->M, a->H);
+        return 1;
+    }
+    if (row0 < 0 || nrows < 0 || row0 > q->n - nrows) { gkm_set_error("rows [%d,+%d) outside the problem (n=%d)", row0, nrows, q->n); return 1; }
+    if (nrows == 0) return 0;
+    pthread_mutex_lock(&g_lock);
+    int rc = upload_locked(q, 0);
+    if (!rc) {
+        int same = q->dev->ndev == t->ndev;
+        for (int i = 0; same && i < t->ndev; i++) same = q->dev->dev[i] == t->dev[i];
+        if (!same) { gkm_set_error("the problem lives on other GPUs than the L-mer table (%d against %d)", q->dev->ndev, t->ndev); rc = 1; }
+    }
+    if (!rc) {
+        const int nd = t->ndev, per = ((nrows + nd - 1) / nd + 7) & ~7;
+        rc = for_each_gpu(q->dev, [&](int slot) {
+            int b = slot * per, e = b + per;
+            if (b > nrows) b = nrows;
+            if (e > nrows) e = nrows;
+            return lmer_scores_slice(t, q, slot, row0 + b, e - b, bias, out + b);
         });
     }
     pthread_mutex_unlock(&g_lock);

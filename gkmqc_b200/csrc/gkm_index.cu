@@ -42,13 +42,6 @@
 /* ------------------------------------------------------------------ */
 /* build                                                                */
 /* ------------------------------------------------------------------ */
-__device__ __forceinline__ uint32_t idx_window(const uint32_t *pl, int W, int lo, uint32_t mask)
-{
-    const int w = lo >> 5, s = lo & 31;
-    const uint32_t x = pl[w], y = (w + 1 < W) ? pl[w + 1] : 0u;
-    return __funnelshift_r(x, y, (uint32_t) s) & mask;
-}
-
 template <bool WEIGHTED>
 __global__ void __launch_bounds__(128)
 gkm_idx_keys_kernel(const uint32_t *__restrict__ planes, const int32_t *__restrict__ lens, const uint8_t *__restrict__ wend,
@@ -174,36 +167,62 @@ size_t gkm_idx_scratch_bytes(size_t P, int L, size_t *cub_bytes_out)
     return 2 * align256(P * 8) + 2 * align256(P * 4) + cubb + 256;
 }
 
+/* the scratch of a build: keys as generated | keys sorted | run lengths | overflow demands | cub temporary storage */
+struct idx_scratch {
+    unsigned long long *keys_a, *keys_b;
+    uint32_t *runlen, *need;
+    void *cub_tmp;
+};
+
+static idx_scratch idx_carve(const gkm_idx_build_args *a)
+{
+    const size_t P = a->P;
+    unsigned char *s = (unsigned char *) a->scratch;
+    idx_scratch r;
+    r.keys_a = (unsigned long long *) s; s += align256(P * 8);
+    r.keys_b = (unsigned long long *) s; s += align256(P * 8);
+    r.runlen = (uint32_t *) s; s += align256(P * 4);
+    r.need = (uint32_t *) s; s += align256(P * 4);
+    r.cub_tmp = s;
+    return r;
+}
+
+cudaError_t gkm_idx_sort_keys(const gkm_idx_build_args *a, cudaStream_t st, const unsigned long long **sorted)
+{
+    const idx_scratch sc = idx_carve(a);
+    size_t cub_bytes = a->cub_bytes;
+    if (a->wend) gkm_idx_keys_kernel<true><<<(unsigned) (a->ce - a->cb), 128, 0, st>>>(a->planes, a->lens, a->wend, a->W, a->L, a->cb, a->offs, sc.keys_a);
+    else gkm_idx_keys_kernel<false><<<(unsigned) (a->ce - a->cb), 128, 0, st>>>(a->planes, a->lens, a->wend, a->W, a->L, a->cb, a->offs, sc.keys_a);
+    /* the keys are generated in column order and the radix sort is stable: sorting by the code bits alone leaves
+     * every run in ascending column order (3 passes instead of 6 at L = 11) */
+    *sorted = sc.keys_b;
+    return cub::DeviceRadixSort::SortKeys(sc.cub_tmp, cub_bytes, sc.keys_a, sc.keys_b, (int) a->P, 32, 32 + 2 * a->L, st);
+}
+
 int gkm_idx_build(const gkm_idx_build_args *a, cudaStream_t st)
 {
     const size_t P = a->P;
     if (P == 0 || P > 0x7FFFFFF0u) { gkm_set_error("index block with %zu postings", P); return 1; }
-    unsigned char *s = (unsigned char *) a->scratch;
-    unsigned long long *keys_a = (unsigned long long *) s; s += align256(P * 8);
-    unsigned long long *keys_b = (unsigned long long *) s; s += align256(P * 8);
-    uint32_t *runlen = (uint32_t *) s; s += align256(P * 4);
-    uint32_t *need = (uint32_t *) s; s += align256(P * 4);
-    void *cub_tmp = s;
-    size_t cub_bytes = a->cub_bytes;
+    const idx_scratch sc = idx_carve(a);
+    uint32_t *runlen = sc.runlen, *need = sc.need;
+    void *cub_tmp = sc.cub_tmp;
+    size_t cub_bytes;
+    const unsigned long long *sorted;
     cudaError_t e;
     if ((e = cudaMemsetAsync(a->tab, 0xFF, gkm_idx_tab_bytes(a->L, a->fmt), st)) != cudaSuccess) goto fail;
-    if (a->wend) gkm_idx_keys_kernel<true><<<(unsigned) (a->ce - a->cb), 128, 0, st>>>(a->planes, a->lens, a->wend, a->W, a->L, a->cb, a->offs, keys_a);
-    else gkm_idx_keys_kernel<false><<<(unsigned) (a->ce - a->cb), 128, 0, st>>>(a->planes, a->lens, a->wend, a->W, a->L, a->cb, a->offs, keys_a);
-    /* the keys are generated in column order and the radix sort is stable: sorting by the code bits alone leaves
-     * every run in ascending column order (3 passes instead of 6 at L = 11) */
-    if ((e = cub::DeviceRadixSort::SortKeys(cub_tmp, cub_bytes, keys_a, keys_b, (int) P, 32, 32 + 2 * a->L, st)) != cudaSuccess) goto fail;
+    if ((e = gkm_idx_sort_keys(a, st, &sorted)) != cudaSuccess) goto fail;
     {
         const unsigned blocks = (unsigned) ((P + 255) / 256);
         unsigned long long *sumsq = (unsigned long long *) ((unsigned char *) cub_tmp + a->cub_bytes); /* in the slack behind the cub area */
         if ((e = cudaMemsetAsync(sumsq, 0, sizeof(*sumsq), st)) != cudaSuccess) goto fail;
-        gkm_idx_runs_kernel<<<blocks, 256, 0, st>>>(keys_b, (uint32_t) P, a->fmt, runlen, need, sumsq);
+        gkm_idx_runs_kernel<<<blocks, 256, 0, st>>>(sorted, (uint32_t) P, a->fmt, runlen, need, sumsq);
         if (a->h_sumsq && (e = cudaMemcpyAsync(a->h_sumsq, sumsq, sizeof(*sumsq), cudaMemcpyDeviceToHost, st)) != cudaSuccess) goto fail;
-        uint32_t *ovfofs = (uint32_t *) keys_a; /* the unsorted keys are dead now */
+        uint32_t *ovfofs = (uint32_t *) sc.keys_a; /* the unsorted keys are dead now */
         cub_bytes = a->cub_bytes;
         if ((e = cub::DeviceScan::ExclusiveSum(cub_tmp, cub_bytes, need, ovfofs, (int) P, st)) != cudaSuccess) goto fail;
-        if (a->fmt == GKM_IDX_FMT_C16) gkm_idx_fill_kernel<GKM_IDX_FMT_C16><<<blocks, 256, 0, st>>>(keys_b, (uint32_t) P, runlen, ovfofs, a->tab, a->ovf);
-        else if (a->fmt == GKM_IDX_FMT_W20) gkm_idx_fill_kernel<GKM_IDX_FMT_W20><<<blocks, 256, 0, st>>>(keys_b, (uint32_t) P, runlen, ovfofs, a->tab, a->ovf);
-        else gkm_idx_fill_kernel<GKM_IDX_FMT_P32><<<blocks, 256, 0, st>>>(keys_b, (uint32_t) P, runlen, ovfofs, a->tab, a->ovf);
+        if (a->fmt == GKM_IDX_FMT_C16) gkm_idx_fill_kernel<GKM_IDX_FMT_C16><<<blocks, 256, 0, st>>>(sorted, (uint32_t) P, runlen, ovfofs, a->tab, a->ovf);
+        else if (a->fmt == GKM_IDX_FMT_W20) gkm_idx_fill_kernel<GKM_IDX_FMT_W20><<<blocks, 256, 0, st>>>(sorted, (uint32_t) P, runlen, ovfofs, a->tab, a->ovf);
+        else gkm_idx_fill_kernel<GKM_IDX_FMT_P32><<<blocks, 256, 0, st>>>(sorted, (uint32_t) P, runlen, ovfofs, a->tab, a->ovf);
     }
     if ((e = cudaGetLastError()) != cudaSuccess) goto fail;
     return 0;

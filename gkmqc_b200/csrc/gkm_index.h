@@ -91,6 +91,13 @@ GKM_IDX_HD uint32_t gkm_idx_code(uint32_t p0, uint32_t p1, int L)
     return c;
 }
 
+/* the code bit that holds bit `hi` (0: the p0 bit, 1: the p1 bit) of base t of the window, in the layout above */
+GKM_IDX_HD int gkm_idx_base_bit(int t, int L, int hi)
+{
+    const int lb = gkm_idx_lowb(L);
+    return t < lb ? 2 * t + hi : (hi ? L : lb) + t;
+}
+
 GKM_IDX_HD uint32_t gkm_idx_posting(uint32_t col, uint32_t wt) { return col | (wt << GKM_IDX_COL_BITS); }
 
 /* number of XOR masks with at most d substituted bases: sum_{m<=d} C(L,m) 3^m (0 if it overflows 2^31) */

@@ -48,10 +48,23 @@ struct gkm_idx_rowargs {
     int maxq;      /* upper bound of query L-mers per row */
 };
 
+/* bits [lo, lo + L) of a bit plane of W words (mask = 2^L - 1): the window of the L-mer that starts at lo */
+static __device__ __forceinline__ uint32_t idx_window(const uint32_t *pl, int W, int lo, uint32_t mask)
+{
+    const int w = lo >> 5, s = lo & 31;
+    const uint32_t x = pl[w], y = (w + 1 < W) ? pl[w + 1] : 0u;
+    return __funnelshift_r(x, y, (uint32_t) s) & mask;
+}
+
 size_t gkm_idx_tab_bytes(int L, int fmt);
 size_t gkm_idx_ovf_bytes(size_t P, int fmt);
 size_t gkm_idx_scratch_bytes(size_t P, int L, size_t *cub_bytes_out);
 int gkm_idx_build(const gkm_idx_build_args *a, cudaStream_t st);
+/* the first steps of gkm_idx_build, shared with the L-mer table (gkm_lmer_table.cu): the keys code << 32 | column - cb << 8 |
+ * weight of every L-mer of both strands of the columns [cb, ce), radix-sorted by code (stable: by column inside a code,
+ * and in generation order inside a column).  Only planes .. P, scratch and cub_bytes of `a` are read; *sorted points
+ * into the scratch. */
+cudaError_t gkm_idx_sort_keys(const gkm_idx_build_args *a, cudaStream_t st, const unsigned long long **sorted);
 /* most columns one block may hold so that the hot histogram rows + the query fit 227 KB of shared memory (0: none) */
 int gkm_idx_max_cols(int nbins, int maxq, int weighted);
 unsigned gkm_idx_row_smem(int nbins, int ldh, int maxq, int weighted, int c16);

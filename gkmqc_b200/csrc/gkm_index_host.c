@@ -29,9 +29,7 @@ long long gkm_idx_delta_count(int L, int d)
 /* mask of a substitution by XOR value v (1..3) at base t (gkm_idx_code layout) */
 static uint32_t sub_mask(int t, int v, int L)
 {
-    const int lb = gkm_idx_lowb(L);
-    if (t < lb) return (uint32_t) v << (2 * t);
-    return ((uint32_t) (v & 1) << (lb + t)) | ((uint32_t) (v >> 1) << (L + t));
+    return ((uint32_t) (v & 1) << gkm_idx_base_bit(t, L, 0)) | ((uint32_t) (v >> 1) << gkm_idx_base_bit(t, L, 1));
 }
 
 struct emit_ctx {

@@ -150,6 +150,27 @@ int gkmb200_svm_cv_ex(gkmb200_problem *p, const double *kmat, long ld, int n, in
  * GPUs in one process every GPU writes its chunks straight into the first GPU's matrix (peer stores over NVLink). */
 int gkmb200_resident_rows(gkmb200_problem *p, int row0, int nrows, double *out, long ld);
 
+/* ---- the model folded into one weight per L-mer (kernel types 0, 1, 2, 4) ---- */
+/* A model f(r) = bias + sum_c alpha[c] K(r, c) of a kernel type that is linear in the gkm features is a table of 4^L
+ * weights T: f(r) = bias + (sum over the forward L-mers x of r of wt_r(x) T[x]) / |r|, whatever the number of SVs.
+ * T[u] is also the model's weight of the L-mer u: the score of the sequence u (exactly L bases) is T[u] / |u| + bias.
+ * The table needs (d + 2) 4^L doubles per GPU while it is built (A_0..A_d and T; 4^L stay); more than
+ * GKM_LT_MAX_BYTES (16 GiB: L = 16 always, L = 15 above d = 0) is refused, as are the RBF types 3 and 5 and more than
+ * 2^24 columns.  DESIGN.md 4.5. */
+typedef struct gkmb200_lmer_table gkmb200_lmer_table;
+/* the model sum_c alpha[c - col0] K(., c), c in [col0, col0 + ncols) of p, folded into T[4^L]; built on every GPU of p.
+ * NULL on failure (gkmb200_last_error) */
+gkmb200_lmer_table *gkmb200_lmer_table_new(gkmb200_problem *p, int col0, int ncols, const double *alpha);
+void gkmb200_lmer_table_free(gkmb200_lmer_table *t);
+/* out[4^L]: T in lexicographic L-mer order (A, C, G, T = 0..3, first base most significant) */
+int gkmb200_lmer_table_get(gkmb200_lmer_table *t, double *out);
+/* out[r - row0] = bias + sum_c alpha[c] K(r, c) for r in [row0, row0 + nrows) of q, evaluated through the table.  q may be
+ * the problem of the table or another one with the same (type, L, k, d, M, H) on the same GPUs; its rows are cut into
+ * one slice per GPU.  Equal to gkmb200_decision_values up to the rounding of two different summation orders. */
+int gkmb200_lmer_table_scores(gkmb200_lmer_table *t, gkmb200_problem *q, int row0, int nrows, double bias, double *out);
+/* out[3] = device milliseconds of the table's build on its first GPU: S (keys, sort, run sums), transform, combine */
+int gkmb200_lmer_table_build_ms(const gkmb200_lmer_table *t, double *out);
+
 /* the packed image as it lies on GPU 0: planes[n][3][W] (code bit 0, code bit 1, window-end plane E; both strands in one
  * circular string) and, weighted kernel types only, wend[n][32 W]; either may be NULL; out_shape = {n, W} */
 int gkmb200_problem_image(gkmb200_problem *p, uint32_t *planes, uint8_t *wend, int *out_shape);
