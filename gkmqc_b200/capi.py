@@ -146,6 +146,7 @@ def _declare(lib):
         ("gkmb200_lmer_table_get", [P, c_dbl_p]),
         ("gkmb200_lmer_table_scores", [P, P, I, I, ctypes.c_double, c_dbl_p]),
         ("gkmb200_lmer_table_build_ms", [P, c_dbl_p]),
+        ("gkmb200_lmer_table_substitutions", [P, P, ctypes.c_longlong, c_int_p, c_int_p, ctypes.c_double, c_dbl_p]),
         ("gkmb200_device_count", []),
         ("gkmb200_set_devices", [c_int_p, I]),
         ("gkmb200_set_option", [ctypes.c_char_p, ctypes.c_char_p]),
@@ -419,6 +420,27 @@ class LmerTable:
         out = np.zeros(nrows)
         _check(self.lib.gkmb200_lmer_table_scores(self.h, problem.h, row0, nrows, bias, out.ctypes.data_as(c_dbl_p)), self.lib)
         return out
+
+    def substitutions(self, problem, rows, pos, bias=0.0):
+        """out[i, v] = bias + the score of row rows[i] of `problem` with base pos[i] replaced by v (A, C, G, T = 0..3), bit for
+        bit what scores() gives for a problem holding that mutant; sites in any order, repeats allowed.  (nsites, 4)"""
+        rows = np.ascontiguousarray(rows, np.int32)
+        pos = np.ascontiguousarray(pos, np.int32)
+        if rows.shape != pos.shape or rows.ndim != 1:
+            raise ValueError("rows and pos must be 1-D arrays of one length")
+        out = np.zeros((len(rows), 4))
+        _check(self.lib.gkmb200_lmer_table_substitutions(self.h, problem.h, len(rows), rows.ctypes.data_as(c_int_p),
+                                                         pos.ctypes.data_as(c_int_p), bias, out.ctypes.data_as(c_dbl_p)), self.lib)
+        return out
+
+    def ism(self, problem, row0, nrows, bias=0.0):
+        """in-silico mutagenesis of the rows [row0, row0 + nrows): one (len, 4) array per row, entry [p, v] the score with base p
+        replaced by v (the row's own base gives its score), all through one substitutions() call"""
+        lens = [problem.seqlen(r) for r in range(row0, row0 + nrows)]
+        rows = np.repeat(np.arange(row0, row0 + nrows, dtype=np.int32), lens)
+        pos = np.concatenate([np.arange(n, dtype=np.int32) for n in lens]) if lens else np.zeros(0, np.int32)
+        out = self.substitutions(problem, rows, pos, bias)
+        return np.split(out, np.cumsum(lens)[:-1]) if lens else []
 
     def build_ms(self):
         """device milliseconds of the build on the first GPU: (S, transform, combine)"""

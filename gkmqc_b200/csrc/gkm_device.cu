@@ -1562,24 +1562,36 @@ static int lmer_scores_slice(const gkmb200_lmer_table *t, gkmb200_problem *q, in
     return rc;
 }
 
-extern "C" int gkmb200_lmer_table_scores(gkmb200_lmer_table *t, gkmb200_problem *q, int row0, int nrows, double bias, double *out)
+/* the checks of every use of a table on a problem q: the same (type, L, k, d, M, H) before anything is done ... */
+static int lmer_table_params_match(const gkmb200_lmer_table *t, const gkmb200_problem *q)
 {
-    if (!t || !q || !out) { gkm_set_error("null argument"); return 1; }
     const gkm_parameter *a = &t->param, *b = &q->param;
     if (a->kernel_type != b->kernel_type || a->L != b->L || a->k != b->k || a->d != b->d || a->M != b->M || a->H != b->H) {
         gkm_set_error("problem (type %d, L=%d, k=%d, d=%d, M=%d, H=%g) does not match the L-mer table (type %d, L=%d, k=%d, d=%d, M=%d, H=%g)",
                       b->kernel_type, b->L, b->k, b->d, b->M, b->H, a->kernel_type, a->L, a->k, a->d, a->M, a->H);
-        return 1;
+        return 0;
     }
+    return 1;
+}
+
+/* ... and, under g_lock, q uploaded to the table's GPUs in the table's slot order */
+static int lmer_table_upload(const gkmb200_lmer_table *t, gkmb200_problem *q)
+{
+    if (upload_locked(q, 0)) return 1;
+    int same = q->dev->ndev == t->ndev;
+    for (int i = 0; same && i < t->ndev; i++) same = q->dev->dev[i] == t->dev[i];
+    if (!same) { gkm_set_error("the problem lives on other GPUs than the L-mer table (%d against %d)", q->dev->ndev, t->ndev); return 1; }
+    return 0;
+}
+
+extern "C" int gkmb200_lmer_table_scores(gkmb200_lmer_table *t, gkmb200_problem *q, int row0, int nrows, double bias, double *out)
+{
+    if (!t || !q || !out) { gkm_set_error("null argument"); return 1; }
+    if (!lmer_table_params_match(t, q)) return 1;
     if (row0 < 0 || nrows < 0 || row0 > q->n - nrows) { gkm_set_error("rows [%d,+%d) outside the problem (n=%d)", row0, nrows, q->n); return 1; }
     if (nrows == 0) return 0;
     pthread_mutex_lock(&g_lock);
-    int rc = upload_locked(q, 0);
-    if (!rc) {
-        int same = q->dev->ndev == t->ndev;
-        for (int i = 0; same && i < t->ndev; i++) same = q->dev->dev[i] == t->dev[i];
-        if (!same) { gkm_set_error("the problem lives on other GPUs than the L-mer table (%d against %d)", q->dev->ndev, t->ndev); rc = 1; }
-    }
+    int rc = lmer_table_upload(t, q);
     if (!rc) {
         const int nd = t->ndev, per = ((nrows + nd - 1) / nd + 7) & ~7;
         rc = for_each_gpu(q->dev, [&](int slot) {
@@ -1587,6 +1599,99 @@ extern "C" int gkmb200_lmer_table_scores(gkmb200_lmer_table *t, gkmb200_problem 
             if (b > nrows) b = nrows;
             if (e > nrows) e = nrows;
             return lmer_scores_slice(t, q, slot, row0 + b, e - b, bias, out + b);
+        });
+    }
+    pthread_mutex_unlock(&g_lock);
+    return rc;
+}
+
+/* sites per launch of the substitution kernel: 16 MB of sites and 64 MB of results on the device, whatever nsites is */
+#define GKM_LS_CHUNK ((long long) 1 << 21)
+
+/* H(r, r) of the rows [r0, r1) into H ([r1 - r0][d + 1]): the upload's diagonal launch, with histograms kept */
+static int self_hist(gkmb200_problem *q, const gkm_image *im, gkm_gpu *g, int r0, int r1, int32_t *H)
+{
+    gkm_kparams kp;
+    fill_kparams(q, im, GKM_MODE_DIAG, &kp);
+    const int step = (pick_variant(q, GKM_MODE_DIAG) == GKM_KERNEL_DIAG) ? 131070 : 1024;
+    for (int r = r0; r < r1; r += step) {
+        kp.row_begin = kp.col_begin = kp.row_base = kp.col_base = r;
+        kp.row_end = kp.col_end = (r + step < r1) ? r + step : r1;
+        kp.hist = H + (size_t) (r - r0) * (size_t) q->nbins;
+        kp.hist_cols = 0; /* the diagonal: entry (r, r) lands at row r - row_base */
+        if (launch_hist(q, im, g, kp, g->sc, NULL)) return 1;
+    }
+    return 0;
+}
+
+/* one GPU's slice of the sites, in chunks of GKM_LS_CHUNK */
+static int lmer_subst_slice(const gkmb200_lmer_table *t, gkmb200_problem *q, int slot, long long nsites, const int *row, const int *pos,
+                            double bias, double *out)
+{
+    if (nsites <= 0) return 0;
+    gkm_gpu *g = &g_gpu[q->dev->dev[slot]];
+    const gkm_image *im = &q->dev->img[slot];
+    const long long cap = nsites < GKM_LS_CHUNK ? nsites : GKM_LS_CHUNK;
+    int *d_row = NULL, *d_pos = NULL;
+    int32_t *d_H = NULL;
+    double *d_out = NULL;
+    size_t hcap = 0;
+    int rc = 0;
+    cudaError_t e = dev_malloc(g, (void **) &d_row, (size_t) cap * sizeof(int));
+    if (e == cudaSuccess) e = dev_malloc(g, (void **) &d_pos, (size_t) cap * sizeof(int));
+    if (e == cudaSuccess) e = dev_malloc(g, (void **) &d_out, (size_t) cap * 4 * sizeof(double));
+    for (long long c0 = 0; e == cudaSuccess && !rc && c0 < nsites; c0 += cap) {
+        const long long nc = nsites - c0 < cap ? nsites - c0 : cap;
+        int rmin = row[c0], rmax = row[c0];
+        for (long long i = c0; i < c0 + nc; i++) { rmin = row[i] < rmin ? row[i] : rmin; rmax = row[i] > rmax ? row[i] : rmax; }
+        const size_t hbytes = (size_t) (rmax - rmin + 1) * (size_t) q->nbins * sizeof(int32_t);
+        if (hbytes > hcap) {
+            if ((e = cudaStreamSynchronize(g->sc)) != cudaSuccess) break;
+            cudaFree(d_H); d_H = NULL; hcap = 0;
+            if ((e = dev_malloc(g, (void **) &d_H, hbytes)) != cudaSuccess) break;
+            hcap = hbytes;
+        }
+        if ((e = cudaMemcpyAsync(d_row, row + c0, (size_t) nc * sizeof(int), cudaMemcpyHostToDevice, g->sc)) != cudaSuccess) break;
+        if ((e = cudaMemcpyAsync(d_pos, pos + c0, (size_t) nc * sizeof(int), cudaMemcpyHostToDevice, g->sc)) != cudaSuccess) break;
+        rc = self_hist(q, im, g, rmin, rmax + 1, d_H);
+        if (!rc) rc = gkm_lt_subst(t->T[slot], im->planes, im->lens, q->weighted ? im->wend : NULL, q->Wmax, q->param.L, q->param.d, q->w,
+                                   d_H, rmin, q->maxlen, d_row, d_pos, nc, d_out, g->sc);
+        if (!rc) {
+            e = cudaMemcpyAsync(out + 4 * c0, d_out, (size_t) nc * 4 * sizeof(double), cudaMemcpyDeviceToHost, g->sc);
+            if (e == cudaSuccess) e = cudaStreamSynchronize(g->sc);
+        }
+    }
+    if (e != cudaSuccess && !rc) { gkm_set_error("CUDA: L-mer table substitutions: %s", cudaGetErrorString(e)); rc = 1; }
+    cudaStreamSynchronize(g->sc); /* the pageable sources and the buffers stay until the stream has drained */
+    cudaFree(d_row); cudaFree(d_pos); cudaFree(d_out); cudaFree(d_H);
+    if (!rc) for (long long i = 0; i < 4 * nsites; i++) out[i] += bias; /* as lmer_scores_slice adds it */
+    return rc;
+}
+
+extern "C" int gkmb200_lmer_table_substitutions(gkmb200_lmer_table *t, gkmb200_problem *q, long long nsites, const int *row, const int *pos,
+                                                double bias, double *out)
+{
+    if (!t || !q) { gkm_set_error("null argument"); return 1; }
+    if (nsites < 0) { gkm_set_error("%lld sites", nsites); return 1; }
+    if (nsites > 0 && (!row || !pos || !out)) { gkm_set_error("null argument"); return 1; }
+    if (!lmer_table_params_match(t, q)) return 1;
+    for (long long i = 0; i < nsites; i++) {
+        if (row[i] < 0 || row[i] >= q->n) { gkm_set_error("site %lld: row %d outside the problem (n=%d)", i, row[i], q->n); return 1; }
+        if (pos[i] < 0 || pos[i] >= q->len[row[i]]) {
+            gkm_set_error("site %lld: position %d outside row %d (length %d)", i, pos[i], row[i], q->len[row[i]]);
+            return 1;
+        }
+    }
+    if (nsites == 0) return 0;
+    pthread_mutex_lock(&g_lock);
+    int rc = lmer_table_upload(t, q);
+    if (!rc) {
+        const long long nd = t->ndev, per = (nsites + nd - 1) / nd;
+        rc = for_each_gpu(q->dev, [&](int slot) {
+            long long b = slot * per, e = b + per;
+            if (b > nsites) b = nsites;
+            if (e > nsites) e = nsites;
+            return lmer_subst_slice(t, q, slot, e - b, row + b, pos + b, bias, out + 4 * b);
         });
     }
     pthread_mutex_unlock(&g_lock);

@@ -26,5 +26,11 @@ int gkm_lt_export(const double *T, int L, double *out, cudaStream_t st);
 /* out[r] = (sum over the forward L-mers of row row0 + r of wt * T[code]) / norm[row0 + r], r < nrows; wend = NULL: unit weights */
 int gkm_lt_score(const double *T, const uint32_t *planes, const int32_t *lens, const uint8_t *wend, int W, int L,
                  const double *norm, int row0, int nrows, double *out, cudaStream_t st);
+/* out[4 i + v] = (numerator of the row row[i] with base pos[i] replaced by v) / its norm, i < nsites (gkm_lmer_subst.h):
+ * H = the rows' self histograms, [rows][d + 1] int32 from row hrow0; w[0..d] host; maxlen = the longest row of the
+ * problem; row, pos, out device buffers.  Sites of one row are best consecutive: each block of 64 stages a row once per run. */
+int gkm_lt_subst(const double *T, const uint32_t *planes, const int32_t *lens, const uint8_t *wend, int W, int L, int d,
+                 const double *w, const int32_t *H, int hrow0, int maxlen, const int *row, const int *pos, long long nsites,
+                 double *out, cudaStream_t st);
 
 #endif

@@ -168,6 +168,17 @@ int gkmb200_lmer_table_get(gkmb200_lmer_table *t, double *out);
  * the problem of the table or another one with the same (type, L, k, d, M, H) on the same GPUs; its rows are cut into
  * one slice per GPU.  Equal to gkmb200_decision_values up to the rounding of two different summation orders. */
 int gkmb200_lmer_table_scores(gkmb200_lmer_table *t, gkmb200_problem *q, int row0, int nrows, double bias, double *out);
+/* Single-base substitutions (in-silico mutagenesis, variant effects): for the sites i < nsites, with 0 <= row[i] < n and
+ * 0 <= pos[i] < len(row[i]), in any order and repeats allowed,
+ *   out[4 i + v] = bias + the score of row[i] with base pos[i] replaced by v   (v = A, C, G, T = 0..3).
+ * Each entry equals, bit for bit, gkmb200_lmer_table_scores of a problem holding that mutated sequence, its norm as the
+ * upload computes it included (and the inf / NaN of a zero norm).  The entry of the row's own base (gkmb200_problem_codes:
+ * an N counts as A) is the row's unmutated score.  The norm and the sum are updated, not recomputed: only the <= L windows
+ * of each strand that cover the base change (DESIGN.md 4.6).  q as for gkmb200_lmer_table_scores; the sites are cut into
+ * one slice per GPU.  Refused: null pointers (when nsites > 0), nsites < 0, a row outside q, a position outside its row,
+ * mismatched parameters and other GPUs. */
+int gkmb200_lmer_table_substitutions(gkmb200_lmer_table *t, gkmb200_problem *q, long long nsites, const int *row, const int *pos,
+                                     double bias, double *out);
 /* out[3] = device milliseconds of the table's build on its first GPU: S (keys, sort, run sums), transform, combine */
 int gkmb200_lmer_table_build_ms(const gkmb200_lmer_table *t, double *out);
 
