@@ -28,7 +28,7 @@ int gkm_calc_weights(int kernel_type, int L, int k, double *w /* L+1 slots */);
 void gkm_calc_posweights(int nk, int kernel_type, int M, double H, uint8_t *wt, uint8_t *wt_rc);
 
 /* ---- the problem: sequences, their packed form, and (opaque) device state ---- */
-struct gkm_devstate; /* gkm_device.cu */
+struct gkm_devstate; /* gkm_dev.h */
 
 struct gkmb200_problem {
     gkm_parameter param;
@@ -99,8 +99,10 @@ int gkm_plan_chunks_rows(int row0, int nrows, int col0, int ncols, int lower, in
                          long long max_chunk_bytes, int max_rows, gkm_chunk *out, int max_chunks);
 /* which chunks belong to shard `rank` of `world` (round-robin by descending cost) */
 int gkm_chunk_owner(int chunk_index, int nchunks, int world);
+/* the index variant's column blocks: how many, and the width of all but the last in *cols */
+int gkm_plan_index_blocks(int span, int cap, int greedy, int *cols);
 
-/* ---- device layer (gkm_device.cu) ---- */
+/* ---- device layer (gkm_device.cu, gkm_compute.cu, gkm_resident.cu, gkm_microbench.cu) ---- */
 int gkm_dev_count(void);
 int gkm_dev_select(const int *ids, int n);
 int gkm_dev_upload(gkmb200_problem *p);            /* planes -> every selected GPU, sqnorm on GPU */

@@ -1,5 +1,5 @@
-/* gkm_sched.c -- how the kernel matrix is cut into chunks of row tiles and which
- * process owns which chunk.  Pure host logic (tested on CPU, world_size 2).
+/* gkm_sched.c -- how the kernel matrix is cut into chunks of row tiles and which process owns
+ * which chunk, and the index variant's column blocks.  Pure host logic (tested on CPU, world_size 2).
  *
  * The reference interleaves single rows over pthreads (gkmkern_pylib.c:70-90,
  * row a = i*NTHREADS + t) because row a costs ~a.  Here the unit is a chunk of
@@ -66,4 +66,17 @@ int gkm_chunk_owner(int chunk_index, int nchunks, int world)
     (void) nchunks;
     if (world <= 1) return 0;
     return chunk_index % world;
+}
+
+/* span columns in blocks of at most cap (a multiple of 32), block k = [k cols, min((k + 1) cols, span)): equal shares of
+ * whole warps of columns, or -- greedy -- full blocks first and the rest in the last one: in a lower triangle row a probes
+ * only the blocks that start below it, so the earlier a block ends the fewer rows pay for the next one. */
+int gkm_plan_index_blocks(int span, int cap, int greedy, int *cols)
+{
+    if (span < 1 || cap < 32) { *cols = 0; return 0; }
+    const int nblk = (span + cap - 1) / cap;
+    int c = (((span + nblk - 1) / nblk) + 31) & ~31;
+    if (c > cap || greedy) c = cap & ~31;
+    *cols = c;
+    return nblk;
 }

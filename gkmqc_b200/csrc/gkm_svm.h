@@ -1,4 +1,4 @@
-/* gkm_svm.h -- device side of the C-SVC cross-validation consumer (gkm_svm.cu), used by gkm_device.cu */
+/* gkm_svm.h -- device side of the C-SVC cross-validation consumer (gkm_svm.cu), used by gkm_resident.cu */
 #ifndef GKM_SVM_H_INCLUDED
 #define GKM_SVM_H_INCLUDED
 

@@ -1,4 +1,5 @@
-/* tests/emu/dev_stub.cc -- a host stand-in for the device layer (gkm_device.cu), for ONE purpose: to run the
+/* tests/emu/dev_stub.cc -- a host stand-in for the device layer (the gkm_dev_* functions of
+ * gkm_device.cu, gkm_compute.cu, gkm_resident.cu and gkm_microbench.cu), for ONE purpose: to run the
  * reference-ABI shim gkm_capi.c (gkmkernel_init / read_problems / new_object / build_tree / kernelfunc_batch[_all] /
  * swap_index / update_index, libgkm.h:132-147) in the CPU-only test tier, also under ASan + UBSan
  * (tools/asan_host.sh).  gkm_capi.c is pointer bookkeeping over caller-visible structs -- the code ADVICE r1 found a heap

@@ -6,7 +6,7 @@ Two launch-time choices decide which device code runs:
 * the compiled instance of the bit-sliced kernel, gkm_diag_kernel<L, NB, WEIGHTED, D4> (gkm_bitslice.h: gkm_diag_nb,
   gkm_diag_instance).  INSTANCE_CASES holds one case per instance the parameter gate lets a caller reach (86 of the 105
   compiled ones);
-* the tile shape launch_hist (gkm_device.cu) picks from the longest sequence of the problem: (TA, TB) of the bit-sliced
+* the tile shape launch_hist (gkm_launch.cu) picks from the longest sequence of the problem: (TA, TB) of the bit-sliced
   and lmer kernels (pick_tile, first candidate within 74 KB / 100 KB of shared memory) and the queries per CTA of the
   tcgen05 kernel, QA = min(4, 2176 // L-mers).  SHAPE_CASES holds one case per shape class, its longest sequence at the
   largest length of the class: the shared-memory footprint closest to the limit.

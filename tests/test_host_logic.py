@@ -198,7 +198,7 @@ def test_svm_task_preparation_follows_libsvm_grouping():
 def test_copy_threads_policy(monkeypatch):
     """the reference's nthreads (default 1 in bin/gkmqc.py) is only a lower bound on the copy-out threads: the library
     takes the cores of its affinity mask (no fixed cap: the 8-GPU box has 32), shared among the ranks of a
-    one-process-per-GPU run; GKM_COPY_THREADS overrides (gkm_device.cu:gkm_copy_threads_shared)"""
+    one-process-per-GPU run; GKM_COPY_THREADS overrides (gkm_compute.cu:gkm_copy_threads_shared)"""
     import ctypes
     lib = capi.load()
     for f in (lib.gkm_copy_threads, lib.gkm_copy_threads_shared):

@@ -89,3 +89,34 @@ def test_round_robin_ownership_is_balanced(n, world, index):
         assert max(rows) - min(rows) <= 2 * 592
     else:
         assert max(share) <= total / world + biggest
+
+
+def index_blocks(span, cap, greedy):
+    lib = capi.load()
+    lib.gkm_plan_index_blocks.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.POINTER(ctypes.c_int)]
+    cols = ctypes.c_int(-1)
+    nblk = lib.gkm_plan_index_blocks(span, cap, int(greedy), ctypes.byref(cols))
+    return nblk, cols.value
+
+
+def test_index_blocks_of_the_gpu_layout_tests():
+    """the layouts the GPU tier reads back (gkmb200_problem_index_layout), stated without a GPU: 150 columns under
+    index_cols = 128, and 20 000 columns under 16 384 (unit weights) or the compact weighted slots' 16 352"""
+    assert index_blocks(150, 128, False) == (2, 96)
+    assert index_blocks(150, 128, True) == (2, 128)
+    assert index_blocks(20000, 16384, False) == (2, 10016)
+    assert index_blocks(20000, 16384, True) == (2, 16384)
+    assert index_blocks(20000, 16352, True) == (2, 16352)
+
+
+@settings(derandomize=True, max_examples=300, deadline=None)
+@given(span=st.integers(1, 200000), cap=st.integers(1, 1024).map(lambda x: 32 * x), greedy=st.booleans())
+def test_index_blocks_tile_the_columns(span, cap, greedy):
+    """block k holds columns [k cols, min((k + 1) cols, span)) (ensure_index): every column in exactly one block, none
+    wider than the cap (a multiple of 32, as index_block_cap gives it), whole warps of columns but for the last block"""
+    nblk, cols = index_blocks(span, cap, greedy)
+    assert nblk == -(-span // cap) and cols % 32 == 0 and 0 < cols <= cap
+    blocks = [(k * cols, min((k + 1) * cols, span)) for k in range(nblk)]
+    assert blocks[-1][1] == span and all(ce > cb for cb, ce in blocks), "every block non-empty, the last ends the span"
+    if greedy:
+        assert cols == cap

@@ -1,5 +1,5 @@
 #!/bin/bash
-# builds variants of one CUDA source (-D flags; AB_UNIT = gkm_index (default) | gkm_device | gkm_svm) into
+# builds variants of one CUDA source (-D flags; AB_UNIT = gkm_index (default) | gkm_launch | gkm_svm) into
 # build/variants/<name>/gkmkern_pylib.so for A/B runs on the GPU:
 #   tools/ab_variants.sh name1:"-DFLAG1 -DFLAG2" name2:"" ...    then   GKM_PYLIB=build/variants/name1/gkmkern_pylib.so python tools/probe_r2.py variants
 set -e
