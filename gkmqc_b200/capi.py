@@ -132,6 +132,7 @@ def _declare(lib):
         ("gkmb200_get_stats", [P, ctypes.POINTER(gkmb200_stats)]),
         ("gkmb200_problem_index_layout", [P, c_int_p]),
         ("gkmb200_problem_launch_shape", [P, c_int_p]),
+        ("gkmb200_problem_index_blocks", [P, ctypes.POINTER(ctypes.c_longlong), I]),
         ("gkmb200_problem_image", [P, ctypes.c_void_p, ctypes.c_void_p, c_int_p]),
         ("gkmb200_resident_rows", [P, I, I, c_dbl_p, ctypes.c_long]),
         ("gkmb200_trim", []),
@@ -368,6 +369,22 @@ class Problem:
         out = (ctypes.c_int * 3)()
         _check(self.lib.gkmb200_problem_index_layout(self.h, out), self.lib)
         return tuple(out)
+
+    INDEX_BLOCK_FIELDS = ("cb", "ce", "fmt", "postings", "sumsq", "inst", "smem", "launches")
+
+    def index_blocks(self):
+        """the index variant's column blocks of the last compute call, on the first GPU: one dict per block with cb, ce
+        (columns), fmt (0 P32, 1 C16, 2 W20), postings, sumsq (sum of squared posting-list lengths), inst (bit
+        2 RANGE + MINB - 1 for each gkm_index_rows_kernel build that ran), smem (most dynamic shared memory of a launch)
+        and launches; [] when another variant ran"""
+        n = self.lib.gkmb200_problem_index_blocks(self.h, None, 0)
+        if n < 0:
+            raise GkmError(last_error(self.lib))
+        out = (ctypes.c_longlong * (8 * max(n, 1)))()
+        n = self.lib.gkmb200_problem_index_blocks(self.h, out, n)
+        if n < 0:
+            raise GkmError(last_error(self.lib))
+        return [dict(zip(self.INDEX_BLOCK_FIELDS, out[8 * k: 8 * k + 8])) for k in range(n)]
 
     def launch_shape(self):
         """(variant, TA, TB, dynamic shared memory bytes) of the last bit-sliced, lmer or mma launch for this problem on its

@@ -216,6 +216,29 @@ extern "C" int gkmb200_problem_index_layout(const gkmb200_problem *p, int *out)
     return 0;
 }
 
+/* the index blocks of the last compute call of this problem on its first GPU (0 when another variant ran); per block, up to
+ * max of them, 8 values from out[8 k]: {first column, end column, slot format, postings, sum of squared posting-list
+ * lengths, builds that ran (bit 2 RANGE + MINB - 1 of gkm_index_rows_kernel), most dynamic shared memory of a launch,
+ * launches}.  For tests: which row-kernel builds a call ran. */
+extern "C" int gkmb200_problem_index_blocks(const gkmb200_problem *p, long long *out, int max)
+{
+    if (!p || (!out && max > 0)) { gkm_set_error("null argument"); return -1; }
+    int nblk = 0;
+    pthread_mutex_lock(&g_lock);
+    if (p->dev && p->dev->variant == GKM_KERNEL_INDEX && p->dev->img[0].blk) {
+        const gkm_image *im = &p->dev->img[0];
+        nblk = im->nblk;
+        for (int k = 0; k < nblk && k < max; k++) {
+            const gkm_idx_block *b = &im->blk[k];
+            long long *o = out + 8 * (size_t) k;
+            o[0] = b->cb; o[1] = b->ce; o[2] = b->fmt; o[3] = (long long) b->postings; o[4] = (long long) b->sumsq;
+            o[5] = b->inst_mask; o[6] = b->max_smem; o[7] = b->launches;
+        }
+    }
+    pthread_mutex_unlock(&g_lock);
+    return nblk;
+}
+
 /* {variant, TA, TB, dynamic shared memory bytes} of the last bit-sliced, lmer or mma launch made for this problem on its
  * first GPU (mma: TA = queries per CTA, TB = 8); zeros if none.  For tests: which tile shape a problem ran. */
 extern "C" int gkmb200_problem_launch_shape(const gkmb200_problem *p, int *out)

@@ -555,23 +555,30 @@ int gkm_idx_max_cols(int nbins, int maxq, int weighted)
     return cols < 32 ? 0 : (int) cols;
 }
 
-int gkm_idx_rows(const gkm_kparams *kp, const gkm_idx_rowargs *ra, int weighted, cudaStream_t st)
+int gkm_idx_two_cta(int nbins, int blk_cols, int maxq, int weighted, int fmt, int nblk, double skew)
 {
-    const int rows = kp->row_end - kp->row_begin;
-    if (rows <= 0 || ra->bhi <= ra->blo) return 0;
-    const bool range = ra->blo != 0;
-    const int c16 = ra->fmt == GKM_IDX_FMT_C16;
-    const unsigned smem = gkm_idx_row_smem(kp->nbins, ra->ldh, ra->maxq, weighted, c16);
     /* Two CTAs per SM where two full histogram rows of the block fit shared memory (blocks up to ~12 000 columns):
      * that build is held to 32 registers, which the compact-slot code meets without spills (41.0 instead of 46.1 ms
      * at 10k).  The decision is per block, not per launch: mixing the two builds inside one problem measured
      * slower (28 288 sequences: 272 ms against 228 ms), and the 16-byte-slot code spills at 32 registers
      * (wgkm at 10k: 70 ms against 49 ms), so that format always runs one CTA per SM. */
-    const unsigned pair = 2u * (gkm_idx_row_smem(kp->nbins, (ra->blk_cols + 31) & ~31, ra->maxq, weighted, c16) + 1280u);
-    bool two = ra->fmt != GKM_IDX_FMT_P32 && pair <= (ra->nblk > 1 ? GKM_IDX_TWO_SMEM : 227u * 1024u);
+    const unsigned pair = 2u * (gkm_idx_row_smem(nbins, (blk_cols + 31) & ~31, maxq, weighted, fmt == GKM_IDX_FMT_C16) + 1280u);
+    if (fmt == GKM_IDX_FMT_P32 || pair > (nblk > 1 ? GKM_IDX_TWO_SMEM : 227u * 1024u)) return 0;
     /* weighted types on input with repeats (long-tailed rows): one CTA per SM (everything-mixed workload of
      * tools/nonuniform.py: 80 against 95 ms; uniform input: 50.4 against 47.4 ms the other way round) */
-    if (weighted && ra->skew > GKM_IDX_SKEW_ONE_CTA) two = false;
+    if (weighted && skew > GKM_IDX_SKEW_ONE_CTA) return 0;
+    return 1;
+}
+
+int gkm_idx_rows(const gkm_kparams *kp, const gkm_idx_rowargs *ra, int weighted, cudaStream_t st, gkm_idx_launch *ran)
+{
+    const int rows = kp->row_end - kp->row_begin;
+    if (ran) { ran->range = 0; ran->minb = 0; ran->smem = 0; }
+    if (rows <= 0 || ra->bhi <= ra->blo) return 0;
+    const bool range = ra->blo != 0;
+    const int c16 = ra->fmt == GKM_IDX_FMT_C16;
+    const unsigned smem = gkm_idx_row_smem(kp->nbins, ra->ldh, ra->maxq, weighted, c16);
+    const bool two = gkm_idx_two_cta(kp->nbins, ra->blk_cols, ra->maxq, weighted, ra->fmt, ra->nblk, ra->skew) != 0;
     if ((ra->fmt == GKM_IDX_FMT_C16 && weighted) || (ra->fmt == GKM_IDX_FMT_W20 && !weighted)) { gkm_set_error("index slot format does not match the kernel type"); return 1; }
     const void *fn;
 #define GKM_IDX_PICK(W, F) (range ? (two ? (const void *) gkm_index_rows_kernel<W, true, F, 2> : (const void *) gkm_index_rows_kernel<W, true, F, 1>) \
@@ -596,5 +603,6 @@ int gkm_idx_rows(const gkm_kparams *kp, const gkm_idx_rowargs *ra, int weighted,
         e = cudaLaunchKernel(fn, dim3((unsigned) rows, 1, 1), dim3(GKM_IDX_THREADS, 1, 1), args, smem, st);
     }
     if (e != cudaSuccess) { gkm_set_error("CUDA: index row kernel (%u bytes of shared memory): %s", smem, cudaGetErrorString(e)); return 1; }
+    if (ran) { ran->range = range; ran->minb = two ? 2 : 1; ran->smem = smem; }
     return 0;
 }

@@ -17,7 +17,14 @@ struct gkm_idx_block {
     size_t tab_bytes, ovf_bytes; /* block sizes as handed out by the pool */
     unsigned long long sumsq;    /* sum of squared posting-list lengths (gkm_idx_runs_kernel) */
     double skew;                 /* sumsq / postings: ~1 + postings per slot on uniform input, far more with repeats */
+    size_t postings;
     int built;
+    /* the row-kernel launches of this block since the compute call began (choose_variant clears them; first GPU only):
+     * bit 2 RANGE + MINB - 1 per build gkm_index_rows_kernel<., RANGE, ., MINB> that ran, the most dynamic shared memory
+     * one asked for, and the number of launches */
+    int inst_mask;
+    unsigned max_smem;
+    long long launches;
 };
 
 struct gkm_idx_build_args {
@@ -65,12 +72,25 @@ int gkm_idx_build(const gkm_idx_build_args *a, cudaStream_t st);
  * and in generation order inside a column).  Only planes .. P, scratch and cub_bytes of `a` are read; *sorted points
  * into the scratch. */
 cudaError_t gkm_idx_sort_keys(const gkm_idx_build_args *a, cudaStream_t st, const unsigned long long **sorted);
+/* host rules of the row kernel's launch, C linkage so that the CPU tests can call them */
+extern "C" {
 /* most columns one block may hold so that the hot histogram rows + the query fit 227 KB of shared memory (0: none) */
 int gkm_idx_max_cols(int nbins, int maxq, int weighted);
 unsigned gkm_idx_row_smem(int nbins, int ldh, int maxq, int weighted, int c16);
+/* 1 when the row kernel of a block of blk_cols columns (format fmt, one of nblk blocks, sum len^2 / postings = skew) runs
+ * two CTAs per SM, 0 for one */
+int gkm_idx_two_cta(int nbins, int blk_cols, int maxq, int weighted, int fmt, int nblk, double skew);
+}
 /* bytes of cold-bin scratch a launch of `rows` rows needs */
 size_t gkm_idx_cold_bytes(int nbins, int ldh, int rows);
-/* rows [kp->row_begin, kp->row_end) against the wanted columns of one block; outputs as in gkm_kparams */
-int gkm_idx_rows(const gkm_kparams *kp, const gkm_idx_rowargs *ra, int weighted, cudaStream_t st);
+/* the build gkm_index_rows_kernel<WEIGHTED, RANGE, FMT, MINB> a launch ran: RANGE, MINB (0: nothing launched) and its
+ * dynamic shared memory */
+struct gkm_idx_launch {
+    int range, minb;
+    unsigned smem;
+};
+/* rows [kp->row_begin, kp->row_end) against the wanted columns of one block; outputs as in gkm_kparams; *ran (may be NULL)
+ * tells which build ran */
+int gkm_idx_rows(const gkm_kparams *kp, const gkm_idx_rowargs *ra, int weighted, cudaStream_t st, gkm_idx_launch *ran);
 
 #endif

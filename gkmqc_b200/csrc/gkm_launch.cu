@@ -79,8 +79,15 @@ static int launch_index(const gkmb200_problem *p, const gkm_image *im, gkm_gpu *
             }
             ra.cold = g->d_cold[si];
         }
-        if (gkm_idx_rows(&kp, &ra, p->weighted, st)) return 1;
+        gkm_idx_launch ran;
+        if (gkm_idx_rows(&kp, &ra, p->weighted, st, &ran)) return 1;
         g->nkernels++;
+        if (im == &p->dev->img[0] && ran.minb) { /* what gkmb200_problem_index_blocks reports */
+            gkm_idx_block *bw = const_cast<gkm_idx_block *>(b);
+            bw->inst_mask |= 1 << (2 * ran.range + ran.minb - 1);
+            if (ran.smem > bw->max_smem) bw->max_smem = ran.smem;
+            bw->launches++;
+        }
     }
     return 0;
 }
@@ -373,6 +380,7 @@ static int ensure_index(gkmb200_problem *p, gkm_gpu *g, gkm_image *im, int col_b
         pool_free(g, scratch, scratch_got);
         pool_free(g, d_offs, offs_got);
         if (rc) return 1;
+        b->postings = P;
         b->skew = (double) b->sumsq / (double) (P ? P : 1);
         gkm_log(GKM_LOG_DEBUG, "index block %d: %zu postings, sum len^2 / postings = %.2f", k, P, b->skew);
         b->built = 1;
@@ -450,5 +458,9 @@ int choose_variant(gkmb200_problem *p, int row0, int nrows, int col0, int ncols,
     }
     (void) row0;
     ds->variant = v;
+    for (int k = 0; k < ds->img[0].nblk; k++) { /* the launch record starts over with every compute call */
+        gkm_idx_block *b = &ds->img[0].blk[k];
+        b->inst_mask = 0; b->max_smem = 0; b->launches = 0;
+    }
     return 0;
 }

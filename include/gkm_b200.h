@@ -189,6 +189,11 @@ int gkmb200_problem_image(gkmb200_problem *p, uint32_t *planes, uint8_t *wend, i
 /* ---- measurement ---- */
 /* out[3] = {column blocks, columns per block, first column} of the index variant's last compute call on p (zeros: another variant ran) */
 int gkmb200_problem_index_layout(const gkmb200_problem *p, int *out);
+/* the index variant's column blocks of the last compute call on p, on its first GPU: returns their number (0: another
+ * variant ran; -1: error) and fills 8 values per block for the first `max` of them: {first column, end column, slot format
+ * (0 P32, 1 C16, 2 W20), postings, sum of squared posting-list lengths, row-kernel builds that ran (bit 2 RANGE + MINB - 1),
+ * most dynamic shared memory of one launch, launches} */
+int gkmb200_problem_index_blocks(const gkmb200_problem *p, long long *out, int max);
 /* out[4] = {variant (1 lmer, 2 diag, 3 mma), TA, TB, dynamic shared memory bytes} of the last bit-sliced, lmer or mma launch
  * made for p on its first GPU (mma: TA = queries per CTA, TB = targets per CTA); zeros if none */
 int gkmb200_problem_launch_shape(const gkmb200_problem *p, int *out);

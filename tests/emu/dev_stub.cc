@@ -103,5 +103,7 @@ int gkm_dev_bench_lower(gkmb200_problem *, int, int, int, double *) { return no_
 int gkm_dev_microbench(const char *, double *) { return no_device("a micro-benchmark"); }
 int gkm_dev_svm_cv(gkmb200_problem *, const double *, long, int, int, const gkmb200_svm_task *, const int *, const signed char *,
                    const int *, double, double, int, double *, gkmb200_svm_fit *, double *) { return no_device("the SVM consumer"); }
+/* the index variant never runs here: the launch record (gkm_device.cu) has nothing to report */
+int gkmb200_problem_index_blocks(const gkmb200_problem *, long long *, int) { no_device("the index launch record"); return -1; }
 
 } /* extern "C" */

@@ -2,7 +2,8 @@
 
 tests/launch_grid.py names the cases: one per bit-sliced kernel instance a caller can reach, and one per tile-shape class
 of the bit-sliced, lmer and tcgen05 (mma) kernels.  Every case is compared with the oracle in each launch mode the library
-has (the sqnorm diagonal, the lower triangle, a rectangle across the diagonal, fused decision values), and
+has (the sqnorm diagonal, the lower triangle, a rectangle across the diagonal, a lower block off the origin, fused
+decision values), and
 gkmb200_problem_launch_shape confirms that the case ran the instance and the tile shape it was built for.  Each test
 records the shape it saw as the junit property "launch_shape" ((variant, TA, TB, shared bytes); mma: TA = queries per CTA).
 
@@ -89,6 +90,20 @@ def run_against_oracle(params, seqs, variant, ran, shape=None, diag_shape=None, 
         Kb = P.kernel_block(r0, n - r0, c0, c1 - c0)
         check_kmat(Kb, K[r0:, c0:c1], kt, "kernel_block")
         assert P.stats()["kernel_variant"] == ran
+        # a lower block off the origin (row0 > col0 > 0) through the raw ABI, into a NaN-filled buffer with ld > ncols: the
+        # entries below the diagonal and the unit diagonal are written, the cells above it and the padding stay NaN
+        lr0, lc0, lnc, ld = r0 + 4, c0 + 2, c1 - c0 - 2, c1 - c0 + 3
+        buf = np.full((n - lr0, ld), np.nan)
+        capi._check(P.lib.gkmb200_kernel_block(P.h, lr0, n - lr0, lc0, lnc, 1, buf.ctypes.data_as(capi.c_dbl_p), ld), P.lib)
+        rr, cc = np.arange(lr0, n)[:, None], np.arange(lc0, lc0 + lnc)[None, :]
+        want = np.full_like(buf, np.nan)
+        want[:, :lnc] = np.where(cc < rr, K[lr0:, lc0:lc0 + lnc], np.where(cc == rr, 1.0, np.nan))
+        if kt in launch_grid.RBF_TYPES:
+            np.testing.assert_allclose(buf, want, rtol=RTOL_RBF, atol=0, equal_nan=True, err_msg="lower block off the origin")
+        else:
+            assert np.array_equal(buf, want, equal_nan=True), "lower block off the origin"
+        assert P.stats()["kernel_variant"] == ran
+        expect(shape, "kernel_block lower off the origin")
         dv = P.decision_values(r0, n - r0, c0, c1 - c0, alpha, bias=0.25)
         # the device's own kernel values (RBF: within 1e-9 of the oracle's, checked above), summed exactly
         want, bound = pysvm.exact_scores(Kb, np.arange(n - r0), np.arange(c1 - c0), alpha, -0.25)
