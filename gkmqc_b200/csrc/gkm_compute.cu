@@ -414,6 +414,7 @@ static int decision_slice(gkmb200_problem *p, int slot, int row0, int nrows, int
     kp.alpha = d_alpha; kp.decision = d_dec;
     kp.col_begin = kp.col_base = col0; kp.col_end = col0 + ncols;
     kp.row_base = row0;
+    const long long k_before = g->nkernels;
     int launches = 0;
     /* index variant: whole waves of rows per launch, and a bounded cold-bin scratch */
     const int rows_per_launch = (ds->variant == GKM_KERNEL_INDEX) ? 16 * GKM_WAVE_ROWS : 8192;
@@ -422,6 +423,8 @@ static int decision_slice(gkmb200_problem *p, int slot, int row0, int nrows, int
         kp.row_end = (r + rows_per_launch < row0 + nrows) ? r + rows_per_launch : row0 + nrows;
         rc = launch_hist(p, &ds->img[slot], g, kp, (launches++ & 1) ? g->sc2 : g->sc, NULL);
     }
+    /* kernels, not row blocks: the index variant launches one per column block; the GPUs of a call add side by side */
+    __atomic_fetch_add(&p->stats.launches, g->nkernels - k_before, __ATOMIC_RELAXED);
     if (!rc) {
         rc = (cudaStreamSynchronize(g->sc2) != cudaSuccess) ||
              (cudaMemcpyAsync(out, d_dec, sizeof(double) * (size_t) nrows, cudaMemcpyDeviceToHost, g->sc) != cudaSuccess) ||
@@ -442,8 +445,10 @@ extern "C" int gkm_dev_decision(gkmb200_problem *p, int row0, int nrows, int col
         return 1;
     }
     pthread_mutex_lock(&g_lock);
+    p->stats.launches = 0;
     int rc = upload_locked(p, 0);
     if (!rc) rc = choose_variant(p, row0, nrows, col0, ncols, 0);
+    if (!rc) p->stats.kernel_variant = p->dev->variant;
     if (!rc) rc = for_each_gpu_share(p->dev, nrows, 8, [&](int slot, long long b, long long e) {
         return decision_slice(p, slot, row0 + (int) b, (int) (e - b), col0, ncols, alpha, bias, out + b);
     });

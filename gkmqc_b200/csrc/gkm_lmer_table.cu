@@ -386,6 +386,7 @@ static int lmer_scores_slice(const gkmb200_lmer_table *t, gkmb200_problem *q, in
     if (e == cudaSuccess) e = cudaMemcpyAsync(out, d_out, (size_t) nrows * sizeof(double), cudaMemcpyDeviceToHost, g->sc);
     if (e == cudaSuccess) e = cudaStreamSynchronize(g->sc);
     if (e != cudaSuccess) { gkm_set_error("CUDA: L-mer table scores: %s", cudaGetErrorString(e)); return 1; }
+    __atomic_fetch_add(&q->stats.launches, 1, __ATOMIC_RELAXED);
     for (int i = 0; i < nrows; i++) out[i] += bias; /* as decision_slice adds it */
     return 0;
 }
@@ -419,6 +420,7 @@ extern "C" int gkmb200_lmer_table_scores(gkmb200_lmer_table *t, gkmb200_problem 
     if (row0 < 0 || nrows < 0 || row0 > q->n - nrows) { gkm_set_error("rows [%d,+%d) outside the problem (n=%d)", row0, nrows, q->n); return 1; }
     if (nrows == 0) return 0;
     pthread_mutex_lock(&g_lock);
+    q->stats.launches = 0;
     int rc = lmer_table_upload(t, q);
     if (!rc) rc = for_each_gpu_share(q->dev, nrows, 8, [&](int slot, long long b, long long e) {
         return lmer_scores_slice(t, q, slot, row0 + (int) b, (int) (e - b), bias, out + b);
@@ -463,7 +465,9 @@ static int lmer_subst_slice(const gkmb200_lmer_table *t, gkmb200_problem *q, int
         gkm_kparams kp;
         fill_kparams(q, im, GKM_MODE_DIAG, &kp);
         kp.hist = d_H;
-        if (launch_diag_rows(q, im, g, rmin, rmax + 1, kp) < 0) { rc = 1; break; }
+        const int diag = launch_diag_rows(q, im, g, rmin, rmax + 1, kp);
+        if (diag < 0) { rc = 1; break; }
+        __atomic_fetch_add(&q->stats.launches, diag + 1, __ATOMIC_RELAXED);
         e = gkm_lt_subst(t->T[slot], im->planes, im->lens, q->weighted ? im->wend : NULL, q->Wmax, q->param.L, q->param.d, q->w,
                          d_H, rmin, q->maxlen, d_row, d_pos, nc, d_out, g->sc);
         if (e == cudaSuccess) e = cudaMemcpyAsync(out + 4 * c0, d_out, (size_t) nc * 4 * sizeof(double), cudaMemcpyDeviceToHost, g->sc);
@@ -491,6 +495,7 @@ extern "C" int gkmb200_lmer_table_substitutions(gkmb200_lmer_table *t, gkmb200_p
     }
     if (nsites == 0) return 0;
     pthread_mutex_lock(&g_lock);
+    q->stats.launches = 0;
     int rc = lmer_table_upload(t, q);
     if (!rc) rc = for_each_gpu_share(q->dev, nsites, 1, [&](int slot, long long b, long long e) {
         return lmer_subst_slice(t, q, slot, e - b, row + b, pos + b, bias, out + 4 * b);

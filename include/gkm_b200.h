@@ -27,7 +27,12 @@ typedef struct gkmb200_stats {
     double kernel_ms;        /* device time of the histogram kernels of the last compute call (CUDA events) */
     double wall_ms;          /* host wall time of the last compute call */
     double upload_ms;        /* pack + H2D + sqnorm of the last upload */
-    long long launches;      /* kernel launches of the last compute call */
+    long long launches;      /* kernel launches of the last call on this problem, over all its GPUs: an upload, a compute
+                              * call, decision values, or (on the scored problem) L-mer table scores and substitutions.
+                              * An upload or index build the call made is included (pack 1, sqnorm 1 per diagonal step,
+                              * index 5 per column block).  Decision values: one per row block of 8 192 rows (index: one per
+                              * column block per 2 368 rows); scores: one per GPU share; substitutions: per batch of 2^21
+                              * sites, the diagonal launches of its rows plus one */
     long long entries;       /* kernel entries produced by the last compute call */
     long long lmer_pairs;    /* L-mer pair comparisons those entries stand for */
     long long h2d_bytes;     /* bytes copied host->device by the last upload */
