@@ -79,7 +79,8 @@ _lib = None
 
 
 def lib_path():
-    # GKM_PYLIB: another build of the same library (kernel A/B runs, tools/ab_variants.sh); the product path is bin/
+    # GKM_PYLIB: another build of the same library (the sanitised host build of tools/asan_host.sh, or a build that
+    # tools/mma_time.py and tools/wgkm_time.py time); the product path is bin/
     return os.environ.get("GKM_PYLIB") or os.path.join(BIN_DIR, LIB_NAME)
 
 

@@ -5,6 +5,7 @@
 
 #include "gkm_dev.h"
 #include "gkm_options.h"
+#include "gkm_pack.h"
 
 gkm_gpu g_gpu[GKM_MAX_DEV];
 int g_sel[GKM_MAX_DEV];
@@ -179,7 +180,7 @@ void pool_free(gkm_gpu *g, void *ptr, size_t bytes)
 }
 
 
-/* the image as it lies on GPU 0 (tests: device packing against the host packer): planes [n][3][W] and, for the
+/* the image as it lies on GPU 0 (tests: the device packer against a model of the image): planes [n][3][W] and, for the
  * weighted kernel types, wend [n][32 W]; either pointer may be NULL.  out_shape = {n, W}. */
 extern "C" int gkmb200_problem_image(gkmb200_problem *p, uint32_t *planes, uint8_t *wend, int *out_shape)
 {
@@ -289,43 +290,29 @@ extern "C" void gkm_dev_release(gkmb200_problem *p)
     p->dev = NULL;
 }
 
-/* ---- packing on the device (SURVEY.md 8f/f2): base codes -> the image of 3 ---- */
-/* What gkm_seq.c:pack_worker does on the host (it stays there for the CPU emulators of the test tier), one CTA per
- * sequence, one warp per 32-position word of the circular string.  The input is the sequence TEXT, one byte per base as
- * the FASTA file or the caller spelled it: the letter -> code rule (A,C,G,T in either case -> 0..3, anything else -> A,
- * libgkm.c:864-875; gkm_base_code) is applied here.  Layout: forward strand at [0, len), reverse complement
- * (3 - code, mirrored: libgkm.c:878-888) at [len, 2 len), zero padding; plane bits by warp ballot; E = positions at
- * which an L-mer of either strand may end; wend[j] = positional weight of the L-mer ending at j, looked up by its
- * distance from the centre L-mer in a table the host computed with the reference's expression (libgkm.c:910-932) --
- * no exp() on the device, so the bytes are the host's. */
+/* ---- packing on the device (SURVEY.md 8f/f2): sequence letters -> the image of 3 ---- */
+/* The rule of gkm_pack.h, one CTA per sequence, one warp per 32-position word of the circular string, plane bits by warp
+ * ballot.  The input is the sequence TEXT, one byte per base as the FASTA file or the caller spelled it. */
 template <bool WEIGHTED>
 __global__ void __launch_bounds__(128)
 gkm_pack_kernel(const uint8_t *__restrict__ codes, const unsigned long long *__restrict__ off, const int32_t *__restrict__ lens,
                 int W, int L, const uint8_t *__restrict__ wtab, uint32_t *__restrict__ planes, uint8_t *__restrict__ wend)
 {
     const int i = (int) blockIdx.x;
-    const int len = lens[i], nk = len - L + 1, centre = nk / 2;
+    const int len = lens[i], centre = (len - L + 1) / 2;
     const uint8_t *c = codes + off[i];
     const int lane = (int) threadIdx.x & 31;
     for (int wi = (int) threadIdx.x >> 5; wi < W; wi += 4) {
         const int j = wi * 32 + lane;
-        uint32_t code = 0;
-        int s = -1; /* start index (forward-strand numbering of wt[]) of the L-mer that ends at j, if any */
-        if (j < len) {
-            code = gkm_base_code(c[j]);
-            if (j >= L - 1) s = j - (L - 1);
-        } else if (j < 2 * len) {
-            code = 3u - gkm_base_code(c[2 * len - 1 - j]);
-            const int rel = j - len;
-            if (rel >= L - 1) s = nk - 1 - (rel - (L - 1)); /* wt_rc[t] = wt[nk - 1 - t] */
-        }
+        int s;
+        const uint32_t code = gkm_pack_code(c, len, L, j, &s);
         const uint32_t p0 = __ballot_sync(0xFFFFFFFFu, code & 1u), p1 = __ballot_sync(0xFFFFFFFFu, code & 2u);
         const uint32_t pe = __ballot_sync(0xFFFFFFFFu, s >= 0);
         if (lane == 0) {
             uint32_t *pl = planes + (size_t) i * 3 * (size_t) W;
             pl[wi] = p0; pl[W + wi] = p1; pl[2 * W + wi] = pe;
         }
-        if (WEIGHTED) wend[(size_t) i * 32 * (size_t) W + (size_t) j] = (s >= 0) ? wtab[abs(centre - s)] : (uint8_t) 0;
+        if (WEIGHTED) wend[(size_t) i * 32 * (size_t) W + (size_t) j] = gkm_pack_weight(wtab, centre, s);
     }
 }
 
@@ -349,10 +336,9 @@ int upload_locked(gkmb200_problem *p, int need_host)
     if (ensure_selected()) return 1;
     const double t0 = now_ms();
     gkm_dev_release(p);
-    const int pack_host = gkm_opt_pack_host();
-    if (pack_host ? gkm_pack_problem(p) : gkm_shape_problem(p)) return 1;
+    if (gkm_shape_problem(p)) return 1;
     uint8_t wtab[GKM_MAX_BASES + 1];
-    if (!pack_host && p->weighted) gkm_posweight_table(p->param.kernel_type, p->param.M, p->param.H, wtab);
+    if (p->weighted) gkm_posweight_table(p->param.kernel_type, p->param.M, p->param.H, wtab);
     gkm_devstate *ds = (gkm_devstate *) calloc(1, sizeof(gkm_devstate));
     if (!ds) { gkm_set_error("out of memory"); return 1; }
     p->dev = ds;
@@ -370,28 +356,19 @@ int upload_locked(gkmb200_problem *p, int need_host)
         CK(cudaMemcpyAsync(im->lens, p->len, n * sizeof(int32_t), cudaMemcpyHostToDevice, g->sc));
         h2d += (long long) (n * sizeof(int32_t));
         if (p->weighted && pool_alloc(g, (void **) &im->wend, &im->wend_bytes, n * 32 * W)) return 1;
-        if (pack_host) {
-            CK(cudaMemcpyAsync(im->planes, p->planes, n * 3 * W * sizeof(uint32_t), cudaMemcpyHostToDevice, g->sc));
-            h2d += (long long) (n * 3 * W * sizeof(uint32_t));
-            if (p->weighted) {
-                CK(cudaMemcpyAsync(im->wend, p->wend, n * 32 * W, cudaMemcpyHostToDevice, g->sc));
-                h2d += (long long) (n * 32 * W);
-            }
-        } else {
-            /* one byte per base goes up (3 MB at 10k x 300 bp; the packed image of a weighted problem was 8.3 MB) and the
-             * GPU packs: codes | offsets | weight table in one block */
-            const size_t off_at = (p->arena_len + 15) & ~(size_t) 15, tab_at = off_at + n * sizeof(unsigned long long);
-            if (pool_alloc(g, (void **) &im->codes, &im->codes_bytes, tab_at + sizeof(wtab))) return 1;
-            CK(cudaMemcpyAsync(im->codes, p->arena, p->arena_len, cudaMemcpyHostToDevice, g->sc));
-            CK(cudaMemcpyAsync(im->codes + off_at, p->off, n * sizeof(unsigned long long), cudaMemcpyHostToDevice, g->sc));
-            if (p->weighted) CK(cudaMemcpyAsync(im->codes + tab_at, wtab, sizeof(wtab), cudaMemcpyHostToDevice, g->sc));
-            h2d += (long long) (p->arena_len + n * sizeof(unsigned long long) + (p->weighted ? sizeof(wtab) : 0));
-            const unsigned long long *d_off = (const unsigned long long *) (im->codes + off_at);
-            if (p->weighted) gkm_pack_kernel<true><<<(unsigned) n, 128, 0, g->sc>>>(im->codes, d_off, im->lens, (int) W, p->param.L, im->codes + tab_at, im->planes, im->wend);
-            else gkm_pack_kernel<false><<<(unsigned) n, 128, 0, g->sc>>>(im->codes, d_off, im->lens, (int) W, p->param.L, NULL, im->planes, NULL);
-            CK(cudaGetLastError());
-            p->stats.launches++;
-        }
+        /* one byte per base goes up (3 MB at 10k x 300 bp, against 8.3 MB for the packed image of a weighted problem) and
+         * the GPU packs: codes | offsets | weight table in one block */
+        const size_t off_at = (p->arena_len + 15) & ~(size_t) 15, tab_at = off_at + n * sizeof(unsigned long long);
+        if (pool_alloc(g, (void **) &im->codes, &im->codes_bytes, tab_at + sizeof(wtab))) return 1;
+        CK(cudaMemcpyAsync(im->codes, p->arena, p->arena_len, cudaMemcpyHostToDevice, g->sc));
+        CK(cudaMemcpyAsync(im->codes + off_at, p->off, n * sizeof(unsigned long long), cudaMemcpyHostToDevice, g->sc));
+        if (p->weighted) CK(cudaMemcpyAsync(im->codes + tab_at, wtab, sizeof(wtab), cudaMemcpyHostToDevice, g->sc));
+        h2d += (long long) (p->arena_len + n * sizeof(unsigned long long) + (p->weighted ? sizeof(wtab) : 0));
+        const unsigned long long *d_off = (const unsigned long long *) (im->codes + off_at);
+        if (p->weighted) gkm_pack_kernel<true><<<(unsigned) n, 128, 0, g->sc>>>(im->codes, d_off, im->lens, (int) W, p->param.L, im->codes + tab_at, im->planes, im->wend);
+        else gkm_pack_kernel<false><<<(unsigned) n, 128, 0, g->sc>>>(im->codes, d_off, im->lens, (int) W, p->param.L, NULL, im->planes, NULL);
+        CK(cudaGetLastError());
+        p->stats.launches++;
         /* sqnorm: Kraw(a,a) by the same kernel in diagonal mode */
         gkm_kparams kp;
         fill_kparams(p, im, GKM_MODE_DIAG, &kp);

@@ -36,7 +36,7 @@
 /* queue entry: (list, bin row, weight).  Compact slots: 4 bytes; 16-byte slots: 8 bytes.  The queues are kept small on
  * purpose: at 10 000 columns two CTAs per SM need 2 x (80 KB histogram + queues + query) of shared memory, and
  * every KB beyond 196 KB per SM moves the L1/shared split to its last step (28 KB of L1 instead of 60), which
- * measured 4 % slower (the in-flight slot probes live in L1 lines): tools/ab_variants.sh, DESIGN.md 4.4. */
+ * measured 4 % slower (the in-flight slot probes live in L1 lines): DESIGN.md 4.4. */
 #define GKM_IDX_QBYTES_FMT(c16) ((GKM_IDX_THREADS / 32) * (GKM_IDX_QCAP + GKM_IDX_LQCAP) * ((c16) ? 4 : 8) + (GKM_IDX_THREADS / 32) * 4)
 
 /* ------------------------------------------------------------------ */

@@ -46,8 +46,8 @@ struct gkmb200_problem {
     int nonacgt;   /* characters mapped to 'A' so far */
 
     /* shape of the packed image (gkm_shape_problem); the image itself is built ON THE DEVICE from the arena
-     * (gkm_device.cu: gkm_pack_kernel).  planes / wend on the host exist only after gkm_pack_problem, which the CPU
-     * emulators of the test tier and the pack = host A/B option use. */
+     * (gkm_device.cu: gkm_pack_kernel).  planes / wend on the host exist only after gkm_pack_problem, which only the CPU
+     * emulators of the test tier call; both packers apply the rule of gkm_pack.h. */
     int packed;
     int Wmax;        /* 32-bit words per bit plane = ceil(2*maxlen / 32): both strands in one circular string */
     int Wa;          /* ceil(maxlen / 32): 32-position chunks of a query */
@@ -66,7 +66,7 @@ struct gkmb200_problem {
 int gkm_problem_reserve(gkmb200_problem *p, int extra);
 void gkm_problem_shard_from_env(gkmb200_problem *p); /* GKM_SHARD="rank/world": gkm_main_pywrapper only */
 int gkm_shape_problem(gkmb200_problem *p);   /* Wmax, Wa, sqnorm buffer; no image */
-int gkm_pack_problem(gkmb200_problem *p);    /* + the image on the host */
+int gkm_pack_problem(gkmb200_problem *p);    /* + the image on the host (CPU emulators only) */
 static inline const uint8_t *gkm_letters(const gkmb200_problem *p, int i) { return p->arena + p->off[i]; }
 /* A,C,G,T (either case) -> 0..3; anything else counts as 'A' (libgkm.c:864-875).  With the case bit cleared the four letters
  * are 0x41, 0x43, 0x47, 0x54: t = (ch >> 1) & 3 is 0,1,3,2 and t ^ (t >> 1) is 0,1,2,3.  The device packer

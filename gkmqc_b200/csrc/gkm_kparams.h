@@ -7,7 +7,7 @@
 enum { GKM_MODE_RECT = 0, GKM_MODE_LOWER = 1, GKM_MODE_DIAG = 2 };
 
 struct gkm_kparams {
-    /* device-resident problem image (gkm_seq.c: gkm_pack_problem) */
+    /* device-resident problem image (gkm_pack.h; packed by gkm_device.cu: gkm_pack_kernel) */
     const uint32_t *planes; /* [n][3][W]: code bit 0, code bit 1, valid-window-end plane; both strands, circular */
     const int32_t *lens;    /* [n] */
     const uint8_t *wend;    /* [n][32W], weighted kernel types only */

@@ -17,9 +17,10 @@
  *   builders     2 warps expand the target L-mers of the next N tile into a 2-stage ring of B operands
  *   MMA warp     one elected thread issues the two K = 32 MMAs of tile (A[mt], B[stage]) into one of TWO 256-column
  *                accumulators and commits to its mbarrier; a commit per B stage hands the stage back to the builders
- *   epilogue     8 warps (TMEM lane quarter x column half) read an accumulator with tcgen05.ld.32x32b.x32, reject groups
- *                of 16 by a 3-input max tree (VIMNMX3), bin the rest, and hand the accumulator back -- the MMA of tile
- *                n + 1 runs under the epilogue of tile n
+ *   epilogue     16 warps (TMEM lane quarter x column group of 64) read an accumulator with one
+ *                tcgen05.ld.32x32b.x32.pack::16b (two 16-bit columns per register), hand it back -- the MMA of tile n + 1
+ *                runs under the epilogue of tile n -- reject groups of 16 registers by an OR tree on the hit bit that
+ *                the operands' bias sets (a max tree at L = 16), and bin the rest
  *
  * It exists for the measured comparison with the bit-sliced kernel (DESIGN.md 4.3): every accumulator -- one per L-mer
  * PAIR -- has to leave TMEM and meet at least half a CUDA-core instruction.  Selected with GKM_KERNEL=mma.
@@ -31,14 +32,9 @@
 
 #include "gkm_diag_kernel.cuh" /* gkm_emit_entry */
 
-#ifndef GKM_MMA_EPI
 #define GKM_MMA_EPI 16           /* epilogue warps: TMEM lane quarter (w & 3) x column group (w >> 2) */
-#endif
 #define GKM_MMA_CW (GKM_MMA_N / (GKM_MMA_EPI / 4))   /* accumulator columns per epilogue warp */
-#ifndef GKM_MMA_PACK16
-#define GKM_MMA_PACK16 1         /* tcgen05.ld ... .pack::16b: two adjacent accumulator columns per register (0: one) */
-#endif
-#define GKM_MMA_NV (GKM_MMA_PACK16 ? GKM_MMA_CW / 2 : GKM_MMA_CW)   /* registers of one epilogue thread per tile */
+#define GKM_MMA_NV (GKM_MMA_CW / 2)                  /* registers of one epilogue thread per tile: two columns each */
 #define GKM_MMA_HSETS (GKM_MMA_EPI / 4)              /* histogram sets: one per column group */
 #define GKM_MMA_THREADS ((GKM_MMA_EPI + 4) * 32)     /* epilogue warps, then MMA, TMA, two builder warps */
 #define GKM_MMA_M 128
@@ -48,9 +44,6 @@
 #define GKM_MMA_ROWS_CAP 2176    /* stacked query L-mers per CTA (17 tiles of 128: 136 KB of A operand) */
 #define GKM_MMA_BUILDERS 64
 #define GKM_MMA_TMA_BOX 256      /* elements of one TMA box along a plane row, at most */
-#ifndef GKM_MMA_EXP
-#define GKM_MMA_EXP 0            /* timing experiments (tools/ab_variants.sh): 1 no compares, 2 no MMA, 4 no B build, 8 no TMEM loads */
-#endif
 
 struct gkm_mma_args {
     int QA;        /* queries per CTA for this launch: min(4, ROWS_CAP / longest query) */
@@ -265,7 +258,7 @@ gkm_mma_kernel(const __grid_constant__ gkm_kparams p, const __grid_constant__ gk
             const int lenB = bars->lenB[b_l], nkB = lenB - L + 1;
             gkm_mbar_wait(&bars->b_empty[s], ((uint32_t) (t >> 1) & 1u) ^ 1u);
             const uint32_t *plb = sPl + (size_t) (GKM_MMA_QA + b_l) * SW;
-            for (int r = bt; r < ((GKM_MMA_EXP & 4) ? 0 : GKM_MMA_N); r += GKM_MMA_BUILDERS) {
+            for (int r = bt; r < GKM_MMA_N; r += GKM_MMA_BUILDERS) {
                 const int jj = GKM_MMA_N * nt + r;
                 const bool valid = jj < 2 * nkB;
                 const int strand = (jj >= nkB) ? 1 : 0;
@@ -294,7 +287,7 @@ gkm_mma_kernel(const __grid_constant__ gkm_kparams p, const __grid_constant__ gk
                     gkm_mbar_wait(&bars->acc_empty[buf], ((uint32_t) (j >> 1) & 1u) ^ 1u);
                     asm volatile("tcgen05.fence::after_thread_sync;");
 #pragma unroll
-                    for (int ks = 0; ks < ((GKM_MMA_EXP & 2) ? 0 : 2); ks++) { /* K = 64 bytes = two K = 32 instructions = chunks (2ks, 2ks+1) */
+                    for (int ks = 0; ks < 2; ks++) { /* K = 64 bytes = two K = 32 instructions = chunks (2ks, 2ks+1) */
                         const uint64_t adesc = gkm_umma_desc(gkm_smem_u32(sAop + (size_t) mt * GKM_MMA_M * 64 + (size_t) ks * 2 * GKM_MMA_M * 16), GKM_MMA_M, 8);
                         const uint64_t bdesc = gkm_umma_desc(gkm_smem_u32(sBop + (size_t) s * GKM_MMA_N * 64 + (size_t) ks * 2 * GKM_MMA_N * 16), GKM_MMA_N, 8);
                         const uint32_t acc = ks ? 1u : 0u;
@@ -309,7 +302,7 @@ gkm_mma_kernel(const __grid_constant__ gkm_kparams p, const __grid_constant__ gk
         }
         __syncwarp();
     } else if (warp < GKM_MMA_EPI) {
-        /* ---- epilogue: thread = one stacked query L-mer (TMEM lane), 128 target L-mers in 4 loads of 32 columns ---- */
+        /* ---- epilogue: thread = one stacked query L-mer (TMEM lane), 64 target L-mers in one load of 32 registers ---- */
         const int thr = L - d; /* matches needed for a hit; the launcher guarantees thr >= 1 */
         const int lane_base = 32 * (warp & 3), col_half = (warp >> 2) * GKM_MMA_CW;
         int j = 0;
@@ -320,29 +313,19 @@ gkm_mma_kernel(const __grid_constant__ gkm_kparams p, const __grid_constant__ gk
                 const int i = mt * GKM_MMA_M + lane_base + lane;
                 gkm_mbar_wait(&bars->acc_full[buf], (uint32_t) (j >> 1) & 1u);
                 asm volatile("tcgen05.fence::after_thread_sync;");
-                /* all columns of this warp's group are requested before the first is looked at (four load -> wait -> compare
-                 * rounds exposed the TMEM latency four times per tile).  GKM_MMA_PACK16: two adjacent columns per register. */
+                /* one load brings all 64 columns of this warp's group, two adjacent columns per register, before the first
+                 * is looked at (four load -> wait -> compare rounds exposed the TMEM latency four times per tile) */
+                static_assert(GKM_MMA_NV == 32, "one tcgen05.ld .x32 per tile");
                 uint32_t v[GKM_MMA_NV];
                 const uint32_t taddr = tmem_base + ((uint32_t) lane_base << 16) + (uint32_t) (buf * GKM_MMA_N + col_half);
-#define GKM_LDTM32(o, c, PK) \
-                asm volatile("tcgen05.ld.sync.aligned.32x32b.x32" PK ".b32 " \
-                             "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, " \
-                             "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];\n" \
-                             : "=r"(v[o + 0]), "=r"(v[o + 1]), "=r"(v[o + 2]), "=r"(v[o + 3]), "=r"(v[o + 4]), "=r"(v[o + 5]), "=r"(v[o + 6]), "=r"(v[o + 7]), \
-                               "=r"(v[o + 8]), "=r"(v[o + 9]), "=r"(v[o + 10]), "=r"(v[o + 11]), "=r"(v[o + 12]), "=r"(v[o + 13]), "=r"(v[o + 14]), "=r"(v[o + 15]), \
-                               "=r"(v[o + 16]), "=r"(v[o + 17]), "=r"(v[o + 18]), "=r"(v[o + 19]), "=r"(v[o + 20]), "=r"(v[o + 21]), "=r"(v[o + 22]), "=r"(v[o + 23]), \
-                               "=r"(v[o + 24]), "=r"(v[o + 25]), "=r"(v[o + 26]), "=r"(v[o + 27]), "=r"(v[o + 28]), "=r"(v[o + 29]), "=r"(v[o + 30]), "=r"(v[o + 31]) \
-                             : "r"(taddr + (uint32_t) (c)))
-                if (GKM_MMA_EXP & 8) { for (int u = 0; u < GKM_MMA_NV; u++) v[u] = 0; }
-                else if (GKM_MMA_PACK16) {
-                    GKM_LDTM32(0, 0, ".pack::16b");
-                    if (GKM_MMA_NV > 32) GKM_LDTM32(32 % GKM_MMA_NV, 64, ".pack::16b");
-                } else {
-                    GKM_LDTM32(0, 0, "");
-                    if (GKM_MMA_NV > 32) GKM_LDTM32(32 % GKM_MMA_NV, 32, "");
-                    if (GKM_MMA_NV > 64) { GKM_LDTM32(64 % GKM_MMA_NV, 64, ""); GKM_LDTM32(96 % GKM_MMA_NV, 96, ""); }
-                }
-#undef GKM_LDTM32
+                asm volatile("tcgen05.ld.sync.aligned.32x32b.x32.pack::16b.b32 "
+                             "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
+                             "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];\n"
+                             : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
+                               "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]),
+                               "=r"(v[16]), "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]),
+                               "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
+                             : "r"(taddr));
                 asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
                 /* the accumulator is in registers: hand it back to the MMA warp before the compares */
                 asm volatile("tcgen05.fence::before_thread_sync;");
@@ -362,16 +345,14 @@ gkm_mma_kernel(const __grid_constant__ gkm_kparams p, const __grid_constant__ gk
                      * A hit is rare per accumulator (0.12 % at L = 11, d = 3) but not per WARP: one of the 32 lanes has one
                      * in a fifth of the groups, and every lane then walks the slow path.  So the slow path is a second look
                      * at the five partial ORs of the tree (three registers each) and only then at single accumulators. */
-                    constexpr uint32_t HB = GKM_MMA_PACK16 ? 0x80008000u : 0x8000u;
+                    constexpr uint32_t HB = 0x80008000u;
                     auto look = [&](int r) {
                         const uint32_t x = v[r];
-                        if (GKM_MMA_PACK16) {
-                            if (x & 0x8000u) hit(2 * r, (int) (x & 0x7FFFu) + thr);
-                            if (x & 0x80000000u) hit(2 * r + 1, (int) ((x >> 16) & 0x7FFFu) + thr);
-                        } else if (x & 0x8000u) hit(r, (int) (x & 0x7FFFu) + thr);
+                        if (x & 0x8000u) hit(2 * r, (int) (x & 0x7FFFu) + thr);
+                        if (x & 0x80000000u) hit(2 * r + 1, (int) ((x >> 16) & 0x7FFFu) + thr);
                     };
 #pragma unroll
-                    for (int g = 0; g < ((GKM_MMA_EXP & 1) ? 0 : GKM_MMA_NV); g += 16) {
+                    for (int g = 0; g < GKM_MMA_NV; g += 16) {
                         uint32_t tr[5];
 #pragma unroll
                         for (int k = 0; k < 5; k++) tr[k] = v[g + 3 * k] | v[g + 3 * k + 1] | v[g + 3 * k + 2];
@@ -389,21 +370,19 @@ gkm_mma_kernel(const __grid_constant__ gkm_kparams p, const __grid_constant__ gk
                 } else {
                     /* L = 16: no spare K byte for the bias; 3-input max tree (VIMNMX3) on the plain match counts */
 #pragma unroll
-                    for (int g = 0; g < ((GKM_MMA_EXP & 1) ? 0 : GKM_MMA_NV); g += 16) {
+                    for (int g = 0; g < GKM_MMA_NV; g += 16) {
                         int mx = 0;
 #pragma unroll
                         for (int u = 0; u < 16; u++) {
                             const uint32_t x = v[g + u];
-                            mx = max(mx, GKM_MMA_PACK16 ? max((int) (x & 0xFFFFu), (int) (x >> 16)) : (int) x);
+                            mx = max(mx, max((int) (x & 0xFFFFu), (int) (x >> 16)));
                         }
                         if (mx >= thr) {
 #pragma unroll
                             for (int u = 0; u < 16; u++) {
                                 const uint32_t x = v[g + u];
-                                if (GKM_MMA_PACK16) {
-                                    if ((int) (x & 0xFFFFu) >= thr) hit(2 * (g + u), (int) (x & 0xFFFFu));
-                                    if ((int) (x >> 16) >= thr) hit(2 * (g + u) + 1, (int) (x >> 16));
-                                } else if ((int) x >= thr) hit(g + u, (int) x);
+                                if ((int) (x & 0xFFFFu) >= thr) hit(2 * (g + u), (int) (x & 0xFFFFu));
+                                if ((int) (x >> 16) >= thr) hit(2 * (g + u) + 1, (int) (x >> 16));
                             }
                         }
                     }

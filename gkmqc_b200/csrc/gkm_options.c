@@ -7,7 +7,6 @@
  *   GKM_CHUNK_MB = n                       upper bound of one chunk's dense output
  *   GKM_INDEX_COLS = n                     upper bound of the columns of one index block (tests: forces several blocks)
  *   GKM_INDEX_SPLIT = equal | greedy       how a column range is cut into index blocks: equal shares, or full blocks first
- *   GKM_PACK     = device | host           who builds the 2-bit plane image from the base codes (default: the GPU)
  *   GKM_DEVICES  = "0,1,.."                GPUs to use (gkm_device.cu)
  */
 #include <stdlib.h>
@@ -22,7 +21,6 @@ static int g_max_L = 12;
 static int g_chunk_mb = 128; /* 50k x 50k: 686 ms per pass with 64 MB chunks (one wave of 148 rows each), 671 with 128, 669 with 256 */
 static int g_index_cols = 0;
 static int g_index_wide = 0;
-static int g_pack_host = 0;
 static int g_index_greedy = -1; /* -1: the library decides per call */
 
 static int parse_kernel(const char *v, int *out)
@@ -46,7 +44,6 @@ static void load_env(void)
     if ((v = getenv("GKM_CHUNK_MB")) != NULL) { int x = atoi(v); if (x >= 1 && x <= 4096) g_chunk_mb = x; }
     if ((v = getenv("GKM_INDEX_COLS")) != NULL) { int x = atoi(v); if (x >= 32) g_index_cols = x & ~31; }
     if ((v = getenv("GKM_INDEX_WIDE")) != NULL) g_index_wide = atoi(v) != 0;
-    if ((v = getenv("GKM_PACK")) != NULL) g_pack_host = !strcmp(v, "host");
     if ((v = getenv("GKM_INDEX_SPLIT")) != NULL) g_index_greedy = !strcmp(v, "greedy") ? 1 : !strcmp(v, "equal") ? 0 : -1;
 }
 
@@ -55,7 +52,6 @@ int gkm_opt_max_L(void) { load_env(); return g_max_L; }
 int gkm_opt_chunk_mb(void) { load_env(); return g_chunk_mb; }
 int gkm_opt_index_cols(void) { load_env(); return g_index_cols; }
 int gkm_opt_index_wide(void) { load_env(); return g_index_wide; }
-int gkm_opt_pack_host(void) { load_env(); return g_pack_host; }
 int gkm_opt_index_greedy(void) { load_env(); return g_index_greedy; }
 
 int gkmb200_set_option(const char *key, const char *value)
@@ -84,11 +80,6 @@ int gkmb200_set_option(const char *key, const char *value)
     }
     if (!strcmp(key, "index_wide")) { /* 1: 16-byte slots even where the compact 8-byte ones would do (A/B, tests) */
         g_index_wide = x != 0;
-        return 0;
-    }
-    if (!strcmp(key, "pack")) { /* device (default): the GPU packs the bit planes from one byte per base; host: gkm_seq.c does (A/B, tests) */
-        if (strcmp(value, "host") && strcmp(value, "device")) { gkm_set_error("pack must be host or device"); return 1; }
-        g_pack_host = !strcmp(value, "host");
         return 0;
     }
     if (!strcmp(key, "index_split")) { /* equal: blocks of equal size; greedy: full blocks first, the rest last; auto: per call */

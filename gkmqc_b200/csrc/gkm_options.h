@@ -9,7 +9,6 @@ int gkm_opt_max_L(void);
 int gkm_opt_chunk_mb(void);
 int gkm_opt_index_cols(void);
 int gkm_opt_index_wide(void);
-int gkm_opt_pack_host(void);
 int gkm_opt_index_greedy(void); /* 1 greedy, 0 equal, -1 per call */
 #ifdef __cplusplus
 }

@@ -1,24 +1,25 @@
-/* gkm_seq.c -- sequences of a problem: FASTA input, base coding, 2-bit plane packing.
+/* gkm_seq.c -- sequences of a problem: FASTA input, base coding, the shape of the 2-bit plane image.
  *
  * Host-side counterpart of gkmkernel_new_object (libgkm.c:841-938) and
  * read_fasta_file (libgkm.c:1251-1314).  What the reference keeps per sequence as
- * byte arrays (seq, seq_rc, wt, wt_rc) is packed here into the image the kernels
- * read: two bit planes per strand (bit p of plane b = bit b of the base code at
- * position p, A,C,G,T = 0,1,2,3) and, for the weighted kernel types, the positional
- * weights re-indexed by window END position.  sqnorm is NOT computed here -- it is
- * the diagonal of the kernel and comes from the GPU (gkm_device.cu).
+ * byte arrays (seq, seq_rc, wt, wt_rc) becomes the image the kernels read: two bit
+ * planes per strand (bit p of plane b = bit b of the base code at position p,
+ * A,C,G,T = 0,1,2,3) and, for the weighted kernel types, the positional weights
+ * re-indexed by window END position (gkm_pack.h).  The GPU packs it (gkm_device.cu);
+ * gkm_pack_problem builds the same image here for the CPU emulators.  sqnorm is NOT
+ * computed here -- it is the diagonal of the kernel and comes from the GPU.
  */
 #include <ctype.h>
 #if defined(__SSE2__)
 #include <emmintrin.h>
 #endif
 #include <pthread.h>
-#include <unistd.h>
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
 
 #include "gkm_internal.h"
+#include "gkm_pack.h"
 
 gkmb200_problem *gkmb200_problem_new(const gkm_parameter *param)
 {
@@ -353,114 +354,6 @@ void gkm_unpack_problem(gkmb200_problem *p)
     p->host_sqnorm = 0;
 }
 
-struct pack_job { gkmb200_problem *p; int i0, i1; };
-
-static inline uint32_t gkm_bitrev32(uint32_t x)
-{
-    x = ((x >> 1) & 0x55555555u) | ((x & 0x55555555u) << 1);
-    x = ((x >> 2) & 0x33333333u) | ((x & 0x33333333u) << 2);
-    x = ((x >> 4) & 0x0F0F0F0Fu) | ((x & 0x0F0F0F0Fu) << 4);
-    return __builtin_bswap32(x);
-}
-
-static void *pack_worker(void *arg)
-{
-    const struct pack_job *job = (const struct pack_job *) arg;
-    gkmb200_problem *p = job->p;
-    const int L = p->param.L, W = p->Wmax;
-    uint8_t wt[GKM_MAX_BASES + 1], wt_rc[GKM_MAX_BASES + 1];
-    int wt_nk = -1; /* positional weights depend on the number of L-mers only: reuse them across equal lengths */
-    for (int i = job->i0; i < job->i1; i++) {
-        const int n = p->len[i];
-        uint8_t c[GKM_MAX_BASES + 9]; /* base codes of this sequence (+ slack: the loop below reads eight at a time) */
-        for (int j = 0; j < n; j++) c[j] = gkm_base_code(gkm_letters(p, i)[j]);
-        memset(c + n, 0, 8);
-        uint32_t *pl = p->planes + (size_t) i * 3 * (size_t) W;
-        /* Forward strand: bit b of the codes, eight bases per multiply (the byte-to-bit gather trick); the reverse
-         * complement half is the forward half mirrored and complemented (3 - c = ~c & 3; libgkm.c:878-888), so it
-         * comes from the forward words by bit reversal instead of a second pass over the bases.  (The first
-         * version set one bit per loop iteration: 2 ms of the 50 ms call at 10k sequences.) */
-        uint32_t f0[GKM_MAX_BASES / 32 + 2], f1[GKM_MAX_BASES / 32 + 2];
-        const int nwf = (n + 31) / 32;
-        for (int wi = 0; wi < nwf; wi++) {
-            uint32_t w0 = 0, w1 = 0;
-            const int base = wi * 32;
-            int b = 0;
-            for (; b + 8 <= 32 && base + b + 8 <= n; b += 8) {
-                uint64_t x;
-                memcpy(&x, c + base + b, 8);
-                w0 |= (uint32_t) ((((x & 0x0101010101010101ULL) * 0x0102040810204080ULL) >> 56) & 0xFFu) << b;
-                w1 |= (uint32_t) (((((x >> 1) & 0x0101010101010101ULL) * 0x0102040810204080ULL) >> 56) & 0xFFu) << b;
-            }
-            for (; b < 32 && base + b < n; b++) {
-                w0 |= (uint32_t) (c[base + b] & 1u) << b;
-                w1 |= (uint32_t) ((c[base + b] >> 1) & 1u) << b;
-            }
-            f0[wi] = w0;
-            f1[wi] = w1;
-        }
-        f0[nwf] = f1[nwf] = 0;
-        /* bit j of the mirrored complement, j in [0, n): ~forward bit n-1-j.  Word wi of it = the bit-reversed
-         * forward bits [n - 32 (wi + 1), n - 32 wi), taken from the two words that hold them. */
-        for (int wi = 0; wi * 32 < 2 * n; wi++) {
-            uint32_t w0 = 0, w1 = 0, we = 0;
-            for (int half = 0; half < 2; half++) {
-                /* output bits [lo, hi) of this word that belong to strand `half` */
-                const int s0 = half ? n : 0, s1 = half ? 2 * n : n;
-                int lo = wi * 32 > s0 ? wi * 32 : s0, hi = wi * 32 + 32 < s1 ? wi * 32 + 32 : s1;
-                if (hi <= lo) continue;
-                const int cnt = hi - lo, sh = lo - wi * 32;
-                const uint32_t m = (cnt >= 32) ? 0xFFFFFFFFu : ((1u << cnt) - 1u);
-                uint32_t v0, v1;
-                if (!half) {
-                    const int q = lo >> 5, r = lo & 31; /* forward bits [lo, hi) */
-                    v0 = (uint32_t) ((((uint64_t) f0[q + 1] << 32) | f0[q]) >> r);
-                    v1 = (uint32_t) ((((uint64_t) f1[q + 1] << 32) | f1[q]) >> r);
-                } else {
-                    /* rc positions j = lo - n .. hi - n - 1  <->  forward positions n-1-j: the forward bits
-                     * [n - (hi - n), n - (lo - n)) reversed and complemented */
-                    const int fb = 2 * n - hi; /* first forward bit of the span */
-                    const int q = fb >> 5, r = fb & 31;
-                    uint32_t g0 = (uint32_t) ((((uint64_t) f0[q + 1] << 32) | f0[q]) >> r);
-                    uint32_t g1 = (uint32_t) ((((uint64_t) f1[q + 1] << 32) | f1[q]) >> r);
-                    /* reverse the low cnt bits */
-                    g0 = gkm_bitrev32(g0) >> (32 - cnt);
-                    g1 = gkm_bitrev32(g1) >> (32 - cnt);
-                    v0 = ~g0;
-                    v1 = ~g1;
-                }
-                w0 |= (v0 & m) << sh;
-                w1 |= (v1 & m) << sh;
-                /* E: positions at which an L-mer of this strand may end: rel >= L - 1 */
-                const int e0 = s0 + L - 1 > lo ? s0 + L - 1 : lo;
-                if (hi > e0) {
-                    const int ec = hi - e0;
-                    const uint32_t em = (ec >= 32) ? 0xFFFFFFFFu : ((1u << ec) - 1u);
-                    we |= em << (e0 - wi * 32);
-                }
-            }
-            pl[0 * W + wi] = w0;
-            pl[1 * W + wi] = w1;
-            pl[2 * W + wi] = we;
-        }
-        if (p->weighted) {
-            const int nk = n - L + 1;
-            if (nk != wt_nk) { gkm_calc_posweights(nk, p->param.kernel_type, p->param.M, p->param.H, wt, wt_rc); wt_nk = nk; }
-            uint8_t *we = p->wend + (size_t) i * 32 * (size_t) W;
-            for (int s = 0; s < nk; s++) {
-                we[s + L - 1] = wt[s];
-                we[n + s + L - 1] = wt_rc[s];
-            }
-        }
-    }
-    return NULL;
-}
-
-/* build the device image on the host.
- * Per sequence one circular string of 32*Wc positions: forward strand at [0,len), reverse
- * complement at [len,2len), zero padding behind.  planes[i][0..1][Wc] = the two code bit planes,
- * planes[i][2][Wc] = E, the positions at which an L-mer of either strand may END
- * (L-1 <= j < len and len+L-1 <= j < 2len).  wend[i][32*Wc] = weight of the L-mer ending at j. */
 /* shape of the image: words per plane and the sqnorm buffer; the image itself is built on the device */
 int gkm_shape_problem(gkmb200_problem *p)
 {
@@ -478,11 +371,13 @@ int gkm_shape_problem(gkmb200_problem *p)
     return 0;
 }
 
+/* the image of every sequence on the host, by the rule the device packer applies (gkm_pack.h): for the CPU emulators of
+ * the test tier only, so one position at a time */
 int gkm_pack_problem(gkmb200_problem *p)
 {
     if (p->packed && p->planes) return 0;
     if (gkm_shape_problem(p)) return 1;
-    const int W = p->Wmax;
+    const int W = p->Wmax, L = p->param.L;
     p->planes = (uint32_t *) calloc((size_t) p->n * 3 * (size_t) W, sizeof(uint32_t));
     if (p->weighted) p->wend = (uint8_t *) calloc((size_t) p->n * 32 * (size_t) W, 1);
     if (!p->planes || (p->weighted && !p->wend)) {
@@ -490,26 +385,21 @@ int gkm_pack_problem(gkmb200_problem *p)
         gkm_set_error("out of memory packing %d sequences", p->n);
         return 1;
     }
-    /* sequences are independent: a few host threads share them (the reference builds its per-sequence
-     * arrays serially inside read_fasta_file, libgkm.c:1251-1314) */
-    int nt = (int) sysconf(_SC_NPROCESSORS_ONLN);
-    if (nt > 8) nt = 8;
-    if (nt > p->n / 512) nt = p->n / 512;
-    if (nt < 1) nt = 1;
-    pthread_t th[8];
-    struct pack_job jobs[8];
-    int started[8];
-    for (int t = 0; t < nt; t++) {
-        jobs[t].p = p;
-        jobs[t].i0 = (int) ((long long) p->n * t / nt);
-        jobs[t].i1 = (int) ((long long) p->n * (t + 1) / nt);
-        started[t] = 0;
-        if (t > 0) started[t] = (pthread_create(&th[t], NULL, pack_worker, &jobs[t]) == 0);
-    }
-    pack_worker(&jobs[0]);
-    for (int t = 1; t < nt; t++) {
-        if (started[t]) pthread_join(th[t], NULL);
-        else pack_worker(&jobs[t]);
+    uint8_t tab[GKM_MAX_BASES + 1];
+    if (p->weighted) gkm_posweight_table(p->param.kernel_type, p->param.M, p->param.H, tab);
+    for (int i = 0; i < p->n; i++) {
+        const int len = p->len[i], centre = (len - L + 1) / 2;
+        uint32_t *pl = p->planes + (size_t) i * 3 * (size_t) W;
+        for (int wi = 0; wi < W; wi++)
+            for (int b = 0; b < 32; b++) {
+                const int j = wi * 32 + b;
+                int s;
+                const uint32_t code = gkm_pack_code(gkm_letters(p, i), len, L, j, &s);
+                pl[wi] |= (code & 1u) << b;
+                pl[W + wi] |= (code >> 1) << b;
+                pl[2 * W + wi] |= (uint32_t) (s >= 0) << b;
+                if (p->weighted) p->wend[(size_t) i * 32 * (size_t) W + (size_t) j] = gkm_pack_weight(tab, centre, s);
+            }
     }
     return 0;
 }

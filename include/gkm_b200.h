@@ -51,7 +51,7 @@ const char *gkmb200_last_error(void);
 int gkmb200_abi_version(void);
 int gkmb200_device_count(void);                      /* visible CUDA devices of compute capability 10.x; 0 if none */
 int gkmb200_set_devices(const int *ids, int n);      /* default: env GKM_DEVICES ("0,1,.."), else all */
-int gkmb200_set_option(const char *key, const char *value); /* "kernel" = auto|lmer|diag|mma|index ; "max_L" = 12|16 ; "chunk_mb", "index_cols", "index_split" = auto|equal|greedy, "index_wide", "pack" = device|host */
+int gkmb200_set_option(const char *key, const char *value); /* "kernel" = auto|lmer|diag|mma|index ; "max_L" = 12|16 ; "chunk_mb", "index_cols", "index_split" = auto|equal|greedy, "index_wide" */
 void gkmb200_set_verbosity(int level);               /* 0..4 like gkmOpt.verbosity */
 int gkmb200_trim(void);                              /* give the cached device blocks of every GPU back to the driver */
 

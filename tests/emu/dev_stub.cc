@@ -1,9 +1,10 @@
 /* tests/emu/dev_stub.cc -- a host stand-in for the device layer (the gkm_dev_* functions of
- * gkm_device.cu, gkm_compute.cu, gkm_resident.cu and gkm_microbench.cu), for ONE purpose: to run the
+ * gkm_device.cu, gkm_compute.cu, gkm_resident.cu and gkm_microbench.cu), to run the
  * reference-ABI shim gkm_capi.c (gkmkernel_init / read_problems / new_object / build_tree / kernelfunc_batch[_all] /
  * swap_index / update_index, libgkm.h:132-147) in the CPU-only test tier, also under ASan + UBSan
  * (tools/asan_host.sh).  gkm_capi.c is pointer bookkeeping over caller-visible structs -- the code ADVICE r1 found a heap
- * overflow in -- and on the GPU box it can only be exercised unsanitised.
+ * overflow in -- and on the GPU box it can only be exercised unsanitised.  It also hands out the host packer's image
+ * (gkmb200_problem_image), so that the CPU tier can check the packing rule the device packer shares with it.
  *
  * TEST INFRASTRUCTURE, not a fallback: this file is linked into build/libgkm_abi_emu.so only; the product
  * (gkmqc_b200/bin/gkmkern_pylib.so) has no CPU path and fails loudly without a B200.
@@ -103,6 +104,19 @@ int gkm_dev_bench_lower(gkmb200_problem *, int, int, int, double *) { return no_
 int gkm_dev_microbench(const char *, double *) { return no_device("a micro-benchmark"); }
 int gkm_dev_svm_cv(gkmb200_problem *, const double *, long, int, int, const gkmb200_svm_task *, const int *, const signed char *,
                    const int *, double, double, int, double *, gkmb200_svm_fit *, double *) { return no_device("the SVM consumer"); }
+/* the image as the host packer builds it (gkm_seq.c: gkm_pack_problem, the rule of gkm_pack.h), in the layout of the
+ * device's gkmb200_problem_image: the CPU tier checks it against an independent model of the image */
+int gkmb200_problem_image(gkmb200_problem *p, uint32_t *planes, uint8_t *wend, int *out_shape)
+{
+    if (!p) { gkm_set_error("null problem"); return 1; }
+    if (gkm_pack_problem(p)) return 1;
+    const size_t n = (size_t) p->n, W = (size_t) p->Wmax;
+    if (out_shape) { out_shape[0] = p->n; out_shape[1] = p->Wmax; }
+    if (planes) memcpy(planes, p->planes, n * 3 * W * sizeof(uint32_t));
+    if (wend && p->weighted) memcpy(wend, p->wend, n * 32 * W);
+    return 0;
+}
+
 /* the index variant never runs here: the launch record (gkm_device.cu) has nothing to report */
 int gkmb200_problem_index_blocks(const gkmb200_problem *, long long *, int) { no_device("the index launch record"); return -1; }
 

@@ -7,6 +7,7 @@ import os
 import numpy as np
 import pytest
 
+import pack_model
 import pyoracle
 from conftest import load_golden, random_seqs
 from gkmqc_b200 import capi
@@ -214,30 +215,19 @@ def test_gkm_shard_reaches_the_pywrapper_only(lib, tmp_path, monkeypatch):
     assert np.array_equal(parts[0][low] + parts[1][low], g["kmat"][low])
 
 
-@pytest.mark.parametrize("kernel_type,L,M,H", [(2, 11, 50, 50.0), (4, 11, 50, 50.0), (5, 10, 255, 20.0), (4, 3, 1, 3.0)])
-def test_device_packing_equals_host_packing(kernel_type, L, M, H, lib):
+@pytest.mark.parametrize("kernel_type,L,M,H", pack_model.PARAMS)
+def test_device_packing_equals_model(kernel_type, L, M, H, lib):
     """SURVEY.md 8f/f2: the GPU builds the 2-bit plane image (both strands, window-end plane, positional weights by end
-    position) from one byte per base; gkm_seq.c builds the same image on the host for the CPU emulators.  Same bytes."""
-    seqs = random_seqs(257, 400, seed=11, ragged=True)
-    rng = np.random.default_rng(5)
-    for ln in (L, L + 1, 31, 32, 33, 63, 64, 65, 96, 1024, 2046, 2047):
-        if ln >= L:
-            seqs.append(np.frombuffer(b"ACGT", np.uint8)[rng.integers(0, 4, ln)].tobytes().decode())
-    seqs = [s for s in seqs if len(s) >= L]
-    seqs[3] = "acgtNNacgtRYacgtacgt" + seqs[3]      # lower case and non-ACGT letters count as A (libgkm.c:864-875)
-    images = {}
-    try:
-        for who in ("device", "host"):
-            capi.set_option("pack", who)
-            with capi.Problem(kernel_type, L, min(L, 7), min(3, L - min(L, 7)), M, H, 1.0) as P:
-                P.add_many(seqs)
-                images[who] = P.image()
-                st = P.stats()
-    finally:
-        capi.set_option("pack", "device")
-    assert np.array_equal(images["device"][0], images["host"][0]), "bit planes"
+    position) from one byte per base, by the rule of gkm_pack.h.  It must equal the numpy model of the image; the CPU tier
+    holds the host packer of the emulators to the same model (test_pack_model.py), so the two packers agree."""
+    seqs = pack_model.sequences(L)
+    with capi.Problem(*pack_model.problem_args(kernel_type, L, M, H)) as P:
+        P.add_many(seqs)
+        planes, wend = P.image()
+    want_planes, want_wend = pack_model.image(seqs, L, kernel_type, M, H)
+    assert np.array_equal(planes, want_planes), "bit planes"
     if kernel_type in (4, 5):
-        assert np.array_equal(images["device"][1], images["host"][1]), "positional weights by window end"
-        assert images["device"][1].max() == (M if M < 255 else 247)  # M = 255: the centre weight 256 wraps to 0 in the reference's u_int8_t
+        assert np.array_equal(wend, want_wend), "positional weights by window end"
+        assert wend.max() == (M if M < 255 else 247)  # M = 255: the centre weight 256 wraps to 0 in the reference's u_int8_t
     else:
-        assert images["device"][1] is None
+        assert wend is None

@@ -140,16 +140,16 @@ def test_chunk_plan_offsets(product_lib):
     assert sum(c[4] for c in chunks) == 50 * 30
 
 
-def test_set_option_keys(product_lib):
+def test_set_option_keys_refuses_retired_switches(product_lib):
     """A/B switches whose measurements are settled are no longer options; the ones tests and callers use are still taken"""
-    for key, value in (("diag_flavor", "2"), ("tile_rows", "4")):
+    for key, value in (("diag_flavor", "2"), ("tile_rows", "4"), ("pack", "host")):
         with pytest.raises(capi.GkmError, match="unknown option " + key):
             capi.set_option(key, value)
     try:
-        for key, value in (("kernel", "diag"), ("index_cols", "128"), ("index_split", "greedy"), ("index_wide", "1"), ("pack", "host")):
+        for key, value in (("kernel", "diag"), ("index_cols", "128"), ("index_split", "greedy"), ("index_wide", "1")):
             capi.set_option(key, value)
     finally:
-        for key, value in (("kernel", "auto"), ("index_cols", "0"), ("index_split", "auto"), ("index_wide", "0"), ("pack", "device")):
+        for key, value in (("kernel", "auto"), ("index_cols", "0"), ("index_split", "auto"), ("index_wide", "0")):
             capi.set_option(key, value)
 
 

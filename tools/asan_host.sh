@@ -29,6 +29,7 @@ LD_PRELOAD=$(gcc -print-file-name=libasan.so) ASAN_OPTIONS=detect_leaks=0 UBSAN_
 GKM_PYLIB=$LIB GKM_EMU_LIB=$LIB GKM_ABI_EMU_LIB=$PWD/$B/libgkm_abi_emu_asan.so python -m pytest -q -x -m "not gpu" \
     tests/test_abi_on_emulator.py tests/test_abi_vs_reference.py tests/test_pywrapper_vs_reference.py tests/test_fasta_fuzz.py tests/test_sched_properties.py tests/test_posweights_properties.py \
     tests/test_host_logic.py tests/test_index_host.py tests/test_emu_bitslice.py tests/test_lmer_table_model.py tests/test_lmer_subst_model.py \
+    tests/test_pack_model.py \
     --deselect tests/test_host_logic.py::test_library_exports_every_declared_symbol \
     --deselect tests/test_host_logic.py::test_copy_threads_policy \
     --deselect tests/test_host_logic.py::test_compute_fails_loudly_without_gpu "$@"
